@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the render path: forward + backward of render_gaussians on synthetic gaussians.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json metric "fwd+bwd ms/frame & Gaussians*px/s at 3M Gauss 2048px"): 3,000,000 seeded random
@@ -396,7 +396,11 @@ def run_ours(args):
       graph_state["graphs"].clear()
       graph_state["capturing"] = False
       torch.cuda.synchronize()
-  run_dev = (lambda: graph_step(False)) if use_graph else (lambda: step(False))
+  last = {}
+
+  def run_dev():
+    last["loss"] = graph_step(False) if use_graph else step(False)
+
   run_e2e = (lambda: graph_step(True)) if use_graph else (lambda: step(True))
 
   for _ in range(args.warmup):
@@ -407,6 +411,11 @@ def run_ours(args):
   stats["record_phases"] = True
   ms_dev = timed(run_dev, args.steps)
   stats["record_phases"] = False
+  # the passes below run the step again and overwrite the bucket: the last timed step's outputs are copied out now
+  dumped = None
+  if args.dump_outputs and rank == 0:
+    names = ("position", "log_scaling", "rotation", "alpha_logit", "feature")
+    dumped = sample_outputs(last["loss"], {k: p.grad for k, p in zip(names, params)})
   ms_eager = None
   if use_graph and world == 1:   # the same step issued eagerly (round 2a's headline), for the record
     for _ in range(2):
@@ -609,8 +618,39 @@ def run_ours(args):
     out["configs"] = run_configs(device)
   if rank == 0 and world == 1 and not args.no_cpu_baseline:
     out["cpu_baseline"] = cpu_baseline(W, budget_s=args.cpu_budget)
+  if dumped is not None:
+    write_outputs(args.dump_outputs, dumped)
   if rank == 0:
     print(json.dumps(out))
+
+
+DUMP_BYTES = 64_000_000
+
+
+def sample_outputs(loss, grads, budget=DUMP_BYTES, seed=0):
+  """What a caller of the timed step receives, copied to the host as float32 numpy arrays: the step's loss (the sum
+  of this rank's view losses) and the gradient of every parameter.  When all gradient rows would take more than
+  `budget` bytes, every gradient is cut down to the same rows: a sorted sample of the gaussians drawn from `seed`, so
+  that two runs with the same arguments dump the same rows."""
+  n = next(iter(grads.values())).shape[0]
+  row_bytes = sum(g[0].numel() * 4 for g in grads.values())
+  keep = (budget - (1 << 16)) // row_bytes   # 64 KB left for the loss and the .npy headers
+  rows = None
+  if n > keep:
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+  out = {"loss": loss.detach().float().reshape(1).cpu().numpy()}
+  for name, g in grads.items():
+    g = g if rows is None else g.index_select(0, rows.to(g.device))
+    out[f"grad_{name}"] = g.detach().float().cpu().numpy()
+  return out
+
+
+def write_outputs(directory, arrays):
+  import numpy as np
+  path = Path(directory)
+  path.mkdir(parents=True, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(path / f"{name}.npy", a)
 
 
 def run_configs(device, steps=5):
@@ -715,7 +755,7 @@ def run_reference(args):
   warmup = min(args.warmup, 1)           # a full-size frame takes seconds: one warm-up frame is enough for a CPU
   for _ in range(warmup):
     frame()
-  steps = max(1, min(args.steps, 10))
+  steps = args.steps
   t0 = time.perf_counter()
   for _ in range(steps):
     V, K = frame()
@@ -777,7 +817,15 @@ def main():
   ap.add_argument("--no-reduce-early", dest="reduce_early", action="store_false",
                   help="N > 1: one all-reduce of the whole bucket after the last view (the default)")
   ap.set_defaults(reduce_early=False)
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32): the loss and "
+                       "the gradient of every parameter, cut down to a fixed seeded sample of the gaussians when larger "
+                       "than 64 MB in all")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl != "ours":
+    ap.error("--dump-outputs writes the outputs of --impl ours")
   if args.impl == "reference":
     run_reference(args)
   else:
