@@ -275,7 +275,10 @@ typedef struct GsRasterParams {
   int32_t dtype;
   int32_t image_width, image_height;
   int32_t tile_size;                 /* 8, 16 or 32 */
-  int32_t num_features;              /* F */
+  int32_t num_features;              /* F: 1..256 in f32 with tile_size 16, alpha blending and no antialiasing
+                                        (antialiased: 1..7; 65..256 read rows of 16-byte aligned features in place
+                                        when F is a multiple of 64); 1..40 in f32 otherwise (tile_size 32: 1..8);
+                                        1..8 in f64 (tile_size 32: 1..4).  Other counts: GS_ERR_UNSUPPORTED */
   int32_t antialias;
   int32_t use_alpha_blending;
   int32_t compute_visibility;

@@ -12,24 +12,34 @@ constexpr int kFastTileArea = kFastTile * kFastTile;
 // padded feature row length used by the fast kernels for a given F (0 = unsupported)
 inline int fast_feature_pad(int F) { return F <= 4 ? 4 : F <= 8 ? 8 : F <= 16 ? 16 : F <= 36 ? 36 : F <= 64 ? 64 : 0; }
 
+// Extra-wide features (65..256 channels, raster_fast_xwide.cu): rows of xwide_row(F) floats, 64-channel slices.
+constexpr int kXwideSlice = 64;
+constexpr int kXwideMaxFeatures = 256;
+inline bool xwide_features(int F) { return F > 64 && F <= kXwideMaxFeatures; }
+__host__ __device__ inline int xwide_row(int F) { return (F + kXwideSlice - 1) / kXwideSlice * kXwideSlice; }
+
 // Workspace layout (all 256 B aligned):
 //   recF  V x 2 float4 : {mx, my, a1x, a1y} {a2x, a2y, log2(alpha), idx}       (forward records)
-//   featP V x FP float  : features padded to FP
+//   featP V x FP float  : features padded to FP (extra-wide: empty when F is a multiple of 64, the kernels then read
+//                         the caller's features in place)
 //   mask  K bytes        : per tile-list entry, which of the tile's eight 8x4 pixel blocks it can reach
 //   recB  V x 2 float4 : {mx, my, ax, ay} {1/sx, 1/sy, alpha, idx}             (records of the wide backward, F > 7;
 //                                                                               the narrow one walks recF)
 struct FastLayout {
   size_t off_recF, off_feat, off_recB, off_mask, total;
   int FP;
+  bool feat_in_place;
 };
 
 inline FastLayout fast_layout(const GsRasterParams& p) {
   FastLayout L;
-  L.FP = fast_feature_pad(p.num_features);
+  const bool xw = xwide_features(p.num_features);
+  L.FP = xw ? xwide_row(p.num_features) : fast_feature_pad(p.num_features);
+  L.feat_in_place = xw && L.FP == p.num_features;
   const size_t V = (size_t)(p.num_points > 0 ? p.num_points : 1);
   size_t off = 0;
   L.off_recF = off; off += align_up(V * 32, 256);
-  L.off_feat = off; off += align_up(V * (size_t)L.FP * 4, 256);
+  L.off_feat = off; off += L.feat_in_place ? 0 : align_up(V * (size_t)L.FP * 4, 256);
   L.off_recB = off; off += align_up(V * 32, 256);
   // one byte per tile-list entry: bit w = the entry can reach the 8x4 pixel block w of its tile (raster_cull_mask)
   L.off_mask = off; off += align_up((size_t)(p.num_overlaps > 0 ? p.num_overlaps : 1), 256);
@@ -89,6 +99,21 @@ __device__ __forceinline__ bool block_may_touch(float mx, float my, float a1x, f
   return fminf(qv, qh) < qmax * 1.001f + 1e-3f;
 }
 
+// ------------------------------------------------------------------------------------------------ tensor cores
+// D += A . B on one m16n8k8 tile, tf32 inputs, f32 accumulate (used by the wide backward kernels)
+__device__ __forceinline__ void mma_tf32_16x8x8(float (&c)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
+  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
+               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+
+// x = hi + lo, both rounded to nearest tf32: residual 2^-24 |x|
+__device__ __forceinline__ unsigned tf32_rna(float x) {
+  unsigned r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+  return r;
+}
+
 // ------------------------------------------------------------------------------------------------ warp reductions
 // Transposed butterfly over NV per-lane partial sums: every exchange step halves the number of live values
 // (the lane keeps the half selected by its lane bit and adds the partner's copy of it), so NV values cost about
@@ -136,11 +161,19 @@ __device__ __forceinline__ int reduce_owner(int lane) {
   return cnt == 1 ? base : -1;
 }
 
+// the padded feature rows the fast kernels stage from (workspace, or the caller's features read in place)
+inline const float* fast_feature_rows(const GsRasterParams& p, const RasterArgs& a) {
+  const FastLayout L = fast_layout(p);
+  return L.feat_in_place ? (const float*)a.features : (const float*)((unsigned char*)a.workspace + L.off_feat);
+}
+
 int raster_fast_pack(const GsRasterParams& p, const RasterArgs& a, bool forward, bool features, cudaStream_t st);
 // cull masks of every tile-list entry against the eight 8x4 pixel blocks of its tile (needs the forward records)
 int raster_cull_mask(const GsRasterParams& p, const RasterArgs& a, cudaStream_t st);
 
 // raster_fast_bwd_wide.cu: backward for 8..64 feature channels (one pixel per lane, image gradient in registers)
 int raster_bwd_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP, cudaStream_t st);
+// raster_fast_xwide.cu: backward for 65..256 feature channels (image gradient in shared memory)
+int raster_bwd_xwide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP, cudaStream_t st);
 
 }  // namespace gs

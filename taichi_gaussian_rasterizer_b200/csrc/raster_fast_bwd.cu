@@ -396,7 +396,9 @@ int raster_bwd_fast(const GsRasterParams& p, const RasterArgs& a, cudaStream_t s
   }
   const FastLayout L = fast_layout(p);
   unsigned char* ws = (unsigned char*)a.workspace;
-  const float* featP = (const float*)(ws + L.off_feat);
+  const float* featP = fast_feature_rows(p, a);
+  if (xwide_features(p.num_features))   // 65..256 channels: the image gradient in shared memory
+    return raster_bwd_xwide(p, a, (const float4*)(ws + L.off_recB), featP, st);
   if (p.num_features > 7)   // 8..64 channels: one pixel per lane, its own records
     return raster_bwd_wide(p, a, (const float4*)(ws + L.off_recB), featP, st);
   const float4* rec = (const float4*)(ws + (p.antialias ? L.off_recB : L.off_recF));   // the forward's records

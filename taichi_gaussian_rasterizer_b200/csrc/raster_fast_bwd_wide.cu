@@ -201,19 +201,6 @@ raster_bwd_wide_kernel(const __grid_constant__ GsRasterParams p, const float4* _
 constexpr int kMmaGroup = 16;   // survivors per product (M of the mma)
 constexpr int kMmaBatch = 32;   // staged tile-list entries per buffer (64: 8.6 ms instead of 6.9 at config 4, the warps of a CTA drift further apart between barriers)
 
-__device__ __forceinline__ void mma_tf32_16x8x8(float (&c)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
-// x = hi + lo, both rounded to nearest tf32: residual 2^-24 |x| (see raster_fast_fwd_wide.cu)
-__device__ __forceinline__ unsigned tf32_rna(float x) {
-  unsigned r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return r;
-}
-
 template <int FP>
 struct WideMmaLayout {
   static constexpr int FP8 = (FP + 7) / 8 * 8;   // channels padded to n-tiles of 8

@@ -52,8 +52,38 @@ raster_pack_kernel(int64_t V, int F, const float* __restrict__ g, const float* _
   }
 }
 
+// extra-wide features whose rows are not a whole number of 64-channel slices: one thread per padded element
+__global__ void __launch_bounds__(256)
+raster_pad_rows_kernel(int64_t n, int F, int FP, const float* __restrict__ feat, float* __restrict__ featP) {
+  const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= n) return;
+  const int64_t i = q / FP;
+  const int c = (int)(q - i * FP);
+  featP[q] = c < F ? feat[i * F + c] : 0.f;
+}
+
 int raster_fast_pack(const GsRasterParams& p, const RasterArgs& a, bool forward, bool features, cudaStream_t st) {
   if (p.num_points == 0) return GS_OK;
+  if (xwide_features(p.num_features)) {   // records as for the wide path, features padded to 64-channel slices
+    const FastLayout L = fast_layout(p);
+    if (L.feat_in_place && ((uintptr_t)a.features & 15) != 0) {   // cp.async stages them in 16 B pieces
+      set_error("rasterizer: %d feature channels are read in place and must be 16-byte aligned", p.num_features);
+      return GS_ERR_INVALID;
+    }
+    unsigned char* ws = (unsigned char*)a.workspace;
+    const bool want_bwd = !forward || p.points_requires_grad || p.features_requires_grad;
+    raster_pack_kernel<4><<<(unsigned)ceil_div(p.num_points, 256), 256, 0, st>>>(
+        p.num_points, p.num_features, (const float*)a.gaussians2d, nullptr, forward ? (float4*)(ws + L.off_recF) : nullptr,
+        nullptr, want_bwd ? (float4*)(ws + L.off_recB) : nullptr);
+    GS_LAUNCH_CHECK();
+    if (features && !L.feat_in_place) {
+      const int64_t n = p.num_points * (int64_t)L.FP;
+      raster_pad_rows_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, st>>>(n, p.num_features, L.FP, (const float*)a.features,
+                                                                         (float*)(ws + L.off_feat));
+      GS_LAUNCH_CHECK();
+    }
+    return GS_OK;
+  }
   const FastLayout L = fast_layout(p);
   unsigned char* ws = (unsigned char*)a.workspace;
   // the forward call also packs the backward records when a gradient will be asked for, so that the backward
@@ -150,7 +180,13 @@ int raster_cull_mask(const GsRasterParams& p, const RasterArgs& a, cudaStream_t 
 // ------------------------------------------------------------------------------------------------ forward
 // BATCH = staged tile-list entries per buffer: 128 for narrow features, 64 for FP >= 16 (shared memory budget).
 // FOURTH: with FP = 4 the fourth accumulator is only needed when F = 4 (it is padding for F <= 3).
-template <int FP, bool VIS, int BATCH, bool FOURTH = true, bool AA = false>
+// XW: extra-wide features (65..256 channels).  The CTA of blockIdx.y = s blends channel slice [64 s, 64 s + 64) of
+// rows of xwide_row(F) floats; every slice walks the tile list with the same records, cull bytes and exit test, and
+// only slice 0 writes image_alpha and visibility.  Why CTAs per slice and not slice warps inside one CTA: a tile's
+// 256 pixels x 256 channels of accumulators (256 KB) are the whole register file of an SM, so a CTA can hold the
+// full channel range of a few pixel blocks only, and each such CTA would stage all F channels of every entry (4 x
+// the feature bytes at F = 256 for four CTAs per tile); a slice CTA stages its own 64 channels and the records.
+template <int FP, bool VIS, int BATCH, bool FOURTH = true, bool AA = false, bool XW = false>
 __global__ void __launch_bounds__(kFwdThreads, FP <= 8 ? 0 : (FP <= 36 ? 4 : 2))   // narrow: no occupancy target (the compiler settles on 30 registers = 8 CTAs per SM by itself; forcing 8 lengthened the VIS walk); 64 / 128 registers for the wide ones
 raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* __restrict__ rec,
                        const float* __restrict__ featP, const int32_t* __restrict__ ranges,
@@ -178,6 +214,10 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
   const float pxf = (float)px + 0.5f, pyf = (float)py + 0.5f;
   const float thr = (float)p.alpha_threshold, cmax = (float)p.clamp_max_alpha;
   const float exit_T = (float)p.forward_exit_transmittance;
+  // feature row stride and this CTA's first channel (XW), whether it writes image_alpha / visibility
+  const int frow = XW ? xwide_row(F) : FP;
+  const int c_base = XW ? (int)blockIdx.y * FP : 0;
+  const bool first_slice = !XW || blockIdx.y == 0;
 
   float acc[FP];
 #pragma unroll
@@ -206,7 +246,7 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
           s_mask[buf][slot] = m;
         } else {
 #pragma unroll
-          for (int c = 0; c < FP; c += 4) cp_async16(&s_e[buf][slot][2 + c / 4], featP + (int64_t)idx * FP + c);
+          for (int c = 0; c < FP; c += 4) cp_async16(&s_e[buf][slot][2 + c / 4], featP + (int64_t)idx * frow + c_base + c);
         }
       }
     } else {  // wide rows: records by the first BATCH threads, the 16 B feature chunks spread over the whole CTA
@@ -229,7 +269,7 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
         const int v = b * kFwdBatch + slot;
         if (q < kFwdBatch * CH && v < total) {
           const int idx = o2p[start + (v < C ? v : v - kFastTileArea)];
-          cp_async16(&s_e[buf][slot][2 + part], featP + (int64_t)idx * FP + part * 4);
+          cp_async16(&s_e[buf][slot][2 + part], featP + (int64_t)idx * frow + c_base + part * 4);
         }
       }
     }
@@ -299,7 +339,7 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
             // makes ptxas emit its warp-aggregation sequence (vote, leader election, popc, multiply: 9 more instructions
             // per survivor) although a single lane enters.
             const unsigned total_q = __reduce_add_sync(kFull, __float_as_uint(1.0f + weight)) - 0xf0000000u;
-            if (lane == 0 && vbase + j < C) s_vis[buf][j][warp] = total_q;
+            if (lane == 0 && vbase + j < C && first_slice) s_vis[buf][j][warp] = total_q;
           }
         }
       }
@@ -327,14 +367,15 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
     const int64_t pix = (int64_t)py * p.image_width + px;
 #pragma unroll
     for (int c = 0; c < FP; ++c)
-      if (c < F) image[pix * F + c] = acc[c];
-    image_alpha[pix] = W;
+      if (c_base + c < F) image[pix * F + c_base + c] = acc[c];
+    if (first_slice) image_alpha[pix] = W;
   }
 }
 
 bool raster_fast_supported(const GsRasterParams& p) {
   return p.dtype == GS_F32 && p.tile_size == kFastTile && (!p.antialias || p.num_features <= 7) &&
-         p.use_alpha_blending && fast_feature_pad(p.num_features) != 0 && p.num_points < (1ll << 31);
+         p.use_alpha_blending && (fast_feature_pad(p.num_features) != 0 || xwide_features(p.num_features)) &&
+         p.num_points < (1ll << 31);
 }
 
 size_t raster_fast_workspace_bytes(const GsRasterParams& p) { return fast_layout(p).total; }
@@ -348,9 +389,20 @@ int raster_fwd_fast(const GsRasterParams& p, const RasterArgs& a, cudaStream_t s
   unsigned char* ws = (unsigned char*)a.workspace;
   const unsigned char* cmask = ws + L.off_mask;
   const float4* rec = (const float4*)(ws + (p.antialias ? L.off_recB : L.off_recF));
-  const float* featP = (const float*)(ws + L.off_feat);
+  const float* featP = fast_feature_rows(p, a);
   const int tiles = tiles_wide(p) * tiles_high(p);
   const bool vis = p.compute_visibility && a.visibility != nullptr;
+  if (xwide_features(p.num_features)) {   // one CTA per (tile, 64-channel slice)
+    const dim3 grid(tiles, L.FP / kXwideSlice);
+#define GS_FWD_XW(VISV)                                                                                            \
+  raster_fwd_fast_kernel<kXwideSlice, VISV, 64, true, false, true><<<grid, kFwdThreads, 0, st>>>(                  \
+      p, rec, featP, a.tile_ranges, a.overlap_to_point, (float*)a.image, (float*)a.image_alpha, (float*)a.visibility, \
+      cmask)
+    if (vis) GS_FWD_XW(true); else GS_FWD_XW(false);
+#undef GS_FWD_XW
+    GS_LAUNCH_CHECK();
+    return GS_OK;
+  }
   if (p.antialias) {   // narrow features only (raster_fast_supported)
 #define GS_FWD_AA(FPV, VISV, FOURTHV)                                                                              \
   raster_fwd_fast_kernel<FPV, VISV, 128, FOURTHV, true><<<tiles, kFwdThreads, 0, st>>>(                            \

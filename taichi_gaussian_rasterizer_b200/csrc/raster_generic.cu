@@ -309,7 +309,8 @@ int raster_fwd_generic(const GsRasterParams& p, const RasterArgs& a, cudaStream_
     if (F <= 8) return fwd_modes<float, 8, 256>(p, a, st);
     if (F <= 16) return fwd_modes<float, 16, 256>(p, a, st);
     if (F <= 40) return fwd_modes<float, 40, 256>(p, a, st);
-    GS_UNSUPPORTED("rasterizer forward: %d feature channels (f32 supports up to 40)", F);
+    GS_UNSUPPORTED("rasterizer forward: %d feature channels (f32 supports up to 40, or up to 256 with "
+                   "tile_size 16, alpha blending and no antialiasing)", F);
   }
   if (big) {
     if (F <= 4) return fwd_modes<double, 4, 1024>(p, a, st);
@@ -333,7 +334,8 @@ int raster_bwd_generic(const GsRasterParams& p, const RasterArgs& a, cudaStream_
     if (F <= 8) return bwd_modes<float, 8, 256>(p, a, st);
     if (F <= 16) return bwd_modes<float, 16, 256>(p, a, st);
     if (F <= 40) return bwd_modes<float, 40, 256>(p, a, st);
-    GS_UNSUPPORTED("rasterizer backward: %d feature channels (f32 supports up to 40)", F);
+    GS_UNSUPPORTED("rasterizer backward: %d feature channels (f32 supports up to 40, or up to 256 with "
+                   "tile_size 16, alpha blending and no antialiasing)", F);
   }
   if (big) {
     if (F <= 4) return bwd_modes<double, 4, 1024>(p, a, st);
