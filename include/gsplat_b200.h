@@ -296,7 +296,11 @@ typedef struct GsRasterParams {
                                         feature gradient with warp butterflies (default: mma.sync product), bit 2 = the
                                         rasterizer kernels launch at the stream's priority (default: the lowest, so that a
                                         caller's high-priority streams put every other kernel first), bits 3-4 = warps per
-                                        CTA of the wide backward: 0 -> two (default), 1 -> eight, 2 -> four, 3 -> one */
+                                        CTA of the wide backward: 0 -> two (default), 1 -> eight, 2 -> four, 3 -> one.
+                                        gs_raster_bwd_with_weight with a weight gradient ignores bits 0, 1, 3 and 4:
+                                        its narrow backward reduces every survivor alone, its wide one is the
+                                        shipped two-warp tensor-core kernel (no other weight-gradient instantiation
+                                        exists) */
   int64_t num_points;                /* V */
   int64_t num_overlaps;              /* K */
   double clamp_max_alpha, alpha_threshold, saturate_threshold;
@@ -324,6 +328,20 @@ int gs_raster_bwd(const GsRasterParams* p, const void* gaussians2d, const void* 
                   const int32_t* tile_ranges, const int32_t* overlap_to_point, const void* image,
                   const void* grad_image, void* grad_gaussians, void* grad_features,
                   void* point_heuristic, void* workspace, size_t workspace_bytes, void* stream);
+
+/* gs_raster_bwd with a differentiable image weight: image_weight (H,W: the forward's image_alpha) and its gradient
+ * grad_image_weight (H,W).  The weight W = sum_i w_i is the blend of a constant feature 1, so its gradient flows into
+ * grad_gaussians and point_heuristic exactly as that of one more channel of ones would (grad_features keeps F
+ * columns).  grad_image_weight NULL: the same call as gs_raster_bwd, the same kernels.  Quantile mode
+ * (use_alpha_blending = 0): the weight is W > 0, piecewise constant, and grad_image_weight is ignored.  With a weight
+ * gradient the narrow backward (F <= 7) reduces every survivor alone (faster there than in pairs) and the wide one
+ * runs the shipped tensor-core kernel: kernel_variant bits 0, 1, 3 and 4 do not apply.
+ * Extra cost per backward row: DESIGN.md §3. */
+int gs_raster_bwd_with_weight(const GsRasterParams* p, const void* gaussians2d, const void* features,
+                              const int32_t* tile_ranges, const int32_t* overlap_to_point, const void* image,
+                              const void* grad_image, const void* image_weight, const void* grad_image_weight,
+                              void* grad_gaussians, void* grad_features, void* point_heuristic, void* workspace,
+                              size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------ visibility-weighted sparse optimizers
  * (SURVEY.md 8f rank 1, the consumers of `visibility`): replace the per point step kernels of

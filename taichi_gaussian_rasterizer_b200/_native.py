@@ -22,7 +22,7 @@ EXPORTS = [
   "gs_radix_sort_pairs_workspace_bytes", "gs_radix_sort_pairs", "gs_radix_sort_pairs_counted", "gs_find_ranges",
   "gs_depth_keys", "gs_depth_keys_counted", "gs_tile_count_perm", "gs_tile_count_perm_counted", "gs_tile_emit_tiles", "gs_find_ranges_tiles",
   "gs_tile_emit_tiles_capped", "gs_tile_emit_tiles_capped_counted", "gs_find_ranges_tiles_counted",
-  "gs_raster_workspace_bytes", "gs_raster_fwd", "gs_raster_bwd",
+  "gs_raster_workspace_bytes", "gs_raster_fwd", "gs_raster_bwd", "gs_raster_bwd_with_weight",
   "gs_opt_update_visibility", "gs_opt_accumulate_weight", "gs_opt_step",
   "gs_morton_codes", "gs_camera_position",
   "gs_multimem_all_reduce_flag_words", "gs_multimem_all_reduce", "gs_cross_rank_barrier",

@@ -19,6 +19,8 @@ struct RasterArgs {
   // backward
   const void* image_in;
   const void* grad_image;
+  const void* image_weight;        // (H, W) forward image_alpha; with grad_image_weight: the weight's gradient too
+  const void* grad_image_weight;   // (H, W) or NULL (no weight gradient: the kernels of gs_raster_bwd)
   void* grad_gaussians;
   void* grad_features;
   void* point_heuristic;

@@ -1,4 +1,4 @@
-// raster_api.cu — gs_raster_fwd / gs_raster_bwd: validation and kernel-family selection.
+// raster_api.cu — gs_raster_fwd / gs_raster_bwd(_with_weight): validation and kernel-family selection.
 #include "raster.cuh"
 
 using namespace gs;
@@ -58,14 +58,19 @@ int gs_raster_fwd(const GsRasterParams* p, const void* gaussians2d, const void* 
   return raster_fwd_generic(*p, a, st);
 }
 
-int gs_raster_bwd(const GsRasterParams* p, const void* gaussians2d, const void* features, const int32_t* tile_ranges,
-                  const int32_t* overlap_to_point, const void* image, const void* grad_image, void* grad_gaussians,
-                  void* grad_features, void* point_heuristic, void* workspace, size_t workspace_bytes, void* stream) {
+int gs_raster_bwd_with_weight(const GsRasterParams* p, const void* gaussians2d, const void* features,
+                              const int32_t* tile_ranges, const int32_t* overlap_to_point, const void* image,
+                              const void* grad_image, const void* image_weight, const void* grad_image_weight,
+                              void* grad_gaussians, void* grad_features, void* point_heuristic, void* workspace,
+                              size_t workspace_bytes, void* stream) {
   int rc = check_raster(p, "gs_raster_bwd");
   if (rc != GS_OK) return rc;
   GS_CHECK_ARG(tile_ranges && grad_image && (image || !p->use_alpha_blending), "gs_raster_bwd: null tensor");
   GS_CHECK_ARG(p->num_points == 0 || (gaussians2d && features), "gs_raster_bwd: null gaussians / features");
   GS_CHECK_ARG(p->num_overlaps == 0 || overlap_to_point, "gs_raster_bwd: null overlap_to_point");
+  // quantile mode: the weight is W > 0, piecewise constant, so its gradient contributes nothing
+  if (!p->use_alpha_blending) grad_image_weight = nullptr;
+  GS_CHECK_ARG(!grad_image_weight || image_weight, "gs_raster_bwd_with_weight: grad_image_weight without image_weight");
   cudaStream_t st = (cudaStream_t)stream;
   const size_t es = p->dtype == GS_F32 ? 4 : 8;
   if (grad_gaussians && p->num_points > 0) GS_CUDA(cudaMemsetAsync(grad_gaussians, 0, (size_t)p->num_points * 7 * es, st));
@@ -74,6 +79,7 @@ int gs_raster_bwd(const GsRasterParams* p, const void* gaussians2d, const void* 
   RasterArgs a = {};
   a.gaussians2d = gaussians2d; a.features = features; a.tile_ranges = tile_ranges;
   a.overlap_to_point = overlap_to_point; a.image_in = image; a.grad_image = grad_image;
+  a.image_weight = grad_image_weight ? image_weight : nullptr; a.grad_image_weight = grad_image_weight;
   a.grad_gaussians = grad_gaussians; a.grad_features = grad_features; a.point_heuristic = point_heuristic;
   a.workspace = workspace; a.workspace_bytes = workspace_bytes;
   if (raster_fast_supported(*p)) {
@@ -85,6 +91,14 @@ int gs_raster_bwd(const GsRasterParams* p, const void* gaussians2d, const void* 
     return raster_bwd_fast(*p, a, st);
   }
   return raster_bwd_generic(*p, a, st);
+}
+
+int gs_raster_bwd(const GsRasterParams* p, const void* gaussians2d, const void* features, const int32_t* tile_ranges,
+                  const int32_t* overlap_to_point, const void* image, const void* grad_image, void* grad_gaussians,
+                  void* grad_features, void* point_heuristic, void* workspace, size_t workspace_bytes, void* stream) {
+  return gs_raster_bwd_with_weight(p, gaussians2d, features, tile_ranges, overlap_to_point, image, grad_image, nullptr,
+                                   nullptr, grad_gaussians, grad_features, point_heuristic, workspace, workspace_bytes,
+                                   stream);
 }
 
 }  // extern "C"

@@ -41,14 +41,17 @@ namespace gs {
 // AA: antialiased pixel function (raster_math.cuh pdf_aa_grad with MUFU arithmetic): the records are the unscaled
 // {mean, axis}{1/sigma, alpha, index}, the seven gradient components are accumulated directly (the moment trick needs
 // a pure gaussian) and no moment pass follows.
-template <int F, int FP, bool HEUR, bool PAIR, bool AA = false>
+// WGT: the image weight W = sum_i w_i is differentiable too (gradient gw (H, W), forward W in wimg).  W is the blend of
+// a constant feature 1, so it enters the replay as one more channel: RG starts with W_final Gw and f . G gains + Gw.
+template <int F, int FP, bool HEUR, bool PAIR, bool AA = false, bool WGT = false>
 __global__ void __launch_bounds__(32, PAIR ? 32 : 1)
 raster_bwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* __restrict__ rec,
                        const float* __restrict__ featP, const int32_t* __restrict__ ranges,
                        const int32_t* __restrict__ o2p, const float* __restrict__ image,
                        const float* __restrict__ grad_image, float* __restrict__ grad_pts,
                        float* __restrict__ grad_feat, float* __restrict__ heuristic,
-                       const unsigned char* __restrict__ cull_mask, const float3 kf) {
+                       const unsigned char* __restrict__ cull_mask, const float3 kf,
+                       const float* __restrict__ wimg, const float* __restrict__ gw) {
   constexpr int NSUB = 4;
   constexpr int kBwdBatch = 64;   // staged tile-list entries per buffer (32 / 128 measured slower)
   constexpr int NM = AA ? 7 : 6;  // moments: g, g u, g w, g u^2, g w^2, g u w; AA: d/d(mean, axis, sigma, alpha)
@@ -95,6 +98,7 @@ raster_bwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
   // Per pixel state: W, the image gradient G and RG = sum_c R_c G_c.  The replay only ever needs the remaining
   // features R through R . G (dL/dalpha = T (f . G) - (R . G) / (1 - alpha)), and R_c -= f_c w means RG -= (f . G) w.
   float W[NSUB], RG[NSUB], Gd[NSUB][F];
+  float Gw[WGT ? NSUB : 1];
 #pragma unroll
   for (int i = 0; i < NSUB; ++i) {
     const int px = x0 + 8 * (i & 1), py = y0 + 4 * (i >> 1);
@@ -106,6 +110,10 @@ raster_bwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
     for (int c = 0; c < F; ++c) {
       Gd[i][c] = inb ? grad_image[pix * F + c] : 0.f;
       RG[i] = fmaf(inb ? image[pix * F + c] : 0.f, Gd[i][c], RG[i]);
+    }
+    if constexpr (WGT) {
+      Gw[i] = inb ? gw[pix] : 0.f;
+      RG[i] = fmaf(inb ? wimg[pix] : 0.f, Gw[i], RG[i]);
     }
   }
 
@@ -172,6 +180,7 @@ raster_bwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
               fG = fmaf(f[c], Gd[i][c], fG);
               gf[c] = fmaf(w, Gd[i][c], gf[c]);
             }
+            if constexpr (WGT) fG += Gw[i];
             RG[i] = fmaf(-fG, w, RG[i]);
             const float ag = fmaf(fG, Ti, -RG[i] * rinv);   // dL/dalpha
             const float aag = a0 * ag * tau;
@@ -217,6 +226,7 @@ raster_bwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
               fG = fmaf(f[c], Gd[i][c], fG);
               gf[c] = fmaf(w, Gd[i][c], gf[c]);
             }
+            if constexpr (WGT) fG += Gw[i];
             RG[i] = fmaf(-fG, w, RG[i]);
             const float ag = fmaf(fG, Ti, -RG[i] * rinv);   // dL/dalpha
             const float gp = ag * araw;                     // alpha0 x the dL/dalpha0 share of this pixel
@@ -357,22 +367,32 @@ static int launch_bwd_fast(const GsRasterParams& p, const RasterArgs& a, const f
   const float3 kf = make_float3((float)p.alpha_threshold, (float)p.clamp_max_alpha, (float)p.saturate_threshold);
   // kernel_variant bit 2 (A/B): launch at the stream's own priority instead of the lowest one (launch_background)
   const bool background = (p.kernel_variant & 4) == 0;
-#define GS_BWD_LAUNCH(HEURV, PAIRV, AAV)                                                                         \
+  const float* wimg = (const float*)a.image_weight;
+  const float* gw = (const float*)a.grad_image_weight;
+#define GS_BWD_LAUNCH(HEURV, PAIRV, AAV, WGTV)                                                                   \
   do {                                                                                                           \
     if (background)                                                                                              \
-      GS_CUDA(launch_background(raster_bwd_fast_kernel<F, FP, HEURV, PAIRV, AAV>, dim3(tiles * 2), dim3(32), 0,  \
-                                st, p, rec, featP, a.tile_ranges, a.overlap_to_point, (const float*)a.image_in,  \
-                                (const float*)a.grad_image, (float*)a.grad_gaussians, (float*)a.grad_features,   \
-                                heur ? (float*)a.point_heuristic : nullptr, cmask, kf));                         \
+      GS_CUDA(launch_background(raster_bwd_fast_kernel<F, FP, HEURV, PAIRV, AAV, WGTV>, dim3(tiles * 2),         \
+                                dim3(32), 0, st, p, rec, featP, a.tile_ranges, a.overlap_to_point,               \
+                                (const float*)a.image_in, (const float*)a.grad_image, (float*)a.grad_gaussians,  \
+                                (float*)a.grad_features, heur ? (float*)a.point_heuristic : nullptr, cmask, kf,  \
+                                wimg, gw));                                                                      \
     else                                                                                                         \
-      raster_bwd_fast_kernel<F, FP, HEURV, PAIRV, AAV><<<tiles * 2, 32, 0, st>>>(                                \
+      raster_bwd_fast_kernel<F, FP, HEURV, PAIRV, AAV, WGTV><<<tiles * 2, 32, 0, st>>>(                          \
           p, rec, featP, a.tile_ranges, a.overlap_to_point, (const float*)a.image_in, (const float*)a.grad_image,\
           (float*)a.grad_gaussians, (float*)a.grad_features, heur ? (float*)a.point_heuristic : nullptr, cmask,  \
-          kf);                                                                                                   \
+          kf, wimg, gw);                                                                                         \
   } while (0)
-  if (p.antialias) { if (heur) GS_BWD_LAUNCH(true, false, true); else GS_BWD_LAUNCH(false, false, true); }
-  else if (heur) { if (pair) GS_BWD_LAUNCH(true, true, false); else GS_BWD_LAUNCH(true, false, false); }
-  else { if (pair) GS_BWD_LAUNCH(false, true, false); else GS_BWD_LAUNCH(false, false, false); }
+  if (gw != nullptr) {
+    // with the weight gradient every survivor is reduced alone: the paired kernel spills 84 B (F = 3) to 296 B (F = 7,
+    // heuristics) under its 64-register cap and measured slower (B200, bench scene: F = 3 1.39 ms paired, 1.37 single;
+    // F = 7 2.60 / 1.84 ms; benchmarks/weight_gradient.py)
+    if (p.antialias) { if (heur) GS_BWD_LAUNCH(true, false, true, true); else GS_BWD_LAUNCH(false, false, true, true); }
+    else if (heur) GS_BWD_LAUNCH(true, false, false, true);
+    else GS_BWD_LAUNCH(false, false, false, true);
+  } else if (p.antialias) { if (heur) GS_BWD_LAUNCH(true, false, true, false); else GS_BWD_LAUNCH(false, false, true, false); }
+  else if (heur) { if (pair) GS_BWD_LAUNCH(true, true, false, false); else GS_BWD_LAUNCH(true, false, false, false); }
+  else { if (pair) GS_BWD_LAUNCH(false, true, false, false); else GS_BWD_LAUNCH(false, false, false, false); }
 #undef GS_BWD_LAUNCH
   GS_LAUNCH_CHECK();
   if (!p.antialias && p.points_requires_grad && a.grad_gaussians != nullptr && p.num_points > 0) {

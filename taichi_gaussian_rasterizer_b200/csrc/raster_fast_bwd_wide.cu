@@ -216,13 +216,16 @@ struct WideMmaLayout {
 
 // WARPS: warps per CTA = 8 (one CTA per tile) or 4 / 2 (two / four CTAs per tile, each staging the tile list for itself:
 // the block barrier of a batch then waits for 4 / 2 warps instead of 8 — 21 % of the stall samples sat there).
-template <int FP, bool HEUR, int WARPS>
+// WGT: the image weight W is differentiable too (gradient gw, forward W in wimg): one more channel whose feature is
+// always 1, so RG starts with W_final Gw and f . G gains + Gw (see raster_bwd_fast_kernel).
+template <int FP, bool HEUR, int WARPS, bool WGT = false>
 __global__ void __launch_bounds__(WARPS * 32, 16 / WARPS)   // 118 registers; an 80-register cap (three CTAs) spills: 8.0 vs 6.8 ms
 raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float4* __restrict__ rec,
                            const float* __restrict__ featP, const int32_t* __restrict__ ranges,
                            const int32_t* __restrict__ o2p, const float* __restrict__ image,
                            const float* __restrict__ grad_image, float* __restrict__ grad_pts,
-                           float* __restrict__ grad_feat, float* __restrict__ heuristic) {
+                           float* __restrict__ grad_feat, float* __restrict__ heuristic,
+                           const float* __restrict__ wimg, const float* __restrict__ gw) {
   using L = WideMmaLayout<FP>;
   constexpr int NG = 7 + (HEUR ? 2 : 0);             // geometry (+ heuristic) values
   extern __shared__ __align__(16) unsigned char smem[];
@@ -254,7 +257,7 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
   const int gid = lane >> 2, tig = lane & 3;
 
   float G[FP];
-  float W = inb ? 0.f : 1.f, RG = 0.f;
+  float W = inb ? 0.f : 1.f, RG = 0.f, Gw = 0.f;
   {
     const int64_t pix = (int64_t)py * p.image_width + px;
 #pragma unroll
@@ -263,6 +266,10 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
       G[c] = ok ? grad_image[pix * F + c] : 0.f;
       RG = fmaf(ok ? image[pix * F + c] : 0.f, G[c], RG);
       s_G[lane * L::GS + c] = G[c];
+    }
+    if constexpr (WGT) {
+      Gw = inb ? gw[pix] : 0.f;
+      RG = fmaf(inb ? wimg[pix] : 0.f, Gw, RG);
     }
 #pragma unroll
     for (int c = FP; c < L::FP8; ++c) s_G[lane * L::GS + c] = 0.f;
@@ -394,7 +401,8 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
             fG0 = fmaf(f4.x, G[c], fG0); fG1 = fmaf(f4.y, G[c + 1], fG1);
             fG2 = fmaf(f4.z, G[c + 2], fG2); fG3 = fmaf(f4.w, G[c + 3], fG3);
           }
-          const float fG = (fG0 + fG1) + (fG2 + fG3);
+          float fG = (fG0 + fG1) + (fG2 + fG3);
+          if constexpr (WGT) fG += Gw;
           RG = fmaf(-fG, wl, RG);
           const float ag = fmaf(fG, Ti, -RG * rinv);
           const float aag = a0 * ag;
@@ -427,16 +435,17 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
   if (ns > 0) flush_group();
 }
 
-template <int FP, bool HEUR, int WARPS>
+template <int FP, bool HEUR, int WARPS, bool WGT = false>
 static int launch_wide_mma_w(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP, int tiles,
                              cudaStream_t st) {
   using L = WideMmaLayout<FP>;
   // per launch: the attribute belongs to the (function, device) pair and the call costs about a microsecond
-  GS_CUDA(cudaFuncSetAttribute(raster_bwd_wide_mma_kernel<FP, HEUR, WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)L::total(WARPS)));
-  raster_bwd_wide_mma_kernel<FP, HEUR, WARPS><<<tiles * (8 / WARPS), WARPS * 32, L::total(WARPS), st>>>(
+  GS_CUDA(cudaFuncSetAttribute(raster_bwd_wide_mma_kernel<FP, HEUR, WARPS, WGT>,
+                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::total(WARPS)));
+  raster_bwd_wide_mma_kernel<FP, HEUR, WARPS, WGT><<<tiles * (8 / WARPS), WARPS * 32, L::total(WARPS), st>>>(
       p, rec, featP, a.tile_ranges, a.overlap_to_point, (const float*)a.image_in, (const float*)a.grad_image,
-      (float*)a.grad_gaussians, (float*)a.grad_features, HEUR ? (float*)a.point_heuristic : nullptr);
+      (float*)a.grad_gaussians, (float*)a.grad_features, HEUR ? (float*)a.point_heuristic : nullptr,
+      (const float*)a.image_weight, (const float*)a.grad_image_weight);
   return GS_OK;
 }
 
@@ -445,7 +454,9 @@ static int launch_wide_mma(const GsRasterParams& p, const RasterArgs& a, const f
                            cudaStream_t st) {
   // Two warps per CTA (four CTAs per tile).  Measured at config 4 (34 channels, 4K; benchmarks/variants.py
   // --variants 0,8,16,24 --scene c4): eight warps 7.05 ms, four 7.35, two 6.39, one 6.99.
-  // kernel_variant bits 3-4 (A/B): 0 = two warps per CTA, 1 = eight, 2 = four, 3 = one
+  // kernel_variant bits 3-4 (A/B): 0 = two warps per CTA, 1 = eight, 2 = four, 3 = one.  With the weight gradient
+  // only the shipped two-warp kernel exists.
+  if (a.grad_image_weight != nullptr) return launch_wide_mma_w<FP, HEUR, 2, true>(p, a, rec, featP, tiles, st);
   switch ((p.kernel_variant >> 3) & 3) {
     case 1: return launch_wide_mma_w<FP, HEUR, 8>(p, a, rec, featP, tiles, st);
     case 2: return launch_wide_mma_w<FP, HEUR, 4>(p, a, rec, featP, tiles, st);
@@ -458,7 +469,8 @@ int raster_bwd_wide(const GsRasterParams& p, const RasterArgs& a, const float4* 
                     cudaStream_t st) {
   const int tiles = tiles_wide(p) * tiles_high(p);
   const bool heur = p.compute_point_heuristic && a.point_heuristic != nullptr;
-  if ((p.kernel_variant & 2) == 0) {   // tensor-core feature gradient (kernel_variant bit 1 = the butterfly kernel)
+  // tensor-core feature gradient (kernel_variant bit 1 = the butterfly kernel, which has no weight gradient)
+  if ((p.kernel_variant & 2) == 0 || a.grad_image_weight != nullptr) {
     int rc = GS_OK;
 #define GS_WIDE_MMA_CASE(FPV) \
   case FPV: rc = heur ? launch_wide_mma<FPV, true>(p, a, rec, featP, tiles, st) \

@@ -38,13 +38,16 @@ struct XwideLayout {
   __host__ __device__ size_t total() const { return stage_bytes + kXwWarps * warp_bytes; }
 };
 
-template <bool HEUR>
+// WGT: the image weight W is differentiable too (gradient gw, forward W in wimg): one more channel whose feature is
+// always 1, so RG starts with W_final Gw and G . f_i gains + Gw (see raster_bwd_fast_kernel).
+template <bool HEUR, bool WGT = false>
 __global__ void __launch_bounds__(kXwWarps * 32)
 raster_bwd_xwide_kernel(const __grid_constant__ GsRasterParams p, const float4* __restrict__ rec,
                         const float* __restrict__ featP, const int32_t* __restrict__ ranges,
                         const int32_t* __restrict__ o2p, const float* __restrict__ image,
                         const float* __restrict__ grad_image, float* __restrict__ grad_pts,
-                        float* __restrict__ grad_feat, float* __restrict__ heuristic) {
+                        float* __restrict__ grad_feat, float* __restrict__ heuristic,
+                        const float* __restrict__ wimg, const float* __restrict__ gw) {
   constexpr int NG = 7 + (HEUR ? 2 : 0);             // geometry (+ heuristic) values
   constexpr int kThreads = kXwWarps * 32, kParts = 8 / kXwWarps;
   const int F = p.num_features;
@@ -77,7 +80,7 @@ raster_bwd_xwide_kernel(const __grid_constant__ GsRasterParams p, const float4* 
   const int gid = lane >> 2, tig = lane & 3;
 
   float* my_G = s_G + lane * GS;
-  float W = inb ? 0.f : 1.f, RG = 0.f;
+  float W = inb ? 0.f : 1.f, RG = 0.f, Gw = 0.f;
   {
     const int64_t pix = (int64_t)py * p.image_width + px;   // 64 bit: a 4K image of 256 channels has 2.1 G elements
 #pragma unroll 4
@@ -86,6 +89,10 @@ raster_bwd_xwide_kernel(const __grid_constant__ GsRasterParams p, const float4* 
       const float g = ok ? grad_image[pix * F + c] : 0.f;
       RG = fmaf(ok ? image[pix * F + c] : 0.f, g, RG);
       my_G[c] = g;
+    }
+    if constexpr (WGT) {
+      Gw = inb ? gw[pix] : 0.f;
+      RG = fmaf(inb ? wimg[pix] : 0.f, Gw, RG);
     }
   }
   __syncwarp();
@@ -215,7 +222,8 @@ raster_bwd_xwide_kernel(const __grid_constant__ GsRasterParams p, const float4* 
             fG0 = fmaf(f4.x, g4.x, fG0); fG1 = fmaf(f4.y, g4.y, fG1);
             fG2 = fmaf(f4.z, g4.z, fG2); fG3 = fmaf(f4.w, g4.w, fG3);
           }
-          const float fG = (fG0 + fG1) + (fG2 + fG3);
+          float fG = (fG0 + fG1) + (fG2 + fG3);
+          if constexpr (WGT) fG += Gw;
           RG = fmaf(-fG, wl, RG);
           const float ag = fmaf(fG, Ti, -RG * rinv);
           const float aag = a0 * ag;
@@ -247,16 +255,18 @@ raster_bwd_xwide_kernel(const __grid_constant__ GsRasterParams p, const float4* 
   if (ns > 0) flush_group();
 }
 
-template <bool HEUR>
+template <bool HEUR, bool WGT>
 static int launch_xwide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP,
                         cudaStream_t st) {
   const size_t smem = XwideLayout(p.num_features).total();
   const int tiles = tiles_wide(p) * tiles_high(p);
   // per launch: the attribute belongs to the (function, device) pair and the call costs about a microsecond
-  GS_CUDA(cudaFuncSetAttribute(raster_bwd_xwide_kernel<HEUR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  raster_bwd_xwide_kernel<HEUR><<<tiles * (8 / kXwWarps), kXwWarps * 32, smem, st>>>(
+  GS_CUDA(cudaFuncSetAttribute(raster_bwd_xwide_kernel<HEUR, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)smem));
+  raster_bwd_xwide_kernel<HEUR, WGT><<<tiles * (8 / kXwWarps), kXwWarps * 32, smem, st>>>(
       p, rec, featP, a.tile_ranges, a.overlap_to_point, (const float*)a.image_in, (const float*)a.grad_image,
-      (float*)a.grad_gaussians, (float*)a.grad_features, HEUR ? (float*)a.point_heuristic : nullptr);
+      (float*)a.grad_gaussians, (float*)a.grad_features, HEUR ? (float*)a.point_heuristic : nullptr,
+      (const float*)a.image_weight, (const float*)a.grad_image_weight);
   GS_LAUNCH_CHECK();
   return GS_OK;
 }
@@ -264,7 +274,9 @@ static int launch_xwide(const GsRasterParams& p, const RasterArgs& a, const floa
 int raster_bwd_xwide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP,
                      cudaStream_t st) {
   const bool heur = p.compute_point_heuristic && a.point_heuristic != nullptr;
-  return heur ? launch_xwide<true>(p, a, rec, featP, st) : launch_xwide<false>(p, a, rec, featP, st);
+  if (a.grad_image_weight != nullptr)
+    return heur ? launch_xwide<true, true>(p, a, rec, featP, st) : launch_xwide<false, true>(p, a, rec, featP, st);
+  return heur ? launch_xwide<true, false>(p, a, rec, featP, st) : launch_xwide<false, false>(p, a, rec, featP, st);
 }
 
 }  // namespace gs

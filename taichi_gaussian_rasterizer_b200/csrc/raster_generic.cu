@@ -124,13 +124,16 @@ __global__ void __launch_bounds__(NT) raster_fwd_generic_kernel(const __grid_con
   }
 }
 
-template <typename T, int MAXF, bool AA, int NT>
+// WGT: the image weight W = sum_i w_i is differentiable too (gradient gw, forward W in wimg).  W is the blend of a
+// constant feature 1: its remaining part Rw starts at W_final, Rw -= w per hit, and dL/dalpha gains (T - Rw / (1 - alpha)) Gw.
+template <typename T, int MAXF, bool AA, int NT, bool WGT = false>
 __global__ void __launch_bounds__(NT) raster_bwd_generic_kernel(const __grid_constant__ GsRasterParams p, int batch,
                                           const T* __restrict__ pts, const T* __restrict__ feat,
                                           const int32_t* __restrict__ ranges, const int32_t* __restrict__ o2p,
                                           const T* __restrict__ image, const T* __restrict__ grad_image,
                                           T* __restrict__ grad_pts, T* __restrict__ grad_feat,
-                                          T* __restrict__ heuristic) {
+                                          T* __restrict__ heuristic, const T* __restrict__ wimg,
+                                          const T* __restrict__ gw) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int ts = p.tile_size, F = p.num_features, B = batch;
   T* s_pts = reinterpret_cast<T*>(smem_raw);  // B*7
@@ -151,7 +154,7 @@ __global__ void __launch_bounds__(NT) raster_bwd_generic_kernel(const __grid_con
   const bool hg = p.compute_point_heuristic && heuristic != nullptr;
 
   T R[MAXF], Gp[MAXF];
-  T W = T(1);
+  T W = T(1), Rw = T(0), Gw = T(0);
 #pragma unroll
   for (int c = 0; c < MAXF; ++c) { R[c] = T(0); Gp[c] = T(0); }
   if (inb) {
@@ -159,6 +162,7 @@ __global__ void __launch_bounds__(NT) raster_bwd_generic_kernel(const __grid_con
 #pragma unroll
     for (int c = 0; c < MAXF; ++c)
       if (c < F) { R[c] = image[pix * F + c]; Gp[c] = grad_image[pix * F + c]; }
+    if constexpr (WGT) { Rw = wimg[pix]; Gw = gw[pix]; }
     W = T(0);
   }
 
@@ -205,6 +209,10 @@ __global__ void __launch_bounds__(NT) raster_bwd_generic_kernel(const __grid_con
             alpha_grad += diff * Gp[c];
             gf[c] = weight * Gp[c];
           }
+        if constexpr (WGT) {
+          Rw -= weight;
+          alpha_grad += (Ti - Rw / (T(1) - alpha)) * Gw;
+        }
         const T aag = g.alpha * alpha_grad;
         gp[0] = aag * d.dmx; gp[1] = aag * d.dmy;
         gp[2] = aag * d.dax; gp[3] = aag * d.day;
@@ -263,17 +271,18 @@ static int launch_fwd(const GsRasterParams& p, const RasterArgs& a, cudaStream_t
   return GS_OK;
 }
 
-template <typename T, int MAXF, bool AA, int NT>
+template <typename T, int MAXF, bool AA, int NT, bool WGT>
 static int launch_bwd(const GsRasterParams& p, const RasterArgs& a, cudaStream_t st) {
   const int A = p.tile_size * p.tile_size;
   const int B = A < 256 ? A : 256;
   const size_t smem = (size_t)B * ((7 + p.num_features) * 2 + 2) * sizeof(T) + (size_t)B * sizeof(int);
-  auto kern = raster_bwd_generic_kernel<T, MAXF, AA, NT>;
+  auto kern = raster_bwd_generic_kernel<T, MAXF, AA, NT, WGT>;
   if (smem > 48 * 1024) GS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int tiles = tiles_wide(p) * tiles_high(p);
   kern<<<tiles, A, smem, st>>>(p, B, (const T*)a.gaussians2d, (const T*)a.features, a.tile_ranges, a.overlap_to_point,
                                (const T*)a.image_in, (const T*)a.grad_image, (T*)a.grad_gaussians,
-                               (T*)a.grad_features, (T*)a.point_heuristic);
+                               (T*)a.grad_features, (T*)a.point_heuristic, (const T*)a.image_weight,
+                               (const T*)a.grad_image_weight);
   GS_LAUNCH_CHECK();
   return GS_OK;
 }
@@ -293,7 +302,9 @@ static int bwd_modes(const GsRasterParams& p, const RasterArgs& a, cudaStream_t 
     return p.antialias ? launch_fwd<T, MAXF, true, kQuantileBwd, NT>(p, a, st)
                        : launch_fwd<T, MAXF, false, kQuantileBwd, NT>(p, a, st);
   }
-  return p.antialias ? launch_bwd<T, MAXF, true, NT>(p, a, st) : launch_bwd<T, MAXF, false, NT>(p, a, st);
+  if (a.grad_image_weight != nullptr)
+    return p.antialias ? launch_bwd<T, MAXF, true, NT, true>(p, a, st) : launch_bwd<T, MAXF, false, NT, true>(p, a, st);
+  return p.antialias ? launch_bwd<T, MAXF, true, NT, false>(p, a, st) : launch_bwd<T, MAXF, false, NT, false>(p, a, st);
 }
 
 int raster_fwd_generic(const GsRasterParams& p, const RasterArgs& a, cudaStream_t st) {

@@ -47,6 +47,12 @@ class RasterConfig:
   compute_point_heuristic: bool = False  # split / prune statistics (backward)
   compute_visibility: bool = False       # per gaussian sum of blend weights (forward)
 
+  # (extension) image_weight is a differentiable output: its gradient reaches the gaussians and the heuristics as
+  # that of one more feature channel of ones would (background compositing, mask losses, depth / (W + eps)).  Off
+  # by default because it changes the gradient of code that already uses image_weight.  Alpha blending only: in
+  # quantile mode image_weight is W > 0 and stays non-differentiable.
+  differentiable_weight: bool = False
+
 
 def check_packed3d(packed_gaussians: torch.Tensor):
   assert len(packed_gaussians.shape) == 2 and packed_gaussians.shape[1] == 11, \

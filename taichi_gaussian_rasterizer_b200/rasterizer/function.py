@@ -4,6 +4,7 @@ Operator surface of taichi_splatting/rasterizer/function.py: ``rasterize_with_ti
 ``rasterize`` (:129-161) and ``RasterOut`` (:18-23), same autograd conventions (:41-91): image is
 differentiable w.r.t. gaussians2d and features; image_weight, visibility and point_heuristic are
 not; point_heuristic is returned zero-filled by forward and filled in place by backward.
+Extension: with ``RasterConfig.differentiable_weight`` (alpha blending only) image_weight is differentiable too.
 The kernels are csrc/raster_fast_*.cu (f32 / blending / tile 16) and csrc/raster_generic.cu.
 
 Two knobs the reference does not have (module level, defaults give reference parity):
@@ -91,14 +92,18 @@ class _RasterFunction(torch.autograd.Function):
     ctx.tile_overlap_ranges = tile_overlap_ranges
     ctx.point_heuristic = point_heuristic
     ctx.config = config
-    ctx.mark_non_differentiable(image_alpha, visibility, point_heuristic)
+    if config.differentiable_weight and config.use_alpha_blending:
+      ctx.mark_non_differentiable(visibility, point_heuristic)
+      ctx.save_for_backward(gaussians, features, image_feature, image_alpha)
+    else:
+      ctx.mark_non_differentiable(image_alpha, visibility, point_heuristic)
+      ctx.save_for_backward(gaussians, features, image_feature)
     ctx.set_materialize_grads(False)   # no zero fills for the non-differentiable outputs' gradients
-    ctx.save_for_backward(gaussians, features, image_feature)
     return image_feature, image_alpha, point_heuristic, visibility
 
   @staticmethod
   def backward(ctx, grad_image_feature, grad_alpha, grad_point_heuristic, grad_visibility):
-    gaussians, features, image_feature = ctx.saved_tensors
+    gaussians, features, image_feature = ctx.saved_tensors[:3]
     need_g, need_f = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
     if grad_image_feature is None:
       grad_image_feature = torch.zeros_like(image_feature)
@@ -109,10 +114,17 @@ class _RasterFunction(torch.autograd.Function):
     params.features_requires_grad = int(need_f)
     params.workspace_holds_packed = 1
     heur = ctx.point_heuristic if ctx.config.compute_point_heuristic else None
-    N.call("gs_raster_bwd", ctypes.byref(params), N.ptr(gaussians), N.ptr(features), N.ptr(ctx.tile_overlap_ranges),
-      N.ptr(ctx.overlap_to_point), N.ptr(image_feature), N.ptr(grad_image_feature.contiguous()),
-      N.ptr(grad_gaussians), N.ptr(grad_features), N.ptr(heur), N.ptr(ctx.workspace),
-      ctypes.c_size_t(ctx.workspace.numel()), N.stream_ptr(gaussians.device))
+    if grad_alpha is None:
+      N.call("gs_raster_bwd", ctypes.byref(params), N.ptr(gaussians), N.ptr(features), N.ptr(ctx.tile_overlap_ranges),
+        N.ptr(ctx.overlap_to_point), N.ptr(image_feature), N.ptr(grad_image_feature.contiguous()),
+        N.ptr(grad_gaussians), N.ptr(grad_features), N.ptr(heur), N.ptr(ctx.workspace),
+        ctypes.c_size_t(ctx.workspace.numel()), N.stream_ptr(gaussians.device))
+    else:   # differentiable_weight: image_alpha was saved as the fourth tensor
+      N.call("gs_raster_bwd_with_weight", ctypes.byref(params), N.ptr(gaussians), N.ptr(features),
+        N.ptr(ctx.tile_overlap_ranges), N.ptr(ctx.overlap_to_point), N.ptr(image_feature),
+        N.ptr(grad_image_feature.contiguous()), N.ptr(ctx.saved_tensors[3]), N.ptr(grad_alpha.contiguous()),
+        N.ptr(grad_gaussians), N.ptr(grad_features), N.ptr(heur), N.ptr(ctx.workspace),
+        ctypes.c_size_t(ctx.workspace.numel()), N.stream_ptr(gaussians.device))
     return grad_gaussians, grad_features, None, None, None, None
 
 
@@ -133,7 +145,8 @@ def rasterize_with_tiles(gaussians2d: torch.Tensor, features: torch.Tensor,
       config: RasterConfig
 
   Returns:
-      RasterOut(image (H, W, F), image_weight (H, W), point_heuristic (N, 2), visibility (N,))
+      RasterOut(image (H, W, F), image_weight (H, W), point_heuristic (N, 2), visibility (N,));
+      image_weight is differentiable when config.differentiable_weight is set (alpha blending only)
   """
   assert gaussians2d.ndim == 2 and gaussians2d.shape[1] == 7, f"gaussians2d must be Nx7, got {gaussians2d.shape}"
   N.require_cuda(gaussians2d, features, overlap_to_point, tile_overlap_ranges)

@@ -280,7 +280,7 @@ def _median_depth(gaussians2d, depths, overlap_to_point, ranges, camera_params, 
   goes to the depth of the gaussian it selected; the selection itself is piecewise constant, so the packed 2D
   gaussians get no gradient and are detached) — the reference's quantile mode is forward only (SURVEY Q7, 8f rank 3)."""
   quantile = replace(config, use_alpha_blending=False, saturate_threshold=0.5,
-                     compute_visibility=False, compute_point_heuristic=False)
+                     compute_visibility=False, compute_point_heuristic=False, differentiable_weight=False)
   raster = rasterize_with_tiles(gaussians2d.detach(), depths, tile_overlap_ranges=ranges,
                                 overlap_to_point=overlap_to_point, image_size=camera_params.image_size,
                                 config=quantile)

@@ -30,7 +30,7 @@ class Rendering:
   """
   # pixel space
   image: torch.Tensor                              # (H, W, C)
-  image_weight: torch.Tensor                       # (H, W) accumulated alpha
+  image_weight: torch.Tensor                       # (H, W) accumulated alpha (differentiable with RasterConfig.differentiable_weight)
   depth: Optional[torch.Tensor] = None             # (H, W)
   depth_var: Optional[torch.Tensor] = None         # (H, W)
   median_depth: Optional[torch.Tensor] = None      # (H, W)
