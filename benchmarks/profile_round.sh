@@ -17,7 +17,7 @@ timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 1500 --
 timeout 600 ncu --set full --clock-control none --import-source on -k regex:'raster_.wd_fast' -s 6 -c 2 -f -o $OUT/prof_raster_$TAG $SMALL > $OUT/ncu_raster_$TAG.log 2>&1; echo "raster capture rc=$?"
 timeout 900 ncu --set full --clock-control none --import-source on -k regex:'project_|sh_|onesweep|tile_query|full_cumsum|radix_hist|find_ranges|depth_keys|raster_pack|raster_bwd_moments|camera_position|gather_rows|raster_cull_mask' -s 96 -c 25 -f -o $OUT/prof_points_$TAG $SMALL > $OUT/ncu_points_$TAG.log 2>&1; echo "point kernel capture rc=$?"
 # BASELINE config 3 (6 M gaussians, visibility + heuristics): the VIS forward / HEUR backward instantiations
-C3="python benchmarks/variants.py --variants 0 --scene c3 --rounds 1 --iters 2"
+C3="python benchmarks/variants.py --scene c3 --rounds 1 --iters 2"
 $C3 > $OUT/c3_plain_$TAG.log 2>&1; echo "c3 plain rc=$?"
 timeout 600 ncu --set full --clock-control none --import-source on -k regex:'raster_fwd_fast|raster_bwd_fast' -s 4 -c 2 -f -o $OUT/prof_c3_$TAG $C3 > $OUT/ncu_c3_$TAG.log 2>&1; echo "c3 capture rc=$?"
 ls -la $OUT/*$TAG*

@@ -1,9 +1,9 @@
 #!/usr/bin/env python
-"""A/B timing of alternative kernel instantiations (GsRasterParams.kernel_variant, set_raster_options(kernel_variant=)):
-device time of gs_raster_fwd / gs_raster_bwd on one view of a BASELINE scene, per variant, plus the relative L2
-difference of every variant's outputs / gradients to variant 0 (they must agree).
+"""Device time of gs_raster_fwd / gs_raster_bwd on one view of a BASELINE scene (min / median over interleaved rounds).
+Alternative kernels are A/B-timed as two library builds, each loaded in its own process with _native.use_library
+(as benchmarks/fast_math_cost.py does).
 
-  python benchmarks/variants.py --variants 0,1 [--scene bench] [--stats] [--iters 20]
+  python benchmarks/variants.py [--scene bench] [--stats] [--iters 20]
 """
 import argparse
 import json
@@ -15,8 +15,8 @@ import torch
 ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
 
-from taichi_gaussian_rasterizer_b200 import (RasterConfig, _native, evaluate_sh_at, map_to_tiles, rasterize_with_tiles,  # noqa: E402
-                                             set_raster_options)
+from taichi_gaussian_rasterizer_b200 import (RasterConfig, _native, evaluate_sh_at, map_to_tiles,  # noqa: E402
+                                             rasterize_with_tiles)
 from taichi_gaussian_rasterizer_b200.perspective.projection import project_to_image  # noqa: E402
 from taichi_gaussian_rasterizer_b200.synthetic import baseline_scene  # noqa: E402
 from taichi_gaussian_rasterizer_b200.torch_lib.projection import ndc_depth  # noqa: E402
@@ -24,7 +24,6 @@ from taichi_gaussian_rasterizer_b200.torch_lib.projection import ndc_depth  # no
 
 def main():
   ap = argparse.ArgumentParser()
-  ap.add_argument("--variants", default="0,1")
   ap.add_argument("--scene", default="bench")
   ap.add_argument("--stats", action="store_true")
   ap.add_argument("--no-stats", action="store_true", help="visibility / heuristics off even if the scene asks for them")
@@ -48,7 +47,6 @@ def main():
   feats = feats.contiguous()
   torch.manual_seed(0)
   gi = torch.rand(cam.image_size[1], cam.image_size[0], feats.shape[1], device=dev) - 0.3
-  variants = [int(v) for v in args.variants.split(",")]
 
   def step():
     a, b = g2d.detach().clone().requires_grad_(True), feats.detach().clone().requires_grad_(True)
@@ -56,39 +54,21 @@ def main():
     (out.image * gi).sum().backward()
     return out, a.grad, b.grad
 
-  # results first (every variant against the first one), then interleaved timing rounds: boxes and clocks drift, so
-  # each round times every variant back to back and the minimum / median over the rounds are reported
-  base, rel = None, {}
-  for variant in variants:
-    set_raster_options(kernel_variant=variant)
-    for _ in range(3):
-      out, ga, gb = step()
-    res = dict(image=out.image, weight=out.image_weight, d_gaussians=ga, d_features=gb)
-    if stats:
-      res.update(visibility=out.visibility, heuristic=out.point_heuristic)
-    if base is None:
-      base = res
-    else:
-      rel[variant] = {k: ((v.double() - base[k].double()).norm() / base[k].double().norm()).item() for k, v in res.items()}
-  times = {v: {} for v in variants}
+  # boxes and clocks drift: the minimum / median over the rounds are reported
+  for _ in range(3):
+    step()
+  times = {}
   for _ in range(args.rounds):
-    for variant in variants:
-      set_raster_options(kernel_variant=variant)
+    step()
+    torch.cuda.synchronize()
+    timer = _native.set_stage_timer(_native.StageTimer())
+    for _ in range(args.iters):
       step()
-      torch.cuda.synchronize()
-      timer = _native.set_stage_timer(_native.StageTimer())
-      for _ in range(args.iters):
-        step()
-      for k, v in timer.summary().items():
-        times[variant].setdefault(k, []).append(v[1] / v[0])
-      _native.set_stage_timer(None)
-  for variant in variants:
-    ms = {k: {"min": round(min(v), 4), "median": round(sorted(v)[len(v) // 2], 4)} for k, v in times[variant].items()}
-    row = {"scene": args.scene, "variant": variant, "stats": stats, "K": int(o2p.shape[0]), "ms": ms}
-    if variant in rel:
-      row["rel_l2_vs_first"] = rel[variant]
-    print(json.dumps(row), flush=True)
-  set_raster_options(kernel_variant=0)
+    for k, v in timer.summary().items():
+      times.setdefault(k, []).append(v[1] / v[0])
+    _native.set_stage_timer(None)
+  ms = {k: {"min": round(min(v), 4), "median": round(sorted(v)[len(v) // 2], 4)} for k, v in times.items()}
+  print(json.dumps({"scene": args.scene, "stats": stats, "K": int(o2p.shape[0]), "ms": ms}), flush=True)
 
 
 if __name__ == "__main__":

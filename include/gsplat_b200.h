@@ -289,18 +289,7 @@ typedef struct GsRasterParams {
   int32_t workspace_holds_packed;    /* bwd: the workspace is untouched since a gs_raster_fwd call made with the same
                                         gaussians / features AND a requires_grad flag set (fwd then packs the
                                         backward records too); 0 = repack */
-  int32_t kernel_variant;            /* 0 = the shipped kernels; bits select alternative instantiations kept for A/B
-                                        timing (benchmarks/variants.py), all tested to the same tolerances
-                                        (tests/test_gpu_rasterizer.py test_kernel_variants_agree): bit 0 = narrow backward
-                                        reduces every survivor alone (default: pairs), bit 1 = wide backward reduces the
-                                        feature gradient with warp butterflies (default: mma.sync product), bit 2 = the
-                                        rasterizer kernels launch at the stream's priority (default: the lowest, so that a
-                                        caller's high-priority streams put every other kernel first), bits 3-4 = warps per
-                                        CTA of the wide backward: 0 -> two (default), 1 -> eight, 2 -> four, 3 -> one.
-                                        gs_raster_bwd_with_weight with a weight gradient ignores bits 0, 1, 3 and 4:
-                                        its narrow backward reduces every survivor alone, its wide one is the
-                                        shipped two-warp tensor-core kernel (no other weight-gradient instantiation
-                                        exists) */
+  int32_t kernel_variant;            /* reserved, must be 0 (GS_ERR_INVALID otherwise) */
   int64_t num_points;                /* V */
   int64_t num_overlaps;              /* K */
   double clamp_max_alpha, alpha_threshold, saturate_threshold;
@@ -334,8 +323,7 @@ int gs_raster_bwd(const GsRasterParams* p, const void* gaussians2d, const void* 
  * grad_gaussians and point_heuristic exactly as that of one more channel of ones would (grad_features keeps F
  * columns).  grad_image_weight NULL: the same call as gs_raster_bwd, the same kernels.  Quantile mode
  * (use_alpha_blending = 0): the weight is W > 0, piecewise constant, and grad_image_weight is ignored.  With a weight
- * gradient the narrow backward (F <= 7) reduces every survivor alone (faster there than in pairs) and the wide one
- * runs the shipped tensor-core kernel: kernel_variant bits 0, 1, 3 and 4 do not apply.
+ * gradient the narrow backward (F <= 7) reduces every survivor alone (faster there than in pairs).
  * Extra cost per backward row: DESIGN.md §3. */
 int gs_raster_bwd_with_weight(const GsRasterParams* p, const void* gaussians2d, const void* features,
                               const int32_t* tile_ranges, const int32_t* overlap_to_point, const void* image,

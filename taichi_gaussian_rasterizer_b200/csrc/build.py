@@ -20,7 +20,7 @@ OUT = PKG / "libgsplat_b200.so"
 OBJ = ROOT / "build" / "obj"
 
 SOURCES = ["api.cu", "geom_kernels.cu", "point_kernels.cu", "scan_sort.cu", "raster_api.cu",
-           "raster_generic.cu", "raster_fast_fwd.cu", "raster_fast_bwd.cu", "raster_fast_bwd_wide.cu", "raster_fast_xwide.cu",
+           "raster_generic.cu", "raster_fast_fwd.cu", "raster_fast_bwd.cu", "raster_fast_bwd_wide.cu",
            "optim_kernels.cu", "morton.cu", "multimem_reduce.cu"]
 HEADERS = ["common.cuh", "geom_math.cuh", "lookback.cuh", "raster.cuh", "raster_math.cuh", "raster_fast.cuh",
            "../../include/gsplat_b200.h", "../../include/gs_numeric.h"]

@@ -1,6 +1,7 @@
 // raster.cuh — internal interface between the rasterizer entry points (raster_api.cu) and the
 // kernel families: raster_generic.cu (every dtype / mode, fidelity first; also the f64 gradcheck
-// path) and raster_fast_fwd.cu / raster_fast_bwd.cu (f32, alpha blending, tile 16: the measured path).
+// path) and raster_fast_fwd.cu / raster_fast_bwd.cu / raster_fast_bwd_wide.cu (f32, alpha blending, tile 16: the
+// measured path).
 #pragma once
 
 #include "common.cuh"

@@ -15,6 +15,10 @@ static int check_raster(const GsRasterParams* p, const char* who) {
     set_error("%s: tile_size must be 8, 16 or 32, got %d", who, p->tile_size);
     return GS_ERR_UNSUPPORTED;
   }
+  if (p->kernel_variant != 0) {
+    set_error("%s: kernel_variant is reserved and must be 0, got %d", who, p->kernel_variant);
+    return GS_ERR_INVALID;
+  }
   const int sx = p->pixel_stride_x, sy = p->pixel_stride_y;
   if (sx <= 0 || sy <= 0 || (p->tile_size * p->tile_size) / (sx * sy) < 32) {  // rasterizer/backward.py:33-34
     set_error("%s: pixel_stride (%d, %d) and tile_size %d must allow at least one warp sized (32) tile", who, sx, sy,

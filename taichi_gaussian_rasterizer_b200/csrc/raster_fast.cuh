@@ -12,7 +12,7 @@ constexpr int kFastTileArea = kFastTile * kFastTile;
 // padded feature row length used by the fast kernels for a given F (0 = unsupported)
 inline int fast_feature_pad(int F) { return F <= 4 ? 4 : F <= 8 ? 8 : F <= 16 ? 16 : F <= 36 ? 36 : F <= 64 ? 64 : 0; }
 
-// Extra-wide features (65..256 channels, raster_fast_xwide.cu): rows of xwide_row(F) floats, 64-channel slices.
+// Extra-wide features (65..256 channels): rows of xwide_row(F) floats, 64-channel slices.
 constexpr int kXwideSlice = 64;
 constexpr int kXwideMaxFeatures = 256;
 inline bool xwide_features(int F) { return F > 64 && F <= kXwideMaxFeatures; }
@@ -171,9 +171,7 @@ int raster_fast_pack(const GsRasterParams& p, const RasterArgs& a, bool forward,
 // cull masks of every tile-list entry against the eight 8x4 pixel blocks of its tile (needs the forward records)
 int raster_cull_mask(const GsRasterParams& p, const RasterArgs& a, cudaStream_t st);
 
-// raster_fast_bwd_wide.cu: backward for 8..64 feature channels (one pixel per lane, image gradient in registers)
+// raster_fast_bwd_wide.cu: backward for 8..256 feature channels (one pixel per lane, tensor-core feature gradient)
 int raster_bwd_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP, cudaStream_t st);
-// raster_fast_xwide.cu: backward for 65..256 feature channels (image gradient in shared memory)
-int raster_bwd_xwide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP, cudaStream_t st);
 
 }  // namespace gs

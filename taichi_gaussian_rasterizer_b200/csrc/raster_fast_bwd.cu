@@ -362,37 +362,24 @@ static int launch_bwd_fast(const GsRasterParams& p, const RasterArgs& a, const f
   const int tiles = tiles_wide(p) * tiles_high(p);
   const bool heur = p.compute_point_heuristic && a.point_heuristic != nullptr;
   const unsigned char* cmask = (const unsigned char*)a.workspace + fast_layout(p).off_mask;
-  // kernel_variant (benchmark A/B switch, 0 in production): bit 0 = reduce every survivor on its own
-  const bool pair = (p.kernel_variant & 1) == 0;
   const float3 kf = make_float3((float)p.alpha_threshold, (float)p.clamp_max_alpha, (float)p.saturate_threshold);
-  // kernel_variant bit 2 (A/B): launch at the stream's own priority instead of the lowest one (launch_background)
-  const bool background = (p.kernel_variant & 4) == 0;
   const float* wimg = (const float*)a.image_weight;
   const float* gw = (const float*)a.grad_image_weight;
-#define GS_BWD_LAUNCH(HEURV, PAIRV, AAV, WGTV)                                                                   \
-  do {                                                                                                           \
-    if (background)                                                                                              \
-      GS_CUDA(launch_background(raster_bwd_fast_kernel<F, FP, HEURV, PAIRV, AAV, WGTV>, dim3(tiles * 2),         \
-                                dim3(32), 0, st, p, rec, featP, a.tile_ranges, a.overlap_to_point,               \
-                                (const float*)a.image_in, (const float*)a.grad_image, (float*)a.grad_gaussians,  \
-                                (float*)a.grad_features, heur ? (float*)a.point_heuristic : nullptr, cmask, kf,  \
-                                wimg, gw));                                                                      \
-    else                                                                                                         \
-      raster_bwd_fast_kernel<F, FP, HEURV, PAIRV, AAV, WGTV><<<tiles * 2, 32, 0, st>>>(                          \
-          p, rec, featP, a.tile_ranges, a.overlap_to_point, (const float*)a.image_in, (const float*)a.grad_image,\
-          (float*)a.grad_gaussians, (float*)a.grad_features, heur ? (float*)a.point_heuristic : nullptr, cmask,  \
-          kf, wimg, gw);                                                                                         \
-  } while (0)
-  if (gw != nullptr) {
-    // with the weight gradient every survivor is reduced alone: the paired kernel spills 84 B (F = 3) to 296 B (F = 7,
-    // heuristics) under its 64-register cap and measured slower (B200, bench scene: F = 3 1.39 ms paired, 1.37 single;
-    // F = 7 2.60 / 1.84 ms; benchmarks/weight_gradient.py)
-    if (p.antialias) { if (heur) GS_BWD_LAUNCH(true, false, true, true); else GS_BWD_LAUNCH(false, false, true, true); }
-    else if (heur) GS_BWD_LAUNCH(true, false, false, true);
-    else GS_BWD_LAUNCH(false, false, false, true);
-  } else if (p.antialias) { if (heur) GS_BWD_LAUNCH(true, false, true, false); else GS_BWD_LAUNCH(false, false, true, false); }
-  else if (heur) { if (pair) GS_BWD_LAUNCH(true, true, false, false); else GS_BWD_LAUNCH(true, false, false, false); }
-  else { if (pair) GS_BWD_LAUNCH(false, true, false, false); else GS_BWD_LAUNCH(false, false, false, false); }
+  // Survivors are reduced in pairs (1.352 against 1.381 ms on the bench workload), except with antialiasing or the
+  // weight gradient: there the paired kernel spills 84 B (F = 3) to 296 B (F = 7, heuristics) under its 64-register cap
+  // and measured slower (B200, bench scene: F = 3 1.39 ms paired, 1.37 single; F = 7 2.60 / 1.84 ms;
+  // benchmarks/weight_gradient.py).
+#define GS_BWD_LAUNCH(HEURV, AAV, WGTV)                                                                                  \
+  GS_CUDA(launch_background(raster_bwd_fast_kernel<F, FP, HEURV, !(AAV || WGTV), AAV, WGTV>, dim3(tiles * 2), dim3(32), \
+                            0, st, p, rec, featP, a.tile_ranges, a.overlap_to_point, (const float*)a.image_in,       \
+                            (const float*)a.grad_image, (float*)a.grad_gaussians, (float*)a.grad_features,           \
+                            heur ? (float*)a.point_heuristic : nullptr, cmask, kf, wimg, gw))
+#define GS_BWD_HEUR(AAV, WGTV) \
+  do { if (heur) GS_BWD_LAUNCH(true, AAV, WGTV); else GS_BWD_LAUNCH(false, AAV, WGTV); } while (0)
+  if (gw != nullptr) { if (p.antialias) GS_BWD_HEUR(true, true); else GS_BWD_HEUR(false, true); }
+  else if (p.antialias) GS_BWD_HEUR(true, false);
+  else GS_BWD_HEUR(false, false);
+#undef GS_BWD_HEUR
 #undef GS_BWD_LAUNCH
   GS_LAUNCH_CHECK();
   if (!p.antialias && p.points_requires_grad && a.grad_gaussians != nullptr && p.num_points > 0) {
@@ -402,8 +389,6 @@ static int launch_bwd_fast(const GsRasterParams& p, const RasterArgs& a, const f
   }
   return GS_OK;
 }
-
-bool raster_bwd_fast_supported(const GsRasterParams& p) { return raster_fast_supported(p) && p.num_features <= 7; }
 
 int raster_bwd_fast(const GsRasterParams& p, const RasterArgs& a, cudaStream_t st) {
   if (!p.workspace_holds_packed) {  // otherwise gs_raster_fwd (called with the requires_grad flags) left both there
@@ -417,9 +402,7 @@ int raster_bwd_fast(const GsRasterParams& p, const RasterArgs& a, cudaStream_t s
   const FastLayout L = fast_layout(p);
   unsigned char* ws = (unsigned char*)a.workspace;
   const float* featP = fast_feature_rows(p, a);
-  if (xwide_features(p.num_features))   // 65..256 channels: the image gradient in shared memory
-    return raster_bwd_xwide(p, a, (const float4*)(ws + L.off_recB), featP, st);
-  if (p.num_features > 7)   // 8..64 channels: one pixel per lane, its own records
+  if (p.num_features > 7)   // 8..256 channels: one pixel per lane, its own records
     return raster_bwd_wide(p, a, (const float4*)(ws + L.off_recB), featP, st);
   const float4* rec = (const float4*)(ws + (p.antialias ? L.off_recB : L.off_recF));   // the forward's records
   switch (p.num_features) {

@@ -415,19 +415,10 @@ int raster_fwd_fast(const GsRasterParams& p, const RasterArgs& a, cudaStream_t s
     GS_LAUNCH_CHECK();
     return GS_OK;
   }
-  // kernel_variant bit 2 (A/B): launch at the stream's own priority instead of the lowest one (launch_background)
-  const bool background = (p.kernel_variant & 4) == 0;
 #define GS_FWD_LAUNCH1(FPV, VISV, BATCHV, FOURTHV)                                                                 \
-  do {                                                                                                             \
-    if (background)                                                                                                \
-      GS_CUDA(launch_background(raster_fwd_fast_kernel<FPV, VISV, BATCHV, FOURTHV, false>, dim3(tiles),            \
-                                dim3(kFwdThreads), 0, st, p, rec, featP, a.tile_ranges, a.overlap_to_point,        \
-                                (float*)a.image, (float*)a.image_alpha, (float*)a.visibility, cmask));             \
-    else                                                                                                           \
-      raster_fwd_fast_kernel<FPV, VISV, BATCHV, FOURTHV, false><<<tiles, kFwdThreads, 0, st>>>(                    \
-          p, rec, featP, a.tile_ranges, a.overlap_to_point, (float*)a.image, (float*)a.image_alpha,                \
-          (float*)a.visibility, cmask);                                                                            \
-  } while (0)
+  GS_CUDA(launch_background(raster_fwd_fast_kernel<FPV, VISV, BATCHV, FOURTHV, false>, dim3(tiles), dim3(kFwdThreads), \
+                            0, st, p, rec, featP, a.tile_ranges, a.overlap_to_point, (float*)a.image,                \
+                            (float*)a.image_alpha, (float*)a.visibility, cmask))
 #define GS_FWD_LAUNCH(FPV, VISV, BATCHV)                                                                           \
   do {                                                                                                             \
     if (FPV == 4 && p.num_features < 4) GS_FWD_LAUNCH1(FPV, VISV, BATCHV, false);                                  \

@@ -31,18 +31,15 @@ RasterOut = NamedTuple('RasterOut', [
   ('visibility', Optional[torch.Tensor])
 ])
 
-_options = dict(emulate_stale_tail=True, forward_exit_transmittance=0.0, kernel_variant=0)
+_options = dict(emulate_stale_tail=True, forward_exit_transmittance=0.0)
 
 
 def set_raster_options(emulate_stale_tail: Optional[bool] = None,
-                       forward_exit_transmittance: Optional[float] = None,
-                       kernel_variant: Optional[int] = None):
+                       forward_exit_transmittance: Optional[float] = None):
   if emulate_stale_tail is not None:
     _options['emulate_stale_tail'] = bool(emulate_stale_tail)
   if forward_exit_transmittance is not None:
     _options['forward_exit_transmittance'] = float(forward_exit_transmittance)
-  if kernel_variant is not None:   # A/B timing of alternative kernel instantiations (same results); 0 = shipped
-    _options['kernel_variant'] = int(kernel_variant)
   return dict(_options)
 
 
@@ -54,7 +51,7 @@ def _raster_params(config: RasterConfig, dtype, image_size, F, V, K, pts_grad, f
     compute_point_heuristic=int(config.compute_point_heuristic), points_requires_grad=int(pts_grad),
     features_requires_grad=int(feat_grad), emulate_stale_tail=int(_options['emulate_stale_tail']),
     pixel_stride_x=config.pixel_stride[0], pixel_stride_y=config.pixel_stride[1], workspace_holds_packed=0,
-    kernel_variant=_options['kernel_variant'], num_points=V, num_overlaps=K, clamp_max_alpha=config.clamp_max_alpha,
+    kernel_variant=0, num_points=V, num_overlaps=K, clamp_max_alpha=config.clamp_max_alpha,
     alpha_threshold=config.alpha_threshold, saturate_threshold=config.saturate_threshold,
     forward_exit_transmittance=_options['forward_exit_transmittance'])
 

@@ -53,6 +53,13 @@ def test_invalid_arguments_return_errors_not_crashes():
                              pixel_stride_x=2, pixel_stride_y=2)
   rc = lib.gs_raster_fwd(ctypes.byref(p), None, None, None, None, None, None, None, None, ctypes.c_size_t(0), None)
   assert rc == -2 and b"tile_size" in lib.gs_last_error_string()
+  p = _native.GsRasterParams(dtype=0, image_width=16, image_height=16, tile_size=16, num_features=3,
+                             pixel_stride_x=1, pixel_stride_y=1, kernel_variant=1)
+  rc = lib.gs_raster_fwd(ctypes.byref(p), None, None, None, None, None, None, None, None, ctypes.c_size_t(0), None)
+  assert rc == -1 and b"kernel_variant" in lib.gs_last_error_string()
+  rc = lib.gs_raster_bwd(ctypes.byref(p), None, None, None, None, None, None, None, None, None, None,
+                         ctypes.c_size_t(0), None)
+  assert rc == -1 and b"kernel_variant" in lib.gs_last_error_string()
   rc = lib.gs_radix_sort_pairs(ctypes.c_int64(10), ctypes.c_int32(3), None, None, None, None, 0, 8, None,
                                ctypes.c_size_t(0), None)
   assert rc == -1
