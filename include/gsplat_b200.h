@@ -97,9 +97,8 @@ typedef struct GsSHParams {
                                     gs_sh_bwd write dense gradient rows without atomics.  0 = no assumption. */
   int64_t num_points;      /* M */
   int64_t num_indexes;     /* V */
-  int32_t accumulate_params; /* gs_sh_bwd: grad_params += instead of = (rows outside `indexes` untouched, no zero
-                                fill); needs indexes_sorted_unique, f32, K = 3, D in {4, 16}; fuses the optimizer-side
-                                gradient accumulation of a multi-view batch into the kernel.  0 = overwrite. */
+  int32_t accumulate_params; /* gs_sh_bwd_flush: 1 = add the sum to grad_params, 0 = overwrite the rows with it.
+                                gs_sh_bwd: reserved, must be 0 (GS_ERR_INVALID otherwise). */
   int32_t params_is_forward_output; /* gs_sh_bwd: the `params` argument holds the forward OUTPUT (V,K) instead of the
                                        coefficients — enough for grad_params (the coefficients only enter through the
                                        clamp mask, and v in (0,1) <=> clamp(v) in (0,1)) and 4KD bytes per gaussian

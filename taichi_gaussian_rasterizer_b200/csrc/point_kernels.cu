@@ -184,7 +184,7 @@ constexpr int kSHDenseBlock = 128;
 // FROM_OUT: `params` holds the forward OUTPUT (V, K) instead of the coefficients.  The coefficient gradient
 // g_k b_j needs the coefficients only for the clamp mask, and v in (0, 1) <=> clamp(v) in (0, 1): when no position /
 // camera gradient is asked for, the 4 K D byte row gather per gaussian (a third of the kernel's traffic) is skipped.
-template <int K, int D, bool FILL, bool ACC, bool FROM_OUT = false>
+template <int K, int D, bool FILL, bool FROM_OUT = false>
 __global__ void __launch_bounds__(kSHDenseBlock, 6)
 sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restrict__ params,
                     const float* __restrict__ positions, const int64_t* __restrict__ indexes,
@@ -278,12 +278,7 @@ sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restric
     const int q = t + m * kSHDenseBlock, r = q / R4, part = q - r * R4;
     if (q < nrows * R4) {
       float4* dst = reinterpret_cast<float4*>(grad_params + s_idx[r + 1] * RL) + part;
-      float4 v = s_row[r * S4 + part];
-      if (ACC) {  // accumulate into the caller's gradient buffer (multi-view batches)
-        const float4 o = *dst;
-        v.x += o.x; v.y += o.y; v.z += o.z; v.w += o.w;
-      }
-      *dst = v;
+      *dst = s_row[r * S4 + part];
     }
   }
 
@@ -792,22 +787,21 @@ int gs_sh_bwd(const GsSHParams* p, const void* params, const void* positions, co
               void* grad_camera_pos, void* stream) {
   int rc = check_sh(p, "gs_sh_bwd");
   if (rc != GS_OK) return rc;
+  if (p->accumulate_params != 0) {
+    set_error("gs_sh_bwd: accumulate_params is reserved and must be 0, got %d", p->accumulate_params);
+    return GS_ERR_INVALID;
+  }
   cudaStream_t st = (cudaStream_t)stream;
   const size_t es = p->dtype == GS_F32 ? 4 : 8;
   const bool dense = p->indexes_sorted_unique && p->dtype == GS_F32 && grad_params != nullptr && p->num_indexes > 0 &&
                      p->num_channels == 3 && (p->num_coeffs == 16 || p->num_coeffs == 4);
-  const bool acc = p->accumulate_params != 0;
   const bool from_out = p->params_is_forward_output != 0;
   if (from_out && (!dense || grad_positions || grad_camera_pos)) {
     set_error("gs_sh_bwd: params_is_forward_output needs the dense path and no position / camera gradient");
     return GS_ERR_UNSUPPORTED;
   }
-  if (acc && !dense) {
-    set_error("gs_sh_bwd: accumulate_params needs the dense path (indexes_sorted_unique, f32, K = 3, D = 4 or 16)");
-    return GS_ERR_UNSUPPORTED;
-  }
-  const bool fill = dense && !acc && 2 * p->num_indexes >= p->num_points;  // mostly visible: zero-fill the gaps in-kernel
-  if (grad_params && !fill && !acc)
+  const bool fill = dense && 2 * p->num_indexes >= p->num_points;  // mostly visible: zero-fill the gaps in-kernel
+  if (grad_params && !fill)
     GS_CUDA(cudaMemsetAsync(grad_params, 0, (size_t)p->num_points * p->num_channels * p->num_coeffs * es, st));
   if (grad_positions && !fill) GS_CUDA(cudaMemsetAsync(grad_positions, 0, (size_t)p->num_points * 3 * es, st));
   if (grad_camera_pos) GS_CUDA(cudaMemsetAsync(grad_camera_pos, 0, 3 * es, st));
@@ -815,16 +809,16 @@ int gs_sh_bwd(const GsSHParams* p, const void* params, const void* positions, co
   GS_CHECK_ARG(params && positions && indexes && camera_pos && grad_out, "gs_sh_bwd: null tensor");
   if (dense) {
     const unsigned blocks = (unsigned)ceil_div(p->num_indexes, kSHDenseBlock);
-#define GS_SH_DENSE_(DD, FILLV, ACCV, FROMV)                                                                      \
-    sh_bwd_dense_kernel<3, DD, FILLV, ACCV, FROMV><<<blocks, kSHDenseBlock, 0, st>>>(                            \
+#define GS_SH_DENSE_(DD, FILLV, FROMV)                                                                            \
+    sh_bwd_dense_kernel<3, DD, FILLV, FROMV><<<blocks, kSHDenseBlock, 0, st>>>(                                  \
         *p, (const float*)params, (const float*)positions, indexes, (const float*)camera_pos,                   \
         (const float*)grad_out, (float*)grad_params, (float*)grad_positions, (float*)grad_camera_pos)
-#define GS_SH_DENSE(DD, FILLV, ACCV) \
-    do { if (from_out) GS_SH_DENSE_(DD, FILLV, ACCV, true); else GS_SH_DENSE_(DD, FILLV, ACCV, false); } while (0)
+#define GS_SH_DENSE(DD, FILLV) \
+    do { if (from_out) GS_SH_DENSE_(DD, FILLV, true); else GS_SH_DENSE_(DD, FILLV, false); } while (0)
     if (p->num_coeffs == 16) {
-      if (acc) GS_SH_DENSE(16, false, true); else if (fill) GS_SH_DENSE(16, true, false); else GS_SH_DENSE(16, false, false);
+      if (fill) GS_SH_DENSE(16, true); else GS_SH_DENSE(16, false);
     } else {
-      if (acc) GS_SH_DENSE(4, false, true); else if (fill) GS_SH_DENSE(4, true, false); else GS_SH_DENSE(4, false, false);
+      if (fill) GS_SH_DENSE(4, true); else GS_SH_DENSE(4, false);
     }
 #undef GS_SH_DENSE
 #undef GS_SH_DENSE_

@@ -51,9 +51,9 @@ class GradientBucket:
       off += n
 
   def zero_(self):
-    """Zero the gradients.  Inside ``fused_accumulation(defer_sh=True)`` the SH coefficient slices are not touched:
-    their deferred state is marked clean and the batch's first flush overwrites them (no 4 K D bytes per gaussian of
-    zero fill, no read of the rows by that flush)."""
+    """Zero the gradients.  Inside ``fused_accumulation()`` the SH coefficient slices are not touched: their deferred
+    state is marked clean and the batch's first flush overwrites them (no 4 K D bytes per gaussian of zero fill, no read
+    of the rows by that flush).  Every view's SH coefficient gradient reaches those slices through that flush."""
     from . import grad_sinks
     assert self._early is None, "reduce_early() must be followed by all_reduce() before the bucket is zeroed"
     clean = [(p, grad_sinks.deferred_sh(p)) for p in self.params]
@@ -69,21 +69,21 @@ class GradientBucket:
       d.mark_clean()
 
   @contextmanager
-  def fused_accumulation(self, defer_sh: bool = True):
+  def fused_accumulation(self):
     """Inside this context the spherical-harmonics backward and the projection backward add their gradients straight
     into the bucket (in the kernel) instead of materialising dense tensors for autograd to add: per view that removes
     a read-modify-write pass over every gradient (576 MB of SH + 132 MB of geometry at 3 M gaussians) and the zero
     fill of the culled rows.  Results are the same sums; parameters the kernels cannot serve this way (other
     dtypes, features used without SH) keep the normal autograd accumulation.
 
-    ``defer_sh``: the SH coefficient gradient (N, 3, D) of the batch is formed ONCE, by ``flush()`` (called on exit and
-    by ``all_reduce``): each view only stages its masked colour gradient (N, 3) and the flush adds
+    The SH coefficient gradient (N, 3, 4 | 16, f32) of the batch is formed ONCE, by ``flush()`` (called on exit and by
+    ``all_reduce``): each view only stages its masked colour gradient (N, 3) and the flush adds
     sum_v staged_v (x) basis(position - camera_v) — one pass over the coefficient rows per batch (or per 16 views)
     instead of one read-modify-write pass per view (grad_sinks.DeferredSH).  Anything that reads the SH gradient
     inside the context (an optimizer step, say) must call ``flush()`` first."""
     from . import grad_sinks
     served = [p for p in self.params if p.is_cuda and p.grad is not None]
-    deferred = [p for p in served if defer_sh and p.dtype == torch.float32 and p.ndim == 3 and p.shape[1] == 3
+    deferred = [p for p in served if p.dtype == torch.float32 and p.ndim == 3 and p.shape[1] == 3
                 and p.shape[2] in (4, 16)]
     for p in served:
       grad_sinks.register_grad_sink(p, p.grad)
@@ -98,7 +98,7 @@ class GradientBucket:
         grad_sinks.unregister_grad_sink(p)
 
   def flush(self):
-    """Add the pending deferred SH gradients (fused_accumulation(defer_sh=True)) to the bucket."""
+    """Add the pending deferred SH gradients (fused_accumulation()) to the bucket."""
     from . import grad_sinks
     for p in self.params:
       d = grad_sinks.deferred_sh(p)

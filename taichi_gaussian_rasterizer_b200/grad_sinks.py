@@ -64,8 +64,10 @@ class DeferredSH:
     self._last_flush = None
 
   def staging_buffer(self):
-    """The buffer the next view should stage into, if the holder asked for a particular one (first held view only)."""
-    if self.hold and self.staging is not None and not self.pending:
+    """The buffer the next view should stage into, if the holder asked for a particular one (the one view that may
+    follow GradientBucket.reduce_early on the symmetric bucket)."""
+    if self.hold and self.staging is not None:
+      assert not self.pending, "reduce_early(): exactly one view may follow it (the held staging buffer is taken)"
       return self.staging
     return None
 

@@ -13,6 +13,7 @@ from beartype import beartype
 
 from . import _native as N
 from .grad_sinks import deferred_sh, grad_sink, register_grad_sink, unregister_grad_sink  # noqa: F401  (re-exported)
+from .grad_sinks import flush_sh_views
 
 
 def check_sh_degree(sh_features):
@@ -52,59 +53,47 @@ class _SHFunction(torch.autograd.Function):
   def backward(ctx, doutput):
     params, points, indexes, camera_pos, out = ctx.saved_tensors
     need = ctx.needs_input_grad
-    sink = grad_sink(params) if need[0] else None
     dense = ctx.sorted_unique and params.dtype == torch.float32 and params.shape[1] == 3 and params.shape[2] in (4, 16) \
       and indexes.shape[0] > 0
-    # only the coefficient gradient is wanted (render_gaussians detaches the positions): the kernel then takes the clamp
-    # mask from the forward output and never reads the coefficient rows
-    from_out = int(dense and need[0] and not need[1] and not need[3])
-    coeffs = out if from_out else params
-    deferred = deferred_sh(params) if (sink is not None and dense and from_out) else None
-    if ctx.count is not None:
-      # the visible count never reached the host (render_gaussians(..., overlap_capacity=)): the masked colour gradient
-      # is staged for the first count rows (gs_sh_bwd_stage_counted) and either joins the batch's deferred flush, or is
-      # turned into coefficient rows right here by a one-view flush (added to the sink, or a fresh dense gradient)
-      assert need[0] and not need[1] and not need[3], "counted SH backward: coefficient gradient only"
+    sink = grad_sink(params) if (need[0] and dense) else None
+    g_points = torch.empty_like(points) if need[1] else None
+    g_cam = torch.empty_like(camera_pos) if need[3] else None
+    if sink is not None or ctx.count is not None:
+      # the masked colour gradient is staged (the stage kernel reads only the forward output) and turned into
+      # coefficient rows by a flush: the batch's deferred one, a one-view flush added to the sink, or (counted path
+      # without a sink: render_gaussians(..., overlap_capacity=)) a one-view flush into a fresh dense gradient
+      if ctx.count is not None:
+        assert need[0] and not need[1] and not need[3], "counted SH backward: coefficient gradient only"
+      deferred = deferred_sh(params) if sink is not None else None
       staged = deferred.staging_buffer() if deferred is not None else None
       if staged is None:
         staged = torch.empty((params.shape[0], params.shape[1]), dtype=params.dtype, device=params.device)
       p = N.GsSHParams(ctx.p.dtype, ctx.p.num_channels, ctx.p.num_coeffs, 1, ctx.p.num_points, ctx.p.num_indexes, 1, 1)
-      N.call("gs_sh_bwd_stage_counted", ctypes.byref(p), N.ptr(out), N.ptr(indexes), N.ptr(doutput.contiguous()),
-             N.ptr(ctx.count), N.ptr(staged), N.stream_ptr(params.device))
+      if ctx.count is not None:
+        N.call("gs_sh_bwd_stage_counted", ctypes.byref(p), N.ptr(out), N.ptr(indexes), N.ptr(doutput.contiguous()),
+               N.ptr(ctx.count), N.ptr(staged), N.stream_ptr(params.device))
+      else:
+        N.call("gs_sh_bwd_stage", ctypes.byref(p), N.ptr(out), N.ptr(indexes), N.ptr(doutput.contiguous()),
+               N.ptr(staged), N.stream_ptr(params.device))
       cam = camera_pos.detach().contiguous()
+      g_params = None
       if deferred is not None:
         deferred.add(staged, cam, points.detach())
-        return None, None, None, None, None, None, None
-      from .grad_sinks import flush_sh_views
-      if sink is not None:
+      elif sink is not None:
         flush_sh_views(sink, points.detach(), [staged], [cam], overwrite=False)
-        return None, None, None, None, None, None, None
-      g_params = torch.empty_like(params)
-      flush_sh_views(g_params, points.detach(), [staged], [cam], overwrite=True)
-      return g_params, None, None, None, None, None, None
-    if deferred is not None:
-      # deferred accumulation (grad_sinks.DeferredSH): this view only stages its masked colour gradient, the batch's
-      # flush forms the coefficient rows once
-      staged = deferred.staging_buffer()
-      if staged is None:
-        staged = torch.empty((params.shape[0], params.shape[1]), dtype=params.dtype, device=params.device)
-      p = N.GsSHParams(ctx.p.dtype, ctx.p.num_channels, ctx.p.num_coeffs, 1, ctx.p.num_points, ctx.p.num_indexes, 1, 1)
-      N.call("gs_sh_bwd_stage", ctypes.byref(p), N.ptr(out), N.ptr(indexes), N.ptr(doutput.contiguous()), N.ptr(staged),
-             N.stream_ptr(params.device))
-      deferred.add(staged, camera_pos.detach().contiguous(), points.detach())
-      return None, None, None, None, None, None, None
-    if sink is not None and dense:
-      # fused accumulation: the kernel adds into the sink, autograd gets no gradient for `params`
-      p = N.GsSHParams(ctx.p.dtype, ctx.p.num_channels, ctx.p.num_coeffs, 1, ctx.p.num_points, ctx.p.num_indexes, 1,
-                       from_out)
-      g_points = torch.empty_like(points) if need[1] else None
-      g_cam = torch.empty_like(camera_pos) if need[3] else None
-      N.call("gs_sh_bwd", ctypes.byref(p), N.ptr(coeffs), N.ptr(points), N.ptr(indexes), N.ptr(camera_pos),
-             N.ptr(doutput.contiguous()), N.ptr(sink), N.ptr(g_points), N.ptr(g_cam), N.stream_ptr(params.device))
-      return None, g_points, None, g_cam, None, None, None
+      else:
+        g_params = torch.empty_like(params)
+        flush_sh_views(g_params, points.detach(), [staged], [cam], overwrite=True)
+      if g_points is not None or g_cam is not None:
+        # position / camera gradient (eager path only): the generic kernel, no coefficient rows
+        N.call("gs_sh_bwd", ctypes.byref(ctx.p), N.ptr(params), N.ptr(points), N.ptr(indexes), N.ptr(camera_pos),
+               N.ptr(doutput.contiguous()), N.ptr(None), N.ptr(g_points), N.ptr(g_cam), N.stream_ptr(params.device))
+      return g_params, g_points, None, g_cam, None, None, None
     g_params = torch.empty_like(params) if need[0] else None
-    g_points = torch.empty_like(points) if need[1] else None
-    g_cam = torch.empty_like(camera_pos) if need[3] else None
+    # only the coefficient gradient is wanted (render_gaussians detaches the positions): the kernel then takes the clamp
+    # mask from the forward output and never reads the coefficient rows
+    from_out = int(dense and need[0] and not need[1] and not need[3])
+    coeffs = out if from_out else params
     p = N.GsSHParams(ctx.p.dtype, ctx.p.num_channels, ctx.p.num_coeffs, ctx.p.indexes_sorted_unique, ctx.p.num_points,
                      ctx.p.num_indexes, 0, from_out)
     N.call("gs_sh_bwd", ctypes.byref(p), N.ptr(coeffs), N.ptr(points), N.ptr(indexes),

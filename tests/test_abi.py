@@ -65,6 +65,14 @@ def test_invalid_arguments_return_errors_not_crashes():
   assert rc == -1
 
 
+def test_sh_bwd_rejects_accumulate_params():
+  """GsSHParams.accumulate_params only selects add / overwrite for gs_sh_bwd_flush; gs_sh_bwd reserves it."""
+  lib = _native.lib()
+  p = _native.GsSHParams(_native.GS_F32, 3, 16, 1, 100, 50, 1, 0)
+  rc = lib.gs_sh_bwd(ctypes.byref(p), None, None, None, None, None, None, None, None, None)
+  assert rc == -1 and b"accumulate_params" in lib.gs_last_error_string()
+
+
 def test_missing_cuda_tensor_fails_loudly():
   import pytest
   import torch

@@ -1,5 +1,7 @@
 """render_gaussians end to end on the GPU against the oracle pipeline (projection -> SH -> tile map ->
 rasterize) and torch autograd through the torch restatements for the 3D parameter gradients."""
+from contextlib import contextmanager, nullcontext
+
 import pytest
 import torch
 
@@ -96,28 +98,50 @@ def test_median_depth_and_depth16(cuda_device):
   assert out.ndc_median_depth.shape == (192, 256)
 
 
-@pytest.mark.parametrize("defer_sh", [True, False])
-@pytest.mark.parametrize("n,margin,views,sh_degree", [(5000, 0.0, 3, 3), (5000, 2.0, 3, 3), (3000, 0.5, 19, 1)])
-def test_fused_gradient_accumulation_matches_autograd(cuda_device, n, margin, views, sh_degree, defer_sh):
-  """GradientBucket.fused_accumulation(): the SH / projection backward add into the bucket inside the kernel, and
-  with defer_sh the SH coefficient gradient of the batch is formed once by the flush (per view only the masked colour
-  gradient is staged; 19 views cross the 16 view auto-flush).  After the batch the bucket must equal plain autograd
-  accumulation (same sums, different rounding order).  Nearly all visible / most gaussians culled / SH degree 1."""
-  from taichi_gaussian_rasterizer_b200.distributed import GradientBucket
+def _nearby_cameras(cam, views):
   from taichi_gaussian_rasterizer_b200.torch_lib.projection import join_rt, quat_to_mat
-  cfg = RasterConfig()
-  g, cam = scene3d(11, n, image_size=(256, 192), scale_factor=0.7, sh_degree=sh_degree, margin=margin)
-  cams = [cam.to(device=cuda_device)]
+  cams = [cam]
   for k in range(views - 1):
     q = torch.tensor([0.01 * (k % 5 + 1), -0.02 + 0.003 * k, 0.005, 1.0])
-    cams.append(cam.transformed(join_rt(quat_to_mat(q / q.norm()), torch.tensor([0.02, 0.001 * k, -0.01]))).to(device=cuda_device))
+    cams.append(cam.transformed(join_rt(quat_to_mat(q / q.norm()), torch.tensor([0.02, 0.001 * k, -0.01]))))
+  return cams
+
+
+@contextmanager
+def _plain_sinks(params):
+  """What fused_accumulation() does without the deferred SH state: every backward adds into p.grad by itself."""
+  from taichi_gaussian_rasterizer_b200.grad_sinks import register_grad_sink, unregister_grad_sink
+  for p in params:
+    register_grad_sink(p, p.grad)
+  try:
+    yield
+  finally:
+    for p in params:
+      unregister_grad_sink(p)
+
+
+@pytest.mark.parametrize("sink", ["deferred", "plain"])
+@pytest.mark.parametrize("n,margin,views,sh_degree", [(5000, 0.0, 3, 3), (5000, 2.0, 3, 3), (3000, 0.5, 19, 1)])
+def test_fused_gradient_accumulation_matches_autograd(cuda_device, n, margin, views, sh_degree, sink):
+  """GradientBucket.fused_accumulation(): the projection backward adds into the bucket inside the kernel and the SH
+  coefficient gradient of the batch is formed once by the deferred flush (per view only the masked colour gradient is
+  staged; 19 views cross the 16 view auto-flush).  With ``sink = plain`` the sinks are registered by hand and every
+  view's SH gradient is added by a one-view flush.  After the batch the bucket must equal plain autograd accumulation
+  (same sums, different rounding order).  Nearly all visible / most gaussians culled / SH degree 1."""
+  from taichi_gaussian_rasterizer_b200.distributed import GradientBucket
+  cfg = RasterConfig()
+  g, cam = scene3d(11, n, image_size=(256, 192), scale_factor=0.7, sh_degree=sh_degree, margin=margin)
+  cams = [c.to(device=cuda_device) for c in _nearby_cameras(cam, views)]
 
   def run(fused):
     gd = g.to(device=cuda_device)
     gd.requires_grad_(True)
     params = [gd.position, gd.log_scaling, gd.rotation, gd.alpha_logit, gd.feature]
     bucket = GradientBucket(params)
-    ctx = bucket.fused_accumulation(defer_sh=defer_sh) if fused else __import__("contextlib").nullcontext()
+    if not fused:
+      ctx = nullcontext()
+    else:
+      ctx = bucket.fused_accumulation() if sink == "deferred" else _plain_sinks(params)
     with ctx:
       bucket.flat.fill_(7.0)   # stale content: zero_() inside the context must void it (deferred slices: overwritten
       bucket.zero_()           # by the first flush instead of zero-filled)
@@ -134,6 +158,36 @@ def test_fused_gradient_accumulation_matches_autograd(cuda_device, n, margin, vi
   assert feat_a.abs().sum() > 0
   assert rel_l2(feat_b, feat_a) < 2e-6
   assert rel_l2(flat_b, flat_a) < 2e-6
+
+
+def test_pose_gradient_views_in_fused_accumulation(cuda_device):
+  """Views whose SH backward also wants the camera gradient (T_camera_world requires grad) inside
+  fused_accumulation(): their coefficient gradient must reach the bucket through the batch's deferred flush like any
+  other view's, after zero_() voided stale content, and the pose gradient must be plain autograd's."""
+  from taichi_gaussian_rasterizer_b200.distributed import GradientBucket
+  cfg = RasterConfig()
+  g, cam = scene3d(13, 5000, image_size=(256, 192), scale_factor=0.7, sh_degree=3)
+  cams_cpu = _nearby_cameras(cam, 3)
+
+  def run(fused):
+    gd = g.to(device=cuda_device)
+    gd.requires_grad_(True)
+    bucket = GradientBucket([gd.position, gd.log_scaling, gd.rotation, gd.alpha_logit, gd.feature])
+    cams = [c.to(device=cuda_device) for c in cams_cpu]
+    for c in cams:
+      c.T_camera_world.requires_grad_(True)
+    with bucket.fused_accumulation() if fused else nullcontext():
+      bucket.flat.fill_(7.0)
+      bucket.zero_()
+      for c in cams:
+        render_gaussians(gd, c, cfg, use_sh=True).image.square().mean().backward()
+    return bucket.flat.clone(), torch.stack([c.T_camera_world.grad for c in cams])
+
+  flat_a, pose_a = run(False)
+  flat_b, pose_b = run(True)
+  assert flat_a.abs().sum() > 0 and pose_a.abs().sum() > 0
+  assert rel_l2(flat_b, flat_a) < 2e-6
+  assert rel_l2(pose_b, pose_a) < 2e-6
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.float64])
@@ -162,7 +216,7 @@ def test_camera_position_kernel(cuda_device, dtype):
 
 
 def test_deferred_sh_clean_bucket_without_views(cuda_device):
-  """zero_() inside fused_accumulation(defer_sh=True) only marks the SH slice clean; leaving the context without a
+  """zero_() inside fused_accumulation() only marks the SH slice clean; leaving the context without a
   single staged view must still leave zeros there."""
   from taichi_gaussian_rasterizer_b200.distributed import GradientBucket
   g, _ = scene3d(5, 500, image_size=(64, 48), sh_degree=3)
