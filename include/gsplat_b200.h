@@ -16,7 +16,8 @@
  *   - return value: GS_OK (0) or a negative GsStatus; gs_last_error_string() describes the last
  *     failure on the calling thread.  Nothing throws or exits across this boundary;
  *   - `dtype` selects float (GS_F32) or double (GS_F64) for every `void*` floating tensor of
- *     the call; the tile mapper is f32 only, like the reference (mapper/tile_mapper.py:12);
+ *     the call; the tile mapper is f32 only, like the reference (mapper/tile_mapper.py:12); GS_BF16 is valid in
+ *     GsRasterParams.dtype only and selects bfloat16 for the feature side of the rasterizer (see there);
  *   - tensors are dense row-major with the shapes stated.
  */
 #ifndef GSPLAT_B200_H
@@ -37,7 +38,7 @@ typedef enum GsStatus {
   GS_ERR_WORKSPACE = -4    /* workspace too small */
 } GsStatus;
 
-typedef enum GsDtype { GS_F32 = 0, GS_F64 = 1 } GsDtype;
+typedef enum GsDtype { GS_F32 = 0, GS_F64 = 1, GS_BF16 = 2 } GsDtype;
 
 int gs_abi_version(void);
 const char* gs_last_error_string(void);
@@ -166,6 +167,14 @@ int gs_gather_rows_strided(int64_t capacity, int32_t row_floats, const float* sr
 int gs_scatter_rows_strided(int64_t capacity, int32_t row_floats, const float* src, int32_t src_stride,
                             int32_t src_offset, const int64_t* indexes, const int32_t* count_dev, int64_t dst_rows,
                             float* dst, void* stream);
+/* The same two for rows of 2-byte elements (bfloat16 features of a GS_BF16 rasterization; the bits are copied):
+ * row_elems, out_stride / out_offset and src_stride / src_offset count 2-byte elements. */
+int gs_gather_rows_strided_u16(int64_t capacity, int32_t row_elems, const uint16_t* src, const int64_t* indexes,
+                               const int32_t* count_dev, uint16_t* out, int32_t out_stride, int32_t out_offset,
+                               void* stream);
+int gs_scatter_rows_strided_u16(int64_t capacity, int32_t row_elems, const uint16_t* src, int32_t src_stride,
+                                int32_t src_offset, const int64_t* indexes, const int32_t* count_dev, int64_t dst_rows,
+                                uint16_t* dst, void* stream);
 
 /* render_depth: the rendered (P, channels) image split into its first `split` channels (depth, depth^2) and the rest,
  * and the inverse for the backward (a NULL part stands for zeros) — replaces the two strided slices of
@@ -277,7 +286,8 @@ typedef struct GsRasterParams {
   int32_t num_features;              /* F: 1..256 in f32 with tile_size 16, alpha blending and no antialiasing
                                         (antialiased: 1..7; 65..256 read rows of 16-byte aligned features in place
                                         when F is a multiple of 64); 1..40 in f32 otherwise (tile_size 32: 1..8);
-                                        1..8 in f64 (tile_size 32: 1..4).  Other counts: GS_ERR_UNSUPPORTED */
+                                        1..8 in f64 (tile_size 32: 1..4); 8..256 in bf16, see below.
+                                        Other counts: GS_ERR_UNSUPPORTED */
   int32_t antialias;
   int32_t use_alpha_blending;
   int32_t compute_visibility;
@@ -296,6 +306,14 @@ typedef struct GsRasterParams {
    * (1-W == 0, after which no output can change).  The reference has no forward exit. */
   double forward_exit_transmittance;
 } GsRasterParams;
+/* dtype GS_BF16: bfloat16 storage of the feature side, f32 arithmetic.  features (V,F), image (H,W,F) and grad_image
+ * (H,W,F) are bfloat16 (the image is the f32 blend rounded to nearest once); gaussians2d, image_alpha, visibility,
+ * point_heuristic, grad_gaussians, image_weight and grad_image_weight are f32, and so is grad_features (V,F): it is
+ * accumulated with f32 atomics, the caller rounds it or keeps it as an f32 master gradient.  Supported with F in
+ * 8..256, tile_size 16, alpha blending, no antialiasing and fewer than 2^31 gaussians; anything else returns
+ * GS_ERR_UNSUPPORTED (convert the features to f32 there).  Rows are padded to 8, 16, 40 or 64 channels (F <= 64) or to
+ * 64-channel slices in the workspace; rows whose length is already that (F = 8, 16, 40, 64, 128, 192, 256) are read in
+ * place and must be 16-byte aligned.  gs_raster_workspace_bytes sizes the bf16 layout (half the feature bytes). */
 
 size_t gs_raster_workspace_bytes(const GsRasterParams* p);
 

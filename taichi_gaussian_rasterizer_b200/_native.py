@@ -12,12 +12,12 @@ import torch
 _PKG = Path(__file__).resolve().parent
 LIB_PATH = _PKG / "libgsplat_b200.so"
 
-GS_F32, GS_F64 = 0, 1
+GS_F32, GS_F64, GS_BF16 = 0, 1, 2
 
 EXPORTS = [
   "gs_abi_version", "gs_last_error_string",
   "gs_project_fwd_workspace_bytes", "gs_project_fwd", "gs_project_bwd", "gs_project_bwd_counted",
-  "gs_sh_fwd", "gs_sh_fwd_counted", "gs_sh_bwd", "gs_sh_bwd_stage", "gs_sh_bwd_stage_counted", "gs_sh_bwd_flush", "gs_sh_fwd_views", "gs_gather_rows_counted", "gs_gather_rows_strided", "gs_scatter_rows_strided", "gs_split_channels", "gs_merge_channels",
+  "gs_sh_fwd", "gs_sh_fwd_counted", "gs_sh_bwd", "gs_sh_bwd_stage", "gs_sh_bwd_stage_counted", "gs_sh_bwd_flush", "gs_sh_fwd_views", "gs_gather_rows_counted", "gs_gather_rows_strided", "gs_scatter_rows_strided", "gs_gather_rows_strided_u16", "gs_scatter_rows_strided_u16", "gs_split_channels", "gs_merge_channels",
   "gs_tile_count", "gs_full_cumsum_workspace_bytes", "gs_full_cumsum", "gs_full_cumsum_counted", "gs_tile_emit_keys",
   "gs_radix_sort_pairs_workspace_bytes", "gs_radix_sort_pairs", "gs_radix_sort_pairs_counted", "gs_find_ranges",
   "gs_depth_keys", "gs_depth_keys_counted", "gs_tile_count_perm", "gs_tile_count_perm_counted", "gs_tile_emit_tiles", "gs_find_ranges_tiles",
@@ -172,12 +172,17 @@ def _invoke(fn, name, args):
   return rc
 
 
-def dtype_code(dtype: torch.dtype) -> int:
+def dtype_code(dtype: torch.dtype, raster: bool = False) -> int:
+  """GsDtype of ``dtype``.  ``raster``: the feature dtype of a rasterizer call, which may also be bfloat16 (GS_BF16:
+  bf16 features / image, f32 geometry and gradients); every other operator is float32 / float64 only."""
   if dtype == torch.float32:
     return GS_F32
   if dtype == torch.float64:
     return GS_F64
-  raise TypeError(f"unsupported dtype {dtype}: the kernels are float32 / float64")
+  if raster and dtype == torch.bfloat16:
+    return GS_BF16
+  raise TypeError(f"unsupported dtype {dtype}: the kernels are float32 / float64"
+                  + (" (the rasterizer's features may also be bfloat16)" if raster else ""))
 
 
 def require_cuda(*tensors):

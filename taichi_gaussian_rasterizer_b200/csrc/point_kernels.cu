@@ -459,11 +459,12 @@ gather_rows_counted_kernel(int64_t capacity, const float* __restrict__ src, cons
 // scatter needs no atomics; the count may still be on the device.
 //   gather : out[j * out_stride + out_offset + c] = src[indexes[j] * row + c]
 //   scatter: dst[indexes[j] * row + c] = src[j * src_stride + src_offset + c]      (dst zero-filled by the caller)
-// IdxT: uint32_t when the element count fits (a 64 bit division per thread costs more than the copy)
-template <typename IdxT>
+// IdxT: uint32_t when the element count fits (a 64 bit division per thread costs more than the copy); T: float, or
+// uint16_t for bf16 rows (gs_*_rows_strided_u16)
+template <typename IdxT, typename T = float>
 __global__ void __launch_bounds__(256)
-gather_rows_strided_kernel(int64_t capacity, int row, const float* __restrict__ src, const int64_t* __restrict__ indexes,
-                           const int32_t* __restrict__ count_dev, float* __restrict__ out, int out_stride,
+gather_rows_strided_kernel(int64_t capacity, int row, const T* __restrict__ src, const int64_t* __restrict__ indexes,
+                           const int32_t* __restrict__ count_dev, T* __restrict__ out, int out_stride,
                            int out_offset) {
   const IdxT e = (IdxT)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t nv = count_dev ? min(capacity, (int64_t)*count_dev) : capacity;
@@ -474,11 +475,11 @@ gather_rows_strided_kernel(int64_t capacity, int row, const float* __restrict__ 
   out[j * out_stride + out_offset + c] = src[indexes[j] * row + c];
 }
 
-template <typename IdxT>
+template <typename IdxT, typename T = float>
 __global__ void __launch_bounds__(256)
-scatter_rows_strided_kernel(int64_t capacity, int row, const float* __restrict__ src, int src_stride, int src_offset,
+scatter_rows_strided_kernel(int64_t capacity, int row, const T* __restrict__ src, int src_stride, int src_offset,
                             const int64_t* __restrict__ indexes, const int32_t* __restrict__ count_dev,
-                            float* __restrict__ dst) {
+                            T* __restrict__ dst) {
   const IdxT e = (IdxT)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t nv = count_dev ? min(capacity, (int64_t)*count_dev) : capacity;
   const IdxT jq = e / (IdxT)row;
@@ -941,43 +942,77 @@ int gs_gather_rows_counted(int64_t capacity, int32_t row_floats, const void* src
   return GS_OK;
 }
 
-int gs_gather_rows_strided(int64_t capacity, int32_t row_floats, const float* src, const int64_t* indexes,
-                           const int32_t* count_dev, float* out, int32_t out_stride, int32_t out_offset, void* stream) {
+}  // extern "C"
+
+template <typename T>
+static int gather_rows_strided(const char* who, int64_t capacity, int32_t row_floats, const T* src,
+                               const int64_t* indexes, const int32_t* count_dev, T* out, int32_t out_stride,
+                               int32_t out_offset, void* stream) {
   GS_CHECK_ARG(capacity >= 0 && row_floats > 0 && out_offset >= 0 && out_stride >= out_offset + row_floats,
-               "gs_gather_rows_strided: bad sizes");
+               "%s: bad sizes", who);
   if (capacity == 0) return GS_OK;
-  GS_CHECK_ARG(src && indexes && out, "gs_gather_rows_strided: null tensor");
+  GS_CHECK_ARG(src && indexes && out, "%s: null tensor", who);
   const int64_t total = capacity * row_floats;
   if (total + 256 < (1ll << 32))
-    gather_rows_strided_kernel<uint32_t><<<(unsigned)ceil_div(total, 256), 256, 0, (cudaStream_t)stream>>>(
+    gather_rows_strided_kernel<uint32_t, T><<<(unsigned)ceil_div(total, 256), 256, 0, (cudaStream_t)stream>>>(
         capacity, row_floats, src, indexes, count_dev, out, out_stride, out_offset);
   else
-    gather_rows_strided_kernel<uint64_t><<<(unsigned)ceil_div(total, 256), 256, 0, (cudaStream_t)stream>>>(
+    gather_rows_strided_kernel<uint64_t, T><<<(unsigned)ceil_div(total, 256), 256, 0, (cudaStream_t)stream>>>(
         capacity, row_floats, src, indexes, count_dev, out, out_stride, out_offset);
   GS_LAUNCH_CHECK();
   return GS_OK;
 }
 
-int gs_scatter_rows_strided(int64_t capacity, int32_t row_floats, const float* src, int32_t src_stride,
-                            int32_t src_offset, const int64_t* indexes, const int32_t* count_dev, int64_t dst_rows,
-                            float* dst, void* stream) {
+template <typename T>
+static int scatter_rows_strided(const char* who, int64_t capacity, int32_t row_floats, const T* src, int32_t src_stride,
+                                int32_t src_offset, const int64_t* indexes, const int32_t* count_dev, int64_t dst_rows,
+                                T* dst, void* stream) {
   GS_CHECK_ARG(capacity >= 0 && row_floats > 0 && src_offset >= 0 && src_stride >= src_offset + row_floats &&
-                   dst_rows >= 0, "gs_scatter_rows_strided: bad sizes");
+                   dst_rows >= 0, "%s: bad sizes", who);
   if (dst_rows == 0) return GS_OK;
-  GS_CHECK_ARG(dst != nullptr, "gs_scatter_rows_strided: null destination");
+  GS_CHECK_ARG(dst != nullptr, "%s: null destination", who);
   cudaStream_t st = (cudaStream_t)stream;
-  GS_CUDA(cudaMemsetAsync(dst, 0, (size_t)dst_rows * row_floats * sizeof(float), st));   // rows outside the visible set
+  GS_CUDA(cudaMemsetAsync(dst, 0, (size_t)dst_rows * row_floats * sizeof(T), st));   // rows outside the visible set
   if (capacity == 0) return GS_OK;
-  GS_CHECK_ARG(src && indexes, "gs_scatter_rows_strided: null tensor");
+  GS_CHECK_ARG(src && indexes, "%s: null tensor", who);
   const int64_t total = capacity * row_floats;
   if (total + 256 < (1ll << 32))
-    scatter_rows_strided_kernel<uint32_t><<<(unsigned)ceil_div(total, 256), 256, 0, st>>>(
+    scatter_rows_strided_kernel<uint32_t, T><<<(unsigned)ceil_div(total, 256), 256, 0, st>>>(
         capacity, row_floats, src, src_stride, src_offset, indexes, count_dev, dst);
   else
-    scatter_rows_strided_kernel<uint64_t><<<(unsigned)ceil_div(total, 256), 256, 0, st>>>(
+    scatter_rows_strided_kernel<uint64_t, T><<<(unsigned)ceil_div(total, 256), 256, 0, st>>>(
         capacity, row_floats, src, src_stride, src_offset, indexes, count_dev, dst);
   GS_LAUNCH_CHECK();
   return GS_OK;
+}
+
+extern "C" {
+
+int gs_gather_rows_strided(int64_t capacity, int32_t row_floats, const float* src, const int64_t* indexes,
+                           const int32_t* count_dev, float* out, int32_t out_stride, int32_t out_offset, void* stream) {
+  return gather_rows_strided("gs_gather_rows_strided", capacity, row_floats, src, indexes, count_dev, out, out_stride,
+                             out_offset, stream);
+}
+
+int gs_scatter_rows_strided(int64_t capacity, int32_t row_floats, const float* src, int32_t src_stride,
+                            int32_t src_offset, const int64_t* indexes, const int32_t* count_dev, int64_t dst_rows,
+                            float* dst, void* stream) {
+  return scatter_rows_strided("gs_scatter_rows_strided", capacity, row_floats, src, src_stride, src_offset, indexes,
+                              count_dev, dst_rows, dst, stream);
+}
+
+int gs_gather_rows_strided_u16(int64_t capacity, int32_t row_elems, const uint16_t* src, const int64_t* indexes,
+                               const int32_t* count_dev, uint16_t* out, int32_t out_stride, int32_t out_offset,
+                               void* stream) {
+  return gather_rows_strided("gs_gather_rows_strided_u16", capacity, row_elems, src, indexes, count_dev, out,
+                             out_stride, out_offset, stream);
+}
+
+int gs_scatter_rows_strided_u16(int64_t capacity, int32_t row_elems, const uint16_t* src, int32_t src_stride,
+                                int32_t src_offset, const int64_t* indexes, const int32_t* count_dev, int64_t dst_rows,
+                                uint16_t* dst, void* stream) {
+  return scatter_rows_strided("gs_scatter_rows_strided_u16", capacity, row_elems, src, src_stride, src_offset,
+                              indexes, count_dev, dst_rows, dst, stream);
 }
 
 int gs_split_channels(int64_t rows, int32_t channels, int32_t split, const float* src, float* first, float* rest,

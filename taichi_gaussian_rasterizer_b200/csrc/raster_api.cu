@@ -5,7 +5,10 @@ using namespace gs;
 
 static int check_raster(const GsRasterParams* p, const char* who) {
   if (!p) { set_error("%s: null params", who); return GS_ERR_INVALID; }
-  if (p->dtype != GS_F32 && p->dtype != GS_F64) { set_error("%s: dtype must be GS_F32 or GS_F64", who); return GS_ERR_INVALID; }
+  if (p->dtype != GS_F32 && p->dtype != GS_F64 && p->dtype != GS_BF16) {
+    set_error("%s: dtype must be GS_F32, GS_F64 or GS_BF16", who);
+    return GS_ERR_INVALID;
+  }
   if (p->image_width <= 0 || p->image_height <= 0 || p->num_features <= 0 || p->num_points < 0 || p->num_overlaps < 0) {
     set_error("%s: bad sizes (image %dx%d, F=%d, V=%lld, K=%lld)", who, p->image_width, p->image_height,
               p->num_features, (long long)p->num_points, (long long)p->num_overlaps);
@@ -24,6 +27,19 @@ static int check_raster(const GsRasterParams* p, const char* who) {
     set_error("%s: pixel_stride (%d, %d) and tile_size %d must allow at least one warp sized (32) tile", who, sx, sy,
               p->tile_size);
     return GS_ERR_INVALID;
+  }
+  if (p->dtype == GS_BF16) {   // bf16 feature storage exists on the fast kernels only (raster_fast_supported)
+    const char* why = p->num_features < 8 || p->num_features > 256 ? "8..256 feature channels"
+                      : p->tile_size != 16                          ? "tile_size 16"
+                      : !p->use_alpha_blending                      ? "alpha blending"
+                      : p->antialias                                ? "no antialiasing"
+                      : p->num_points >= (1ll << 31)                ? "fewer than 2^31 gaussians"
+                                                                    : nullptr;
+    if (why) {
+      set_error("%s: GS_BF16 features need %s (F=%d, tile_size %d, alpha blending %d, antialias %d)", who, why,
+                p->num_features, p->tile_size, p->use_alpha_blending, p->antialias);
+      return GS_ERR_UNSUPPORTED;
+    }
   }
   return GS_OK;
 }
@@ -44,7 +60,7 @@ int gs_raster_fwd(const GsRasterParams* p, const void* gaussians2d, const void* 
   GS_CHECK_ARG(p->num_points == 0 || (gaussians2d && features), "gs_raster_fwd: null gaussians / features");
   GS_CHECK_ARG(p->num_overlaps == 0 || overlap_to_point, "gs_raster_fwd: null overlap_to_point");
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t es = p->dtype == GS_F32 ? 4 : 8;
+  const size_t es = p->dtype == GS_F64 ? 8 : 4;   // GS_BF16: visibility / gradients are f32
   if (p->compute_visibility && visibility && p->num_points > 0)
     GS_CUDA(cudaMemsetAsync(visibility, 0, (size_t)p->num_points * es, st));
   RasterArgs a = {};
@@ -76,7 +92,7 @@ int gs_raster_bwd_with_weight(const GsRasterParams* p, const void* gaussians2d, 
   if (!p->use_alpha_blending) grad_image_weight = nullptr;
   GS_CHECK_ARG(!grad_image_weight || image_weight, "gs_raster_bwd_with_weight: grad_image_weight without image_weight");
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t es = p->dtype == GS_F32 ? 4 : 8;
+  const size_t es = p->dtype == GS_F64 ? 8 : 4;   // GS_BF16: visibility / gradients are f32
   if (grad_gaussians && p->num_points > 0) GS_CUDA(cudaMemsetAsync(grad_gaussians, 0, (size_t)p->num_points * 7 * es, st));
   if (grad_features && p->num_points > 0)
     GS_CUDA(cudaMemsetAsync(grad_features, 0, (size_t)p->num_points * p->num_features * es, st));

@@ -2,6 +2,10 @@
 // packed per-gaussian records, cp.async staging, the lane-parallel ellipse / pixel-block cull test.
 #pragma once
 
+#include <cuda_bf16.h>
+
+#include <type_traits>
+
 #include "raster.cuh"
 
 namespace gs {
@@ -11,6 +15,8 @@ constexpr int kFastTileArea = kFastTile * kFastTile;
 
 // padded feature row length used by the fast kernels for a given F (0 = unsupported)
 inline int fast_feature_pad(int F) { return F <= 4 ? 4 : F <= 8 ? 8 : F <= 16 ? 16 : F <= 36 ? 36 : F <= 64 ? 64 : 0; }
+// bfloat16 feature rows (GS_BF16, 8..64 channels): a multiple of 8 channels, so that a row is whole 16 B cp.async chunks
+inline int bf16_feature_pad(int F) { return F <= 8 ? 8 : F <= 16 ? 16 : F <= 40 ? 40 : F <= 64 ? 64 : 0; }
 
 // Extra-wide features (65..256 channels): rows of xwide_row(F) floats, 64-channel slices.
 constexpr int kXwideSlice = 64;
@@ -20,8 +26,8 @@ __host__ __device__ inline int xwide_row(int F) { return (F + kXwideSlice - 1) /
 
 // Workspace layout (all 256 B aligned):
 //   recF  V x 2 float4 : {mx, my, a1x, a1y} {a2x, a2y, log2(alpha), idx}       (forward records)
-//   featP V x FP float  : features padded to FP (extra-wide: empty when F is a multiple of 64, the kernels then read
-//                         the caller's features in place)
+//   featP V x FP         : features padded to FP, f32 or bf16 like the caller's (extra-wide: empty when F is a
+//                         multiple of 64, bf16: empty when F == FP; the kernels then read the caller's features in place)
 //   mask  K bytes        : per tile-list entry, which of the tile's eight 8x4 pixel blocks it can reach
 //   recB  V x 2 float4 : {mx, my, ax, ay} {1/sx, 1/sy, alpha, idx}             (records of the wide backward, F > 7;
 //                                                                               the narrow one walks recF)
@@ -29,17 +35,19 @@ struct FastLayout {
   size_t off_recF, off_feat, off_recB, off_mask, total;
   int FP;
   bool feat_in_place;
+  int feat_bytes;   // 4 (GS_F32) or 2 (GS_BF16)
 };
 
 inline FastLayout fast_layout(const GsRasterParams& p) {
   FastLayout L;
-  const bool xw = xwide_features(p.num_features);
-  L.FP = xw ? xwide_row(p.num_features) : fast_feature_pad(p.num_features);
-  L.feat_in_place = xw && L.FP == p.num_features;
+  const bool xw = xwide_features(p.num_features), bf = p.dtype == GS_BF16;
+  L.FP = xw ? xwide_row(p.num_features) : bf ? bf16_feature_pad(p.num_features) : fast_feature_pad(p.num_features);
+  L.feat_in_place = (xw || bf) && L.FP == p.num_features;
+  L.feat_bytes = bf ? 2 : 4;
   const size_t V = (size_t)(p.num_points > 0 ? p.num_points : 1);
   size_t off = 0;
   L.off_recF = off; off += align_up(V * 32, 256);
-  L.off_feat = off; off += L.feat_in_place ? 0 : align_up(V * (size_t)L.FP * 4, 256);
+  L.off_feat = off; off += L.feat_in_place ? 0 : align_up(V * (size_t)L.FP * L.feat_bytes, 256);
   L.off_recB = off; off += align_up(V * 32, 256);
   // one byte per tile-list entry: bit w = the entry can reach the 8x4 pixel block w of its tile (raster_cull_mask)
   L.off_mask = off; off += align_up((size_t)(p.num_overlaps > 0 ? p.num_overlaps : 1), 256);
@@ -98,6 +106,26 @@ __device__ __forceinline__ bool block_may_touch(float mx, float my, float a1x, f
   const float qh = A00 * dxh * dxh + 2.f * A01 * dxh * dyc + A11 * dyc * dyc;
   return fminf(qv, qh) < qmax * 1.001f + 1e-3f;
 }
+
+// ------------------------------------------------------------------------------------------------ feature storage
+// The fast kernels take the feature storage type TF as a template parameter: float (GS_F32) or __nv_bfloat16
+// (GS_BF16: features, image and image gradient stored in bf16; every blend and gradient is formed in f32 registers).
+template <typename TF>
+constexpr bool kBf16Storage = std::is_same_v<TF, __nv_bfloat16>;
+// elements of TF per 16 B cp.async chunk
+template <typename TF>
+constexpr int kChunkElems = 16 / (int)sizeof(TF);
+
+__device__ __forceinline__ float to_f32(float x) { return x; }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 x) { return __bfloat162float(x); }
+template <typename TF>
+__device__ __forceinline__ TF from_f32(float x) {   // bf16: round to nearest even, once, at the end
+  if constexpr (kBf16Storage<TF>) return __float2bfloat16_rn(x);
+  else return x;
+}
+// the two bf16 values of a 32 bit word as floats (exact): element 2k sits in the low half
+__device__ __forceinline__ float bf16_lo(unsigned w) { return __uint_as_float(w << 16); }
+__device__ __forceinline__ float bf16_hi(unsigned w) { return __uint_as_float(w & 0xffff0000u); }
 
 // ------------------------------------------------------------------------------------------------ tensor cores
 // D += A . B on one m16n8k8 tile, tf32 inputs, f32 accumulate (used by the wide backward kernels)
@@ -162,9 +190,9 @@ __device__ __forceinline__ int reduce_owner(int lane) {
 }
 
 // the padded feature rows the fast kernels stage from (workspace, or the caller's features read in place)
-inline const float* fast_feature_rows(const GsRasterParams& p, const RasterArgs& a) {
+inline const void* fast_feature_rows(const GsRasterParams& p, const RasterArgs& a) {
   const FastLayout L = fast_layout(p);
-  return L.feat_in_place ? (const float*)a.features : (const float*)((unsigned char*)a.workspace + L.off_feat);
+  return L.feat_in_place ? a.features : (const void*)((unsigned char*)a.workspace + L.off_feat);
 }
 
 int raster_fast_pack(const GsRasterParams& p, const RasterArgs& a, bool forward, bool features, cudaStream_t st);
@@ -172,6 +200,6 @@ int raster_fast_pack(const GsRasterParams& p, const RasterArgs& a, bool forward,
 int raster_cull_mask(const GsRasterParams& p, const RasterArgs& a, cudaStream_t st);
 
 // raster_fast_bwd_wide.cu: backward for 8..256 feature channels (one pixel per lane, tensor-core feature gradient)
-int raster_bwd_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP, cudaStream_t st);
+int raster_bwd_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const void* featP, cudaStream_t st);
 
 }  // namespace gs

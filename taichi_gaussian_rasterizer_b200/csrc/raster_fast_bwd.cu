@@ -401,18 +401,18 @@ int raster_bwd_fast(const GsRasterParams& p, const RasterArgs& a, cudaStream_t s
   }
   const FastLayout L = fast_layout(p);
   unsigned char* ws = (unsigned char*)a.workspace;
-  const float* featP = fast_feature_rows(p, a);
+  const void* featP = fast_feature_rows(p, a);
   if (p.num_features > 7)   // 8..256 channels: one pixel per lane, its own records
     return raster_bwd_wide(p, a, (const float4*)(ws + L.off_recB), featP, st);
   const float4* rec = (const float4*)(ws + (p.antialias ? L.off_recB : L.off_recF));   // the forward's records
   switch (p.num_features) {
-    case 1: return launch_bwd_fast<1, 4>(p, a, rec, featP, st);
-    case 2: return launch_bwd_fast<2, 4>(p, a, rec, featP, st);
-    case 3: return launch_bwd_fast<3, 4>(p, a, rec, featP, st);
-    case 4: return launch_bwd_fast<4, 4>(p, a, rec, featP, st);
-    case 5: return launch_bwd_fast<5, 8>(p, a, rec, featP, st);
-    case 6: return launch_bwd_fast<6, 8>(p, a, rec, featP, st);
-    case 7: return launch_bwd_fast<7, 8>(p, a, rec, featP, st);
+    case 1: return launch_bwd_fast<1, 4>(p, a, rec, (const float*)featP, st);
+    case 2: return launch_bwd_fast<2, 4>(p, a, rec, (const float*)featP, st);
+    case 3: return launch_bwd_fast<3, 4>(p, a, rec, (const float*)featP, st);
+    case 4: return launch_bwd_fast<4, 4>(p, a, rec, (const float*)featP, st);
+    case 5: return launch_bwd_fast<5, 8>(p, a, rec, (const float*)featP, st);
+    case 6: return launch_bwd_fast<6, 8>(p, a, rec, (const float*)featP, st);
+    case 7: return launch_bwd_fast<7, 8>(p, a, rec, (const float*)featP, st);
     default: break;
   }
   GS_UNSUPPORTED("rasterizer backward (fast): %d feature channels", p.num_features);

@@ -38,6 +38,13 @@
 //   * FP = 0, extra-wide (65..256 channels, rows of xwide_row(F) floats): G (up to 256 floats) no longer fits in
 //     registers and is read from the warp's shared tile only; batches of 16 entries so that at F = 256 two CTAs of two
 //     warps fit an SM (2 x 107 KB of shared memory: 32 px x 256 ch x 4 B = 32 KB of G per warp is what limits that).
+// bf16 storage (GS_BF16, TF = __nv_bfloat16): image, image gradient and staged feature rows are bf16 (rows of
+// bf16_feature_pad(F) or xwide_row(F) channels), every sum is formed in f32 and grad_features stays f32 (atomics).  A
+// bf16 value is exact in tf32 (8 significand bits of 11), so the product needs only the weight split: W_hi G + W_lo G,
+// two products instead of three, the same 2^-24 residual on W.  The extra-wide mode keeps its G tile in bf16 (half the
+// shared memory: 60 instead of 110 KB per CTA at F = 256, room for three CTAs per SM instead of two); the F <= 64 modes keep the
+// f32 G tile of the f32 kernel, whose B-fragment loads are conflict free and whose shared memory is not what bounds
+// their occupancy (their register copy of G is f32 either way).
 // The forward of the extra-wide mode is raster_fwd_fast_kernel<64, ..., XW = true> (raster_fast_fwd.cu): one CTA per
 // tile and 64-channel slice.  The backward cannot be sliced that way: aag = alpha_0 * alpha_grad enters the heuristics
 // as aag^2 and |pgx| + |pgy|, which are not linear in the channels, and alpha_grad itself needs the full G . f_i.
@@ -54,37 +61,43 @@ constexpr int kWideWS = 36;      // row stride of the weight tile (float2 units)
 
 // Shared memory of a CTA: two staged batches {records, feature rows}, then per warp the G tile [32][GS], the weight tile
 // [16][kWideWS] of {hi, lo} and the survivors' indices [16].
-template <int FP>
+// TF: feature storage; GT: element of the G tile (bf16 only in the extra-wide bf16 mode).
+template <int FP, typename TF = float>
 struct WideLayout {
   // staged tile-list entries per buffer (F <= 64: 64 gave 8.6 ms instead of 6.9 at config 4, the warps of a CTA drift
   // further apart between barriers)
   static constexpr int kBatch = FP > 0 ? 32 : 16;
-  int row;   // feature row (floats)
+  using GT = std::conditional_t<FP == 0, TF, float>;
+  int row;   // feature row (elements of TF)
   int FP8;   // channels padded to n-tiles of 8
-  // row stride of the G tile (floats).  F <= 64: = 8 or 24 mod 32, so that the B-fragment loads (row = lane & 3 (+4),
-  // column = lane >> 2) hit 32 different banks.  Extra-wide: 4 mod 32, so that a lane reading its own row with LDS.128
-  // (G . f_i) is conflict free; the B fragments take two-way conflicts there.
+  // row stride of the G tile (elements of GT).  F <= 64: = 8 or 24 mod 32, so that the B-fragment loads (row = lane & 3
+  // (+4), column = lane >> 2) hit 32 different banks.  Extra-wide: 16 B past a multiple of 128 B, so that a lane
+  // reading its own row with LDS.128 (G . f_i) is conflict free; the f32 B fragments take two-way conflicts there (the
+  // bf16 ones none: the four rows start 4 banks apart and a row's eight columns share 4 words).
   int GS;
   size_t stage_bytes, warp_bytes;
   __host__ __device__ explicit WideLayout(int F)
       : row(FP > 0 ? FP : xwide_row(F)), FP8((row + 7) / 8 * 8),
-        GS(FP == 0 ? row + 4 : (FP8 % 32 == 8 || FP8 % 32 == 24) ? FP8 : FP8 + 8),
-        stage_bytes((size_t)2 * kBatch * (32 + row * 4)),
-        warp_bytes((size_t)32 * GS * 4 + kWideGroup * kWideWS * 8 + kWideGroup * 4) {}
+        GS(FP == 0 ? row + 16 / (int)sizeof(GT) : (FP8 % 32 == 8 || FP8 % 32 == 24) ? FP8 : FP8 + 8),
+        stage_bytes((size_t)2 * kBatch * (32 + row * (int)sizeof(TF))),
+        warp_bytes((size_t)32 * GS * sizeof(GT) + kWideGroup * kWideWS * 8 + kWideGroup * 4) {}
   __host__ __device__ size_t total() const { return stage_bytes + kWideWarps * warp_bytes; }
 };
 
 // WGT: the image weight W is differentiable too (gradient gw, forward W in wimg): one more channel whose feature is
 // always 1, so RG starts with W_final Gw and f . G gains + Gw (see raster_bwd_fast_kernel).
-template <int FP, bool HEUR, bool WGT>
+template <int FP, bool HEUR, bool WGT, typename TF = float>
 __global__ void __launch_bounds__(kWideWarps * 32, 8)   // eight CTAs of two warps per SM: at most 128 registers
 raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float4* __restrict__ rec,
-                           const float* __restrict__ featP, const int32_t* __restrict__ ranges,
-                           const int32_t* __restrict__ o2p, const float* __restrict__ image,
-                           const float* __restrict__ grad_image, float* __restrict__ grad_pts,
+                           const TF* __restrict__ featP, const int32_t* __restrict__ ranges,
+                           const int32_t* __restrict__ o2p, const TF* __restrict__ image,
+                           const TF* __restrict__ grad_image, float* __restrict__ grad_pts,
                            float* __restrict__ grad_feat, float* __restrict__ heuristic,
                            const float* __restrict__ wimg, const float* __restrict__ gw) {
-  using Layout = WideLayout<FP>;
+  using Layout = WideLayout<FP, TF>;
+  using GT = typename Layout::GT;
+  constexpr bool kBF = kBf16Storage<TF>;
+  constexpr int CE = kChunkElems<TF>;   // features per 16 B chunk
   constexpr int kBatch = Layout::kBatch;
   constexpr int NG = 7 + (HEUR ? 2 : 0);             // geometry (+ heuristic) values
   constexpr int kThreads = kWideWarps * 32, kParts = 8 / kWideWarps;
@@ -95,14 +108,14 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
   extern __shared__ __align__(16) unsigned char smem[];
   float4* s_r0 = reinterpret_cast<float4*>(smem);                       // [2][kBatch]
   float4* s_r1 = s_r0 + 2 * kBatch;                                     // [2][kBatch]
-  float* s_feat = reinterpret_cast<float*>(smem + 2 * kBatch * 32);     // [2][kBatch][row]
+  TF* s_feat = reinterpret_cast<TF*>(smem + 2 * kBatch * 32);           // [2][kBatch][row]
 
   const int tile = blockIdx.x / kParts, t = threadIdx.x, lane = t & 31, lwarp = t >> 5;
   const int warp = (blockIdx.x % kParts) * kWideWarps + lwarp;   // which 8x4 pixel block of the tile
   unsigned char* wbase = smem + L.stage_bytes + (size_t)lwarp * L.warp_bytes;
-  float* s_G = reinterpret_cast<float*>(wbase);                                            // [32][GS]
-  float2* s_W = reinterpret_cast<float2*>(wbase + (size_t)32 * GS * 4);                    // [16][WS] {hi, lo}
-  int* s_idx = reinterpret_cast<int*>(wbase + (size_t)32 * GS * 4 + kWideGroup * kWideWS * 8);   // [16]
+  GT* s_G = reinterpret_cast<GT*>(wbase);                                                        // [32][GS]
+  float2* s_W = reinterpret_cast<float2*>(wbase + (size_t)32 * GS * sizeof(GT));                 // [16][WS] {hi, lo}
+  int* s_idx = reinterpret_cast<int*>(wbase + (size_t)32 * GS * sizeof(GT) + kWideGroup * kWideWS * 8);   // [16]
 
   const int tw = (p.image_width + kFastTile - 1) / kFastTile;
   const int wx0 = (tile % tw) * kFastTile + (warp & 1) * 8;
@@ -119,16 +132,16 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
   const int gid = lane >> 2, tig = lane & 3;
 
   float G[FP > 0 ? FP : 1];   // F <= 64: the register copy of this lane's row of the G tile
-  float* my_G = s_G + lane * GS;
+  GT* my_G = s_G + lane * GS;
   float W = inb ? 0.f : 1.f, RG = 0.f, Gw = 0.f;
   {
     const int64_t pix = (int64_t)py * p.image_width + px;   // 64 bit: a 4K image of 256 channels has 2.1 G elements
 #pragma unroll(FP > 0 ? FP : 4)
     for (int c = 0; c < row; ++c) {
       const bool ok = inb && c < F;
-      const float g = ok ? grad_image[pix * F + c] : 0.f;
-      RG = fmaf(ok ? image[pix * F + c] : 0.f, g, RG);
-      my_G[c] = g;
+      const float g = ok ? to_f32(grad_image[pix * F + c]) : 0.f;
+      RG = fmaf(ok ? to_f32(image[pix * F + c]) : 0.f, g, RG);
+      my_G[c] = from_f32<GT>(g);   // exact: g is a value of TF
       if constexpr (FP > 0) G[c] = g;
     }
     if constexpr (WGT) {
@@ -136,7 +149,7 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
       RG = fmaf(inb ? wimg[pix] : 0.f, Gw, RG);
     }
 #pragma unroll
-    for (int c = row; c < FP8; ++c) my_G[c] = 0.f;
+    for (int c = row; c < FP8; ++c) my_G[c] = GT();
   }
   __syncwarp();
 
@@ -163,12 +176,18 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
         float c[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-          const float b0 = s_G[(tig + 8 * k) * GS + gid + 8 * n], b1 = s_G[(tig + 4 + 8 * k) * GS + gid + 8 * n];
-          const unsigned b0h = tf32_rna(b0), b1h = tf32_rna(b1);
-          const unsigned b0l = tf32_rna(b0 - __uint_as_float(b0h)), b1l = tf32_rna(b1 - __uint_as_float(b1h));
-          mma_tf32_16x8x8(c, ahi[k], b0h, b1h);
-          mma_tf32_16x8x8(c, alo[k], b0h, b1h);
-          mma_tf32_16x8x8(c, ahi[k], b0l, b1l);
+          const float b0 = to_f32(s_G[(tig + 8 * k) * GS + gid + 8 * n]);
+          const float b1 = to_f32(s_G[(tig + 4 + 8 * k) * GS + gid + 8 * n]);
+          if constexpr (kBF) {   // G is exact in tf32
+            mma_tf32_16x8x8(c, ahi[k], __float_as_uint(b0), __float_as_uint(b1));
+            mma_tf32_16x8x8(c, alo[k], __float_as_uint(b0), __float_as_uint(b1));
+          } else {
+            const unsigned b0h = tf32_rna(b0), b1h = tf32_rna(b1);
+            const unsigned b0l = tf32_rna(b0 - __uint_as_float(b0h)), b1l = tf32_rna(b1 - __uint_as_float(b1h));
+            mma_tf32_16x8x8(c, ahi[k], b0h, b1h);
+            mma_tf32_16x8x8(c, alo[k], b0h, b1h);
+            mma_tf32_16x8x8(c, ahi[k], b0l, b1l);
+          }
         }
         const int ch = 8 * n + 2 * tig;
         if (i0 >= 0) {
@@ -199,13 +218,13 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
         cp_async16(&s_r1[buf * kBatch + t], rec + 2 * (int64_t)idx + 1);
       }
     }
-    const int CH = row / 4;
+    const int CH = row / CE;
     auto stage_chunk = [&](int q) {   // 16 B chunk q of the batch's feature rows
       const int slot = q / CH, part = q - slot * CH;
       const int v = b * kBatch + slot;
       if (v < C) {
         const int idx = o2p[start + v];
-        cp_async16(s_feat + (buf * kBatch + slot) * row + part * 4, featP + (int64_t)idx * row + part * 4);
+        cp_async16(s_feat + (buf * kBatch + slot) * row + part * CE, featP + (int64_t)idx * row + part * CE);
       }
     };
     if constexpr (FP > 0) {   // literal trip count, fully unrolled (rolled, the loop cost 2-3 % of the kernel time)
@@ -263,16 +282,36 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
           W += wl;
           const float rinv = fast_rcp(1.f - alpha);
           // G . f_i over all channels (padded channels are zero in both)
-          const float* frow = s_feat + (buf * kBatch + j) * row;
+          const TF* frow = s_feat + (buf * kBatch + j) * row;
           float fG0 = 0.f, fG1 = 0.f, fG2 = 0.f, fG3 = 0.f;   // four independent chains: the dot product is latency bound
+          if constexpr (kBF) {   // eight channels per LDS.128, the chains of the f32 loop (channel c -> chain c % 4)
+#pragma unroll(FP > 0 ? FP / 8 : 4)
+            for (int c = 0; c < row; c += 8) {
+              const uint4 f8 = *reinterpret_cast<const uint4*>(frow + c);
+              float g8[8];
+              if constexpr (FP > 0) {
+#pragma unroll
+                for (int k = 0; k < 8; ++k) g8[k] = G[c + k];
+              } else {
+                const uint4 u = *reinterpret_cast<const uint4*>(my_G + c);
+                g8[0] = bf16_lo(u.x); g8[1] = bf16_hi(u.x); g8[2] = bf16_lo(u.y); g8[3] = bf16_hi(u.y);
+                g8[4] = bf16_lo(u.z); g8[5] = bf16_hi(u.z); g8[6] = bf16_lo(u.w); g8[7] = bf16_hi(u.w);
+              }
+              fG0 = fmaf(bf16_lo(f8.x), g8[0], fG0); fG1 = fmaf(bf16_hi(f8.x), g8[1], fG1);
+              fG2 = fmaf(bf16_lo(f8.y), g8[2], fG2); fG3 = fmaf(bf16_hi(f8.y), g8[3], fG3);
+              fG0 = fmaf(bf16_lo(f8.z), g8[4], fG0); fG1 = fmaf(bf16_hi(f8.z), g8[5], fG1);
+              fG2 = fmaf(bf16_lo(f8.w), g8[6], fG2); fG3 = fmaf(bf16_hi(f8.w), g8[7], fG3);
+            }
+          } else {
 #pragma unroll(FP > 0 ? FP / 4 : 4)
-          for (int c = 0; c < row; c += 4) {
-            const float4 f4 = *reinterpret_cast<const float4*>(frow + c);
-            float4 g4;
-            if constexpr (FP > 0) g4 = make_float4(G[c], G[c + 1], G[c + 2], G[c + 3]);
-            else g4 = *reinterpret_cast<const float4*>(my_G + c);
-            fG0 = fmaf(f4.x, g4.x, fG0); fG1 = fmaf(f4.y, g4.y, fG1);
-            fG2 = fmaf(f4.z, g4.z, fG2); fG3 = fmaf(f4.w, g4.w, fG3);
+            for (int c = 0; c < row; c += 4) {
+              const float4 f4 = *reinterpret_cast<const float4*>(frow + c);
+              float4 g4;
+              if constexpr (FP > 0) g4 = make_float4(G[c], G[c + 1], G[c + 2], G[c + 3]);
+              else g4 = *reinterpret_cast<const float4*>(my_G + c);
+              fG0 = fmaf(f4.x, g4.x, fG0); fG1 = fmaf(f4.y, g4.y, fG1);
+              fG2 = fmaf(f4.z, g4.z, fG2); fG3 = fmaf(f4.w, g4.w, fG3);
+            }
           }
           float fG = (fG0 + fG1) + (fG2 + fG3);
           if constexpr (WGT) fG += Gw;
@@ -307,33 +346,46 @@ raster_bwd_wide_mma_kernel(const __grid_constant__ GsRasterParams p, const float
   if (ns > 0) flush_group();
 }
 
-template <int FP, bool HEUR, bool WGT>
-static int launch_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP,
+template <int FP, bool HEUR, bool WGT, typename TF>
+static int launch_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const void* featP,
                        cudaStream_t st) {
-  const size_t smem = WideLayout<FP>(p.num_features).total();
+  const size_t smem = WideLayout<FP, TF>(p.num_features).total();
   const int tiles = tiles_wide(p) * tiles_high(p);
   // per launch: the attribute belongs to the (function, device) pair and the call costs about a microsecond
-  GS_CUDA(cudaFuncSetAttribute(raster_bwd_wide_mma_kernel<FP, HEUR, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)smem));
-  raster_bwd_wide_mma_kernel<FP, HEUR, WGT><<<tiles * (8 / kWideWarps), kWideWarps * 32, smem, st>>>(
-      p, rec, featP, a.tile_ranges, a.overlap_to_point, (const float*)a.image_in, (const float*)a.grad_image,
+  GS_CUDA(cudaFuncSetAttribute(raster_bwd_wide_mma_kernel<FP, HEUR, WGT, TF>,
+                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  raster_bwd_wide_mma_kernel<FP, HEUR, WGT, TF><<<tiles * (8 / kWideWarps), kWideWarps * 32, smem, st>>>(
+      p, rec, (const TF*)featP, a.tile_ranges, a.overlap_to_point, (const TF*)a.image_in, (const TF*)a.grad_image,
       (float*)a.grad_gaussians, (float*)a.grad_features, HEUR ? (float*)a.point_heuristic : nullptr,
       (const float*)a.image_weight, (const float*)a.grad_image_weight);
   GS_LAUNCH_CHECK();
   return GS_OK;
 }
 
-template <int FP>
-static int dispatch_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP,
+template <int FP, typename TF = float>
+static int dispatch_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const void* featP,
                          cudaStream_t st) {
   const bool heur = p.compute_point_heuristic && a.point_heuristic != nullptr;
   if (a.grad_image_weight != nullptr)
-    return heur ? launch_wide<FP, true, true>(p, a, rec, featP, st) : launch_wide<FP, false, true>(p, a, rec, featP, st);
-  return heur ? launch_wide<FP, true, false>(p, a, rec, featP, st) : launch_wide<FP, false, false>(p, a, rec, featP, st);
+    return heur ? launch_wide<FP, true, true, TF>(p, a, rec, featP, st)
+                : launch_wide<FP, false, true, TF>(p, a, rec, featP, st);
+  return heur ? launch_wide<FP, true, false, TF>(p, a, rec, featP, st)
+              : launch_wide<FP, false, false, TF>(p, a, rec, featP, st);
 }
 
-int raster_bwd_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const float* featP,
+int raster_bwd_wide(const GsRasterParams& p, const RasterArgs& a, const float4* rec, const void* featP,
                     cudaStream_t st) {
+  if (p.dtype == GS_BF16) {
+    using bf16 = __nv_bfloat16;
+    if (xwide_features(p.num_features)) return dispatch_wide<0, bf16>(p, a, rec, featP, st);
+    switch (bf16_feature_pad(p.num_features)) {
+      case 8: return dispatch_wide<8, bf16>(p, a, rec, featP, st);
+      case 16: return dispatch_wide<16, bf16>(p, a, rec, featP, st);
+      case 40: return dispatch_wide<40, bf16>(p, a, rec, featP, st);
+      case 64: return dispatch_wide<64, bf16>(p, a, rec, featP, st);
+      default: GS_UNSUPPORTED("rasterizer backward (wide, bf16): %d feature channels", p.num_features);
+    }
+  }
   if (xwide_features(p.num_features)) return dispatch_wide<0>(p, a, rec, featP, st);
   switch (fast_feature_pad(p.num_features)) {
     case 8: return dispatch_wide<8>(p, a, rec, featP, st);

@@ -52,19 +52,23 @@ raster_pack_kernel(int64_t V, int F, const float* __restrict__ g, const float* _
   }
 }
 
-// extra-wide features whose rows are not a whole number of 64-channel slices: one thread per padded element
+// extra-wide features whose rows are not a whole number of 64-channel slices, and bf16 rows that are not a whole
+// number of 8-channel chunks: one thread per padded element
+template <typename TF>
 __global__ void __launch_bounds__(256)
-raster_pad_rows_kernel(int64_t n, int F, int FP, const float* __restrict__ feat, float* __restrict__ featP) {
+raster_pad_rows_kernel(int64_t n, int F, int FP, const TF* __restrict__ feat, TF* __restrict__ featP) {
   const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= n) return;
   const int64_t i = q / FP;
   const int c = (int)(q - i * FP);
-  featP[q] = c < F ? feat[i * F + c] : 0.f;
+  featP[q] = c < F ? feat[i * F + c] : TF();
 }
 
 int raster_fast_pack(const GsRasterParams& p, const RasterArgs& a, bool forward, bool features, cudaStream_t st) {
   if (p.num_points == 0) return GS_OK;
-  if (xwide_features(p.num_features)) {   // records as for the wide path, features padded to 64-channel slices
+  // extra-wide or bf16 features (8..256 channels): records as for the wide path, features padded to 64-channel slices
+  // (extra-wide) or to bf16_feature_pad
+  if (xwide_features(p.num_features) || p.dtype == GS_BF16) {
     const FastLayout L = fast_layout(p);
     if (L.feat_in_place && ((uintptr_t)a.features & 15) != 0) {   // cp.async stages them in 16 B pieces
       set_error("rasterizer: %d feature channels are read in place and must be 16-byte aligned", p.num_features);
@@ -78,8 +82,12 @@ int raster_fast_pack(const GsRasterParams& p, const RasterArgs& a, bool forward,
     GS_LAUNCH_CHECK();
     if (features && !L.feat_in_place) {
       const int64_t n = p.num_points * (int64_t)L.FP;
-      raster_pad_rows_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, st>>>(n, p.num_features, L.FP, (const float*)a.features,
-                                                                         (float*)(ws + L.off_feat));
+      if (p.dtype == GS_BF16)
+        raster_pad_rows_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, st>>>(
+            n, p.num_features, L.FP, (const __nv_bfloat16*)a.features, (__nv_bfloat16*)(ws + L.off_feat));
+      else
+        raster_pad_rows_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, st>>>(n, p.num_features, L.FP, (const float*)a.features,
+                                                                           (float*)(ws + L.off_feat));
       GS_LAUNCH_CHECK();
     }
     return GS_OK;
@@ -186,16 +194,20 @@ int raster_cull_mask(const GsRasterParams& p, const RasterArgs& a, cudaStream_t 
 // 256 pixels x 256 channels of accumulators (256 KB) are the whole register file of an SM, so a CTA can hold the
 // full channel range of a few pixel blocks only, and each such CTA would stage all F channels of every entry (4 x
 // the feature bytes at F = 256 for four CTAs per tile); a slice CTA stages its own 64 channels and the records.
-template <int FP, bool VIS, int BATCH, bool FOURTH = true, bool AA = false, bool XW = false>
-__global__ void __launch_bounds__(kFwdThreads, FP <= 8 ? 0 : (FP <= 36 ? 4 : 2))   // narrow: no occupancy target (the compiler settles on 30 registers = 8 CTAs per SM by itself; forcing 8 lengthened the VIS walk); 64 / 128 registers for the wide ones
+// TF: feature / image storage (float, or __nv_bfloat16 for GS_BF16: rows of FP = 8, 16, 40, 64 bf16, or 64-channel
+// slices; each feature is widened to f32 where it is used, the blend is the f32 one, the image is rounded once).
+template <int FP, bool VIS, int BATCH, bool FOURTH = true, bool AA = false, bool XW = false, typename TF = float>
+__global__ void __launch_bounds__(kFwdThreads, FP <= 8 ? 0 : (FP <= 40 ? 4 : 2))   // narrow: no occupancy target (the compiler settles on 30 registers = 8 CTAs per SM by itself; forcing 8 lengthened the VIS walk); 64 / 128 registers for the wide ones
 raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* __restrict__ rec,
-                       const float* __restrict__ featP, const int32_t* __restrict__ ranges,
-                       const int32_t* __restrict__ o2p, float* __restrict__ image, float* __restrict__ image_alpha,
+                       const TF* __restrict__ featP, const int32_t* __restrict__ ranges,
+                       const int32_t* __restrict__ o2p, TF* __restrict__ image, float* __restrict__ image_alpha,
                        float* __restrict__ visibility, const unsigned char* __restrict__ cull_mask) {
   constexpr int kFwdBatch = BATCH;
-  // one staged entry = {record (2 x float4), feature row (FP / 4 x float4)} in consecutive 16 B units: one address
-  // per entry in the inner loop.  U is odd so that a lane-per-entry LDS.128 (the cull) is bank-conflict free.
-  constexpr int U = (2 + FP / 4) | 1;
+  constexpr int CE = kChunkElems<TF>;   // features per 16 B unit: 4 f32 or 8 bf16
+  // one staged entry = {record (2 x float4), feature row (FP / CE 16 B units)} in consecutive 16 B units: one address
+  // per entry in the inner loop.  U is odd so that a lane-per-entry LDS.128 (the cull) is bank-conflict free (bf16:
+  // U = 3, 5, 7, 11 for FP = 8, 16, 40, 64).
+  constexpr int U = (2 + FP / CE) | 1;
   __shared__ __align__(16) float4 s_e[2][kFwdBatch][U];
   __shared__ unsigned char s_mask[2][kFwdBatch];   // cull bytes of the staged entries (raster_cull_mask_kernel)
   // VIS: the visibility sums of every staged entry, one word per warp (23 bit fixed point: 32 pixels stay below 2^28),
@@ -246,7 +258,7 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
           s_mask[buf][slot] = m;
         } else {
 #pragma unroll
-          for (int c = 0; c < FP; c += 4) cp_async16(&s_e[buf][slot][2 + c / 4], featP + (int64_t)idx * frow + c_base + c);
+          for (int c = 0; c < FP; c += CE) cp_async16(&s_e[buf][slot][2 + c / CE], featP + (int64_t)idx * frow + c_base + c);
         }
       }
     } else {  // wide rows: records by the first BATCH threads, the 16 B feature chunks spread over the whole CTA
@@ -261,7 +273,7 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
           s_mask[buf][t] = m;
         }
       }
-      constexpr int CH = FP / 4;
+      constexpr int CH = FP / CE;
 #pragma unroll
       for (int q0 = 0; q0 < kFwdBatch * CH; q0 += kFwdThreads) {
         const int q = q0 + t;
@@ -269,7 +281,7 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
         const int v = b * kFwdBatch + slot;
         if (q < kFwdBatch * CH && v < total) {
           const int idx = o2p[start + (v < C ? v : v - kFastTileArea)];
-          cp_async16(&s_e[buf][slot][2 + part], featP + (int64_t)idx * frow + c_base + part * 4);
+          cp_async16(&s_e[buf][slot][2 + part], featP + (int64_t)idx * frow + c_base + part * CE);
         }
       }
     }
@@ -319,13 +331,26 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
           // the divergent branch did (the cull leaves few gaussians that miss every pixel of the block)
           const float weight = alpha > thr ? alpha * (1.f - W) : 0.f;
           W += weight;
+          if constexpr (kBf16Storage<TF>) {
 #pragma unroll
-          for (int c4 = 0; c4 < FP / 4; ++c4) {
-            const float4 f4 = ent[2 + c4];
-            acc[4 * c4] = fmaf(f4.x, weight, acc[4 * c4]);
-            acc[4 * c4 + 1] = fmaf(f4.y, weight, acc[4 * c4 + 1]);
-            acc[4 * c4 + 2] = fmaf(f4.z, weight, acc[4 * c4 + 2]);
-            if (FP > 4 || FOURTH) acc[4 * c4 + 3] = fmaf(f4.w, weight, acc[4 * c4 + 3]);
+            for (int c8 = 0; c8 < FP / 8; ++c8) {
+              const uint4 u = reinterpret_cast<const uint4*>(ent)[2 + c8];
+              const unsigned wd[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+              for (int k = 0; k < 4; ++k) {
+                acc[8 * c8 + 2 * k] = fmaf(bf16_lo(wd[k]), weight, acc[8 * c8 + 2 * k]);
+                acc[8 * c8 + 2 * k + 1] = fmaf(bf16_hi(wd[k]), weight, acc[8 * c8 + 2 * k + 1]);
+              }
+            }
+          } else {
+#pragma unroll
+            for (int c4 = 0; c4 < FP / 4; ++c4) {
+              const float4 f4 = ent[2 + c4];
+              acc[4 * c4] = fmaf(f4.x, weight, acc[4 * c4]);
+              acc[4 * c4 + 1] = fmaf(f4.y, weight, acc[4 * c4 + 1]);
+              acc[4 * c4 + 2] = fmaf(f4.z, weight, acc[4 * c4 + 2]);
+              if (FP > 4 || FOURTH) acc[4 * c4 + 3] = fmaf(f4.w, weight, acc[4 * c4 + 3]);
+            }
           }
           if constexpr (VIS) {
             // visibility[g] += sum over the tile's pixels of the blend weight.  The weights are in [0, 0.99]: summed as
@@ -367,18 +392,54 @@ raster_fwd_fast_kernel(const __grid_constant__ GsRasterParams p, const float4* _
     const int64_t pix = (int64_t)py * p.image_width + px;
 #pragma unroll
     for (int c = 0; c < FP; ++c)
-      if (c_base + c < F) image[pix * F + c_base + c] = acc[c];
+      if (c_base + c < F) image[pix * F + c_base + c] = from_f32<TF>(acc[c]);
     if (first_slice) image_alpha[pix] = W;
   }
 }
 
 bool raster_fast_supported(const GsRasterParams& p) {
-  return p.dtype == GS_F32 && p.tile_size == kFastTile && (!p.antialias || p.num_features <= 7) &&
+  return (p.dtype == GS_F32 || p.dtype == GS_BF16) && p.tile_size == kFastTile && (!p.antialias || p.num_features <= 7) &&
          p.use_alpha_blending && (fast_feature_pad(p.num_features) != 0 || xwide_features(p.num_features)) &&
          p.num_points < (1ll << 31);
 }
 
 size_t raster_fast_workspace_bytes(const GsRasterParams& p) { return fast_layout(p).total; }
+
+// GS_BF16 (8..256 channels, no antialiasing): the f32 kernel's modes instantiated over bf16 rows
+static int raster_fwd_fast_bf16(const GsRasterParams& p, const RasterArgs& a, const float4* rec,
+                                const __nv_bfloat16* featP, const unsigned char* cmask, bool vis, cudaStream_t st) {
+  using bf16 = __nv_bfloat16;
+  const FastLayout L = fast_layout(p);
+  const int tiles = tiles_wide(p) * tiles_high(p);
+  if (xwide_features(p.num_features)) {   // one CTA per (tile, 64-channel slice)
+    const dim3 grid(tiles, L.FP / kXwideSlice);
+#define GS_FWD_XW16(VISV)                                                                                          \
+  raster_fwd_fast_kernel<kXwideSlice, VISV, 64, true, false, true, bf16><<<grid, kFwdThreads, 0, st>>>(            \
+      p, rec, featP, a.tile_ranges, a.overlap_to_point, (bf16*)a.image, (float*)a.image_alpha, (float*)a.visibility, \
+      cmask)
+    if (vis) GS_FWD_XW16(true); else GS_FWD_XW16(false);
+#undef GS_FWD_XW16
+    GS_LAUNCH_CHECK();
+    return GS_OK;
+  }
+#define GS_FWD_LAUNCH16(FPV, VISV, BATCHV)                                                                         \
+  GS_CUDA(launch_background(raster_fwd_fast_kernel<FPV, VISV, BATCHV, true, false, false, bf16>, dim3(tiles),     \
+                            dim3(kFwdThreads), 0, st, p, rec, featP, a.tile_ranges, a.overlap_to_point,           \
+                            (bf16*)a.image, (float*)a.image_alpha, (float*)a.visibility, cmask))
+#define GS_FWD_CASE16(FPV, BATCHV) \
+  case FPV: if (vis) GS_FWD_LAUNCH16(FPV, true, BATCHV); else GS_FWD_LAUNCH16(FPV, false, BATCHV); break
+  switch (L.FP) {
+    GS_FWD_CASE16(8, 128);
+    GS_FWD_CASE16(16, 64);
+    GS_FWD_CASE16(40, 64);
+    GS_FWD_CASE16(64, 64);
+    default: GS_UNSUPPORTED("rasterizer forward (bf16): %d feature channels", p.num_features);
+  }
+#undef GS_FWD_CASE16
+#undef GS_FWD_LAUNCH16
+  GS_LAUNCH_CHECK();
+  return GS_OK;
+}
 
 int raster_fwd_fast(const GsRasterParams& p, const RasterArgs& a, cudaStream_t st) {
   int rc = raster_fast_pack(p, a, /*forward=*/true, /*features=*/true, st);
@@ -389,9 +450,11 @@ int raster_fwd_fast(const GsRasterParams& p, const RasterArgs& a, cudaStream_t s
   unsigned char* ws = (unsigned char*)a.workspace;
   const unsigned char* cmask = ws + L.off_mask;
   const float4* rec = (const float4*)(ws + (p.antialias ? L.off_recB : L.off_recF));
-  const float* featP = fast_feature_rows(p, a);
   const int tiles = tiles_wide(p) * tiles_high(p);
   const bool vis = p.compute_visibility && a.visibility != nullptr;
+  if (p.dtype == GS_BF16)
+    return raster_fwd_fast_bf16(p, a, rec, (const __nv_bfloat16*)fast_feature_rows(p, a), cmask, vis, st);
+  const float* featP = (const float*)fast_feature_rows(p, a);
   if (xwide_features(p.num_features)) {   // one CTA per (tile, 64-channel slice)
     const dim3 grid(tiles, L.FP / kXwideSlice);
 #define GS_FWD_XW(VISV)                                                                                            \

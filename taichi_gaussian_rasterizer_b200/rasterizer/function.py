@@ -5,6 +5,10 @@ Operator surface of taichi_splatting/rasterizer/function.py: ``rasterize_with_ti
 differentiable w.r.t. gaussians2d and features; image_weight, visibility and point_heuristic are
 not; point_heuristic is returned zero-filled by forward and filled in place by backward.
 Extension: with ``RasterConfig.differentiable_weight`` (alpha blending only) image_weight is differentiable too.
+Extension: bfloat16 features with float32 gaussians2d.  The image is bfloat16 (the f32 blend rounded once),
+image_weight, visibility and point_heuristic stay float32.  8..256 channels with tile_size 16, alpha blending and no
+antialiasing run on bf16 kernels (half the feature, image and image-gradient bytes); any other configuration renders
+``features.float()`` and rounds the image, which is what the caller would get doing that cast.
 The kernels are csrc/raster_fast_*.cu (f32 / blending / tile 16) and csrc/raster_generic.cu.
 
 Two knobs the reference does not have (module level, defaults give reference parity):
@@ -45,7 +49,7 @@ def set_raster_options(emulate_stale_tail: Optional[bool] = None,
 
 def _raster_params(config: RasterConfig, dtype, image_size, F, V, K, pts_grad, feat_grad):
   return N.GsRasterParams(
-    dtype=N.dtype_code(dtype), image_width=int(image_size[0]), image_height=int(image_size[1]),
+    dtype=N.dtype_code(dtype, raster=True), image_width=int(image_size[0]), image_height=int(image_size[1]),
     tile_size=config.tile_size, num_features=F, antialias=int(config.antialias),
     use_alpha_blending=int(config.use_alpha_blending), compute_visibility=int(config.compute_visibility),
     compute_point_heuristic=int(config.compute_point_heuristic), points_requires_grad=int(pts_grad),
@@ -64,7 +68,7 @@ class _RasterFunction(torch.autograd.Function):
     V, F = features.shape
     K = overlap_to_point.shape[0]
     w, h = int(image_size[0]), int(image_size[1])
-    image_feature = torch.empty((h, w, F), dtype=dtype, device=device)
+    image_feature = torch.empty((h, w, F), dtype=features.dtype, device=device)   # bf16 features: a bf16 image
     image_alpha = torch.empty((h, w), dtype=dtype, device=device)
 
     if config.compute_point_heuristic:
@@ -76,7 +80,8 @@ class _RasterFunction(torch.autograd.Function):
     else:
       visibility = torch.empty((0,), dtype=dtype, device=device)
 
-    params = _raster_params(config, dtype, image_size, F, V, K, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+    params = _raster_params(config, features.dtype, image_size, F, V, K, ctx.needs_input_grad[0],
+                            ctx.needs_input_grad[1])
     lib = N.lib()
     ws = N.workspace(lib.gs_raster_workspace_bytes(ctypes.byref(params)), device)
     N.call("gs_raster_fwd", ctypes.byref(params), N.ptr(gaussians), N.ptr(features), N.ptr(tile_overlap_ranges), N.ptr(overlap_to_point),
@@ -105,7 +110,8 @@ class _RasterFunction(torch.autograd.Function):
     if grad_image_feature is None:
       grad_image_feature = torch.zeros_like(image_feature)
     grad_gaussians = torch.empty_like(gaussians) if need_g else None   # zeroed by the callee
-    grad_features = torch.empty_like(features) if need_f else None
+    # bf16 features: the kernels accumulate an f32 gradient, rounded to the features' dtype for autograd below
+    grad_features = torch.empty(features.shape, dtype=gaussians.dtype, device=features.device) if need_f else None
     params = ctx.params
     params.points_requires_grad = int(need_g)
     params.features_requires_grad = int(need_f)
@@ -122,6 +128,8 @@ class _RasterFunction(torch.autograd.Function):
         N.ptr(grad_image_feature.contiguous()), N.ptr(ctx.saved_tensors[3]), N.ptr(grad_alpha.contiguous()),
         N.ptr(grad_gaussians), N.ptr(grad_features), N.ptr(heur), N.ptr(ctx.workspace),
         ctypes.c_size_t(ctx.workspace.numel()), N.stream_ptr(gaussians.device))
+    if grad_features is not None and grad_features.dtype != features.dtype:
+      grad_features = grad_features.to(features.dtype)
     return grad_gaussians, grad_features, None, None, None, None
 
 
@@ -149,16 +157,31 @@ def rasterize_with_tiles(gaussians2d: torch.Tensor, features: torch.Tensor,
   N.require_cuda(gaussians2d, features, overlap_to_point, tile_overlap_ranges)
   assert features.ndim == 2 and features.shape[0] == gaussians2d.shape[0], \
     f"features must be NxF, got {features.shape} for {gaussians2d.shape[0]} gaussians"
-  assert features.dtype == gaussians2d.dtype, f"dtype mismatch {features.dtype} != {gaussians2d.dtype}"
+  bf16 = features.dtype == torch.bfloat16
+  if bf16 and gaussians2d.dtype != torch.float32:
+    raise TypeError(f"bfloat16 features need float32 gaussians2d, got {gaussians2d.dtype}")
+  if features.dtype == torch.float16:
+    raise TypeError("float16 features are not supported: use bfloat16 (with float32 gaussians2d) or float32")
+  assert bf16 or features.dtype == gaussians2d.dtype, f"dtype mismatch {features.dtype} != {gaussians2d.dtype}"
   assert overlap_to_point.dtype == torch.int32 and tile_overlap_ranges.dtype == torch.int32
   ranges = tile_overlap_ranges.reshape(-1, 2).contiguous()
   th = -(-int(image_size[1]) // config.tile_size)
   tw = -(-int(image_size[0]) // config.tile_size)
   assert ranges.shape[0] == th * tw, f"expected {th * tw} tile ranges for image {tuple(image_size)}, got {ranges.shape[0]}"
 
+  upcast = bf16 and not bf16_native(features.shape[1], config)
   image, image_weight, point_heuristic, visibility = _RasterFunction.apply(
-    gaussians2d.contiguous(), features.contiguous(), overlap_to_point.contiguous(), ranges, image_size, config)
+    gaussians2d.contiguous(), (features.float() if upcast else features).contiguous(), overlap_to_point.contiguous(),
+    ranges, image_size, config)
+  if upcast:
+    image = image.to(torch.bfloat16)
   return RasterOut(image, image_weight, point_heuristic, visibility)
+
+
+def bf16_native(num_features: int, config: RasterConfig) -> bool:
+  """Whether bfloat16 features of this width and config run on the bf16 kernels (GS_BF16); otherwise they are rendered
+  as float32 and the image is rounded.  More than 256 channels go to the kernels too, which reject them."""
+  return num_features >= 8 and config.tile_size == 16 and config.use_alpha_blending and not config.antialias
 
 
 def rasterize(gaussians2d: torch.Tensor, depth: torch.Tensor,

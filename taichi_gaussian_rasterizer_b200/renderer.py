@@ -56,6 +56,9 @@ def render_gaussians(
       (pass a (1,) int32 CUDA tensor as ``overlap_total_out`` to receive K and compare it with the capacity now and
       then).  Same kernels and the same values as the default path; forward + backward of any number of views can be
       captured in ONE CUDA graph (bench.py).  f32 gaussians only.
+    bfloat16 plain features (use_sh=False, float32 geometry): the image is bfloat16 and the feature rows stay bf16 from
+      the gather to the rasterizer (see rasterizer.function); with render_depth the visible rows are widened to
+      float32 behind the f32 depth channels and only the returned image is rounded back to bf16 (depth, depth_var f32).
 
   Returns:
     Rendering - rendered image, with optional depth / depth variance and per point statistics
@@ -112,10 +115,19 @@ def render_gaussians(
     else:
       features = gaussians.feature[indexes]
 
-  return render_projected(indexes, gaussians2d, features, depths, camera_params, config,
-                          render_depth=render_depth, use_depth16=use_depth16,
-                          render_median_depth=render_median_depth, mapper_front=early.get("front"),
-                          before_total_sync=fill_features, features_include_depth=depth_in_features)
+  rendering = render_projected(indexes, gaussians2d, features, depths, camera_params, config,
+                               render_depth=render_depth, use_depth16=use_depth16,
+                               render_median_depth=render_median_depth, mapper_front=early.get("front"),
+                               before_total_sync=fill_features, features_include_depth=depth_in_features)
+  return _bf16_image(rendering, gaussians.feature, use_sh, render_depth)
+
+
+def _bf16_image(rendering, feature, use_sh, render_depth):
+  """bf16 plain features with render_depth were rendered widened to float32 (the depth channels need it): round the
+  returned image back to the features' dtype."""
+  if not use_sh and render_depth and feature.dtype == torch.bfloat16:
+    return replace(rendering, image=rendering.image.to(torch.bfloat16))
+  return rendering
 
 
 def _render_gaussians_static(gaussians, camera_params, config, use_sh, render_depth, use_depth16, render_median_depth,
@@ -146,7 +158,7 @@ def _render_gaussians_static(gaussians, camera_params, config, use_sh, render_de
     assert sh_colors is None
     assert len(gaussians.feature.shape) == 2, f"Features must be (N, C) if use_sh=False, got {gaussians.feature.shape}"
     features = _visible_features(gaussians.feature, indexes, count, depths if render_depth else None)
-    assert features is not None, "overlap_capacity without SH: dense contiguous float32 features"
+    assert features is not None, "overlap_capacity without SH: dense contiguous float32 or bfloat16 features"
   if render_depth and use_sh:
     features = torch.cat([depths, depths ** 2, features], dim=1)
   overlap_to_point, tile_ranges = map_front_to_tiles_capped(gaussians2d, count, front, size, config, overlap_capacity,
@@ -158,14 +170,14 @@ def _render_gaussians_static(gaussians, camera_params, config, use_sh, render_de
   if render_depth:
     depth2, image = _SplitDepthChannels.apply(image)
     depth_image, depth_var = compute_depth_variance(depth2, raster.image_weight)
-  return Rendering(
+  return _bf16_image(Rendering(
     image=image, image_weight=raster.image_weight, depth=depth_image, depth_var=depth_var,
     median_depth=(_median_depth(gaussians2d, depths, overlap_to_point, ranges, camera_params, config)
                   if render_median_depth else None),
     points_in_view=indexes, point_depth=depths, gaussians2d=gaussians2d,
     point_visibility=raster.visibility if config.compute_visibility else None,
     point_heuristic=raster.point_heuristic if config.compute_point_heuristic else None,
-    camera=camera_params, config=config, points_in_view_count=count)
+    camera=camera_params, config=config, points_in_view_count=count), gaussians.feature, use_sh, render_depth)
 
 
 class _VisibleFeatures(torch.autograd.Function):
@@ -173,7 +185,7 @@ class _VisibleFeatures(torch.autograd.Function):
   ``[depth, depth^2, feature[indexes]]`` assembled by ONE gather kernel (gs_gather_rows_strided) instead of
   ``feature[indexes]`` + ``torch.cat`` (renderer.py:152-153, 199-200 of the reference), the backward ONE scatter
   (gs_scatter_rows_strided: the indexes are unique, no atomics, no sort) instead of index_put with accumulate + the
-  slices of the cat.  ``count`` (optional, (1,) int32 on the device): only the first count[0] rows of ``indexes`` are
+  slices of the cat.  bfloat16 rows (no depth channels) go through the 2-byte entry points *_u16.  ``count`` (optional, (1,) int32 on the device): only the first count[0] rows of ``indexes`` are
   valid (read-back free path); rows past it are left uninitialised / ignored."""
 
   @staticmethod
@@ -183,7 +195,8 @@ class _VisibleFeatures(torch.autograd.Function):
     v, c = indexes.shape[0], feature.shape[1]
     extra = 0 if depths is None else 2
     out = torch.empty((v, c + extra), dtype=feature.dtype, device=feature.device)
-    N.call("gs_gather_rows_strided", ctypes.c_int64(v), ctypes.c_int32(c), N.ptr(feature), N.ptr(indexes),
+    u16 = feature.dtype == torch.bfloat16
+    N.call("gs_gather_rows_strided_u16" if u16 else "gs_gather_rows_strided", ctypes.c_int64(v), ctypes.c_int32(c), N.ptr(feature), N.ptr(indexes),
            N.ptr(count), N.ptr(out), ctypes.c_int32(c + extra), ctypes.c_int32(extra), N.stream_ptr(feature.device))
     if depths is not None:
       out[:, 0:1] = depths
@@ -203,7 +216,7 @@ class _VisibleFeatures(torch.autograd.Function):
     g_feature = g_depths = None
     if ctx.needs_input_grad[0]:
       g_feature = torch.empty((ctx.rows, c), dtype=g.dtype, device=g.device)
-      N.call("gs_scatter_rows_strided", ctypes.c_int64(v), ctypes.c_int32(c), N.ptr(g), ctypes.c_int32(width),
+      N.call("gs_scatter_rows_strided_u16" if g.dtype == torch.bfloat16 else "gs_scatter_rows_strided", ctypes.c_int64(v), ctypes.c_int32(c), N.ptr(g), ctypes.c_int32(width),
              ctypes.c_int32(ctx.extra), N.ptr(indexes), N.ptr(count), ctypes.c_int64(ctx.rows), N.ptr(g_feature),
              N.stream_ptr(g.device))
     if depths is not None and ctx.needs_input_grad[3]:
@@ -213,9 +226,14 @@ class _VisibleFeatures(torch.autograd.Function):
 
 def _visible_features(feature, indexes, count=None, depths=None):
   """feature[indexes] (with the depth channels in front when ``depths`` is given) through the kernels above when the
-  features are dense contiguous float32 on the GPU; None otherwise (the caller indexes with torch)."""
-  if feature.is_cuda and feature.dtype == torch.float32 and feature.ndim == 2 and feature.is_contiguous() and \
-      (depths is None or depths.dtype == torch.float32):
+  features are dense contiguous float32 or bfloat16 on the GPU; None otherwise (the caller indexes with torch).
+  bfloat16 with ``depths``: the gathered rows widened to float32 behind the f32 depth channels."""
+  if not (feature.is_cuda and feature.ndim == 2 and feature.is_contiguous()):
+    return None
+  if feature.dtype == torch.bfloat16 and (depths is None or depths.dtype == torch.float32):
+    rows = _VisibleFeatures.apply(feature, indexes.contiguous(), count, None)
+    return rows if depths is None else torch.cat([depths, depths * depths, rows.float()], dim=1)
+  if feature.dtype == torch.float32 and (depths is None or depths.dtype == torch.float32):
     return _VisibleFeatures.apply(feature, indexes.contiguous(), count, depths)
   return None
 
