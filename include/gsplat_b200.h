@@ -118,12 +118,15 @@ int gs_sh_fwd_counted(const GsSHParams* p, const void* params, const void* posit
                       void* out, void* stream);
 
 /* grad_out (V,K) -> grad_params (M,K,D) grad_positions (M,3) grad_camera_pos (3); each fully
- * written (zeroed then accumulated; repeated indexes are summed).  Any may be NULL. */
+ * written (zeroed then accumulated; repeated indexes are summed).  Any may be NULL.  With p->indexes_sorted_unique,
+ * f32, K = 3 and D in {1, 4, 9, 16} the rows are written densely without atomics (16 B units at D = 4, 16 when the
+ * pointers are 16 B aligned, 4 B units otherwise); every other shape takes the generic atomic kernel. */
 int gs_sh_bwd(const GsSHParams* p, const void* params, const void* positions,
               const int64_t* indexes, const void* camera_pos, const void* grad_out,
               void* grad_params, void* grad_positions, void* grad_camera_pos, void* stream);
 
-/* Deferred coefficient gradient for a multi-view batch (f32, K = 3, D in {4, 16}).  evaluate_sh_at_kernel.grad
+/* Deferred coefficient gradient for a multi-view batch (f32, K = 3, D in {1, 4, 9, 16}; any other shape returns
+ * GS_ERR_UNSUPPORTED).  evaluate_sh_at_kernel.grad
  * (spherical_harmonics.py:154-161) followed by autograd's accumulation rewrites the whole (M,K,D) gradient once per
  * view; the coefficient gradient of a view is the outer product of the masked colour gradient with the basis of the
  * viewing direction, so a view only has to keep K floats per gaussian:
@@ -134,7 +137,8 @@ int gs_sh_bwd(const GsSHParams* p, const void* params, const void* positions,
  *                    ((M,K) and (3,) floats), num_views <= GS_SH_MAX_DEFERRED_VIEWS.  With p->accumulate_params = 0
  *                    the rows are OVERWRITTEN with the sum (zeroed when num_views = 0): the first flush of a batch
  *                    then needs neither a zero fill of grad_params before nor a read of it.
- * p->num_points = M, p->num_indexes = V (stage only). */
+ * p->num_points = M, p->num_indexes = V (stage only).  grad_params may sit at any 4 B aligned address (a slice of a
+ * flat gradient bucket): the flush moves 16 B units only when grad_params is 16 B aligned, 4 B units otherwise. */
 #define GS_SH_MAX_DEFERRED_VIEWS 16
 int gs_sh_bwd_stage(const GsSHParams* p, const void* forward_out, const int64_t* indexes, const void* grad_out,
                     void* staged, void* stream);
@@ -145,13 +149,13 @@ int gs_sh_bwd_stage_counted(const GsSHParams* p, const void* forward_out, const 
 int gs_sh_bwd_flush(const GsSHParams* p, int32_t num_views, const void* const* staged,
                     const void* const* camera_positions, const void* positions, void* grad_params, void* stream);
 
-/* Batched evaluation for the views of a multi-view batch (f32, K = 3, D in {4, 16}): evaluate_sh_at_kernel
+/* Batched evaluation for the views of a multi-view batch (f32, K = 3, D in {1, 4, 9, 16}): evaluate_sh_at_kernel
  * (spherical_harmonics.py:118-134) reads the 4 K D byte coefficient row of every visible gaussian once per VIEW;
  * gs_sh_fwd_views reads every row once per BATCH and writes one dense colour tensor (M,K) per view (outs /
  * camera_positions: HOST arrays of num_views device pointers, num_views <= GS_SH_MAX_DEFERRED_VIEWS; same arithmetic
  * and clamp as gs_sh_fwd).  A view then takes its visible rows with gs_gather_rows_counted: out[j] = src[indexes[j]]
  * for j < *count_dev (count_dev NULL: j < capacity), rows of row_floats = 3 floats — the count may still be on the
- * device, as for gs_sh_fwd_counted. */
+ * device, as for gs_sh_fwd_counted.  params is read in 16 B units only at D = 4, 16 and when 16 B aligned. */
 int gs_sh_fwd_views(const GsSHParams* p, int32_t num_views, const void* params, const void* positions,
                     const void* const* camera_positions, void* const* outs, void* stream);
 int gs_gather_rows_counted(int64_t capacity, int32_t row_floats, const void* src, const int64_t* indexes,

@@ -184,17 +184,25 @@ constexpr int kSHDenseBlock = 128;
 // FROM_OUT: `params` holds the forward OUTPUT (V, K) instead of the coefficients.  The coefficient gradient
 // g_k b_j needs the coefficients only for the clamp mask, and v in (0, 1) <=> clamp(v) in (0, 1): when no position /
 // camera gradient is asked for, the 4 K D byte row gather per gaussian (a third of the kernel's traffic) is skipped.
-template <int K, int D, bool FILL, bool FROM_OUT = false>
+//
+// A16: the gathered coefficient rows (unless FROM_OUT) and the gradient rows move in 16 B units, which needs K D a
+// multiple of 4 and 16 B aligned `params` / `grad_params`.  !A16 moves them in 4 B units (4 B cp.async for the gather),
+// at any alignment: rows of 3 or 27 floats (D = 1, 9) at idx * 12 B or idx * 108 B, or misaligned pointers at D = 4, 16.
+// Odd row lengths sit back to back in shared memory (odd stride: conflict-free scalar LDS / STS per thread).
+template <int K, int D, bool FILL, bool FROM_OUT = false, bool A16 = true>
 __global__ void __launch_bounds__(kSHDenseBlock, 6)
 sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restrict__ params,
                     const float* __restrict__ positions, const int64_t* __restrict__ indexes,
                     const float* __restrict__ cam, const float* __restrict__ grad_out, float* __restrict__ grad_params,
                     float* __restrict__ grad_positions, float* __restrict__ grad_cam) {
   constexpr int RL = K * D, R4 = RL / 4, S4 = (R4 + 1) | 1;  // odd float4 stride: conflict-free LDS.128 per thread
-  static_assert(RL % 4 == 0, "row length must be a multiple of 4 floats");
-  __shared__ float4 s_row[kSHDenseBlock * S4];
+  constexpr bool V4 = RL % 4 == 0;                            // rows of whole float4s: padded rows in shared memory
+  constexpr int SR = V4 ? 4 * S4 : RL;                        // shared row stride in floats
+  static_assert(V4 || !A16, "16 B row units need a row length that is a multiple of 4 floats");
+  __shared__ float4 s_row[V4 ? kSHDenseBlock * S4 : (kSHDenseBlock * RL + 3) / 4];
   __shared__ int64_t s_idx[kSHDenseBlock + 1];
   __shared__ float s_red[3][kSHDenseBlock / 32];
+  float* s_f = reinterpret_cast<float*>(s_row);
 
   const int t = threadIdx.x;
   const int64_t i0 = (int64_t)blockIdx.x * kSHDenseBlock;
@@ -205,13 +213,25 @@ sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restric
   __syncthreads();
 
   if (!FROM_OUT) {
+    if constexpr (A16) {
 #pragma unroll
-    for (int m = 0; m < R4; ++m) {  // R4 independent 16 B cp.async gathers in flight per thread, no staging registers
-      const int q = t + m * kSHDenseBlock, r = q / R4, part = q - r * R4;
-      if (q < nrows * R4) {
-        const unsigned dst = (unsigned)__cvta_generic_to_shared(&s_row[r * S4 + part]);
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst),
-                     "l"(reinterpret_cast<const float4*>(params + s_idx[r + 1] * RL) + part) : "memory");
+      for (int m = 0; m < R4; ++m) {  // R4 independent 16 B cp.async gathers in flight per thread, no staging registers
+        const int q = t + m * kSHDenseBlock, r = q / R4, part = q - r * R4;
+        if (q < nrows * R4) {
+          const unsigned dst = (unsigned)__cvta_generic_to_shared(&s_row[r * S4 + part]);
+          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst),
+                       "l"(reinterpret_cast<const float4*>(params + s_idx[r + 1] * RL) + part) : "memory");
+        }
+      }
+    } else {
+#pragma unroll 4
+      for (int m = 0; m < RL; ++m) {  // RL 4 B cp.async gathers per thread; consecutive lanes read consecutive floats
+        const int q = t + m * kSHDenseBlock, r = q / RL, part = q - r * RL;
+        if (q < nrows * RL) {
+          const unsigned dst = (unsigned)__cvta_generic_to_shared(&s_f[r * SR + part]);
+          asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(params + s_idx[r + 1] * RL + part)
+                       : "memory");
+        }
       }
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
@@ -232,6 +252,7 @@ sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restric
 #pragma unroll
     for (int j = 0; j < D; ++j) gb[j] = 0.f;
     float4* row = s_row + t * S4;
+    float* row_f = s_f + t * SR;
 #pragma unroll
     for (int k = 0; k < K; ++k) {
       float v;
@@ -239,10 +260,15 @@ sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restric
       if (FROM_OUT) {
         v = params[i * K + k];  // the clamped forward value: inside (0, 1) exactly when the unclamped one is
       } else {
+        if constexpr (D % 4 == 0) {
 #pragma unroll
-        for (int j4 = 0; j4 < D / 4; ++j4) {
-          const float4 q4 = row[k * (D / 4) + j4];
-          c[4 * j4] = q4.x; c[4 * j4 + 1] = q4.y; c[4 * j4 + 2] = q4.z; c[4 * j4 + 3] = q4.w;
+          for (int j4 = 0; j4 < D / 4; ++j4) {
+            const float4 q4 = row[k * (D / 4) + j4];
+            c[4 * j4] = q4.x; c[4 * j4 + 1] = q4.y; c[4 * j4 + 2] = q4.z; c[4 * j4 + 3] = q4.w;
+          }
+        } else {
+#pragma unroll
+          for (int j = 0; j < D; ++j) c[j] = row_f[k * D + j];
         }
         float acc = 0.f;
 #pragma unroll
@@ -254,9 +280,14 @@ sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restric
 #pragma unroll
         for (int j = 0; j < D; ++j) gb[j] += g * c[j];
       }
+      if constexpr (D % 4 == 0) {
 #pragma unroll
-      for (int j4 = 0; j4 < D / 4; ++j4)
-        row[k * (D / 4) + j4] = make_float4(g * b[4 * j4], g * b[4 * j4 + 1], g * b[4 * j4 + 2], g * b[4 * j4 + 3]);
+        for (int j4 = 0; j4 < D / 4; ++j4)
+          row[k * (D / 4) + j4] = make_float4(g * b[4 * j4], g * b[4 * j4 + 1], g * b[4 * j4 + 2], g * b[4 * j4 + 3]);
+      } else {
+#pragma unroll
+        for (int j = 0; j < D; ++j) row_f[k * D + j] = g * b[j];
+      }
     }
     if (!FROM_OUT && (grad_positions || grad_cam)) {
       float gx[D], gy[D], gz[D];
@@ -273,12 +304,20 @@ sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restric
   }
   __syncthreads();
 
+  if constexpr (A16) {
 #pragma unroll
-  for (int m = 0; m < R4; ++m) {
-    const int q = t + m * kSHDenseBlock, r = q / R4, part = q - r * R4;
-    if (q < nrows * R4) {
-      float4* dst = reinterpret_cast<float4*>(grad_params + s_idx[r + 1] * RL) + part;
-      *dst = s_row[r * S4 + part];
+    for (int m = 0; m < R4; ++m) {
+      const int q = t + m * kSHDenseBlock, r = q / R4, part = q - r * R4;
+      if (q < nrows * R4) {
+        float4* dst = reinterpret_cast<float4*>(grad_params + s_idx[r + 1] * RL) + part;
+        *dst = s_row[r * S4 + part];
+      }
+    }
+  } else {
+#pragma unroll 4
+    for (int m = 0; m < RL; ++m) {
+      const int q = t + m * kSHDenseBlock, r = q / RL, part = q - r * RL;
+      if (q < nrows * RL) grad_params[s_idx[r + 1] * RL + part] = s_f[r * SR + part];
     }
   }
 
@@ -293,8 +332,13 @@ sh_bwd_dense_kernel(const __grid_constant__ GsSHParams p, const float* __restric
         else if (tail) { lo = s_idx[nrows] + 1; hi = p.num_points; }
         else break;
         if (hi <= lo) continue;
-        float4* gp4 = reinterpret_cast<float4*>(grad_params + lo * RL);
-        for (int64_t q = t; q < (hi - lo) * R4; q += kSHDenseBlock) gp4[q] = z4;
+        if constexpr (A16) {
+          float4* gp4 = reinterpret_cast<float4*>(grad_params + lo * RL);
+          for (int64_t q = t; q < (hi - lo) * R4; q += kSHDenseBlock) gp4[q] = z4;
+        } else {
+          float* gp = grad_params + lo * RL;
+          for (int64_t q = t; q < (hi - lo) * RL; q += kSHDenseBlock) gp[q] = 0.f;
+        }
         if (grad_positions)
           for (int64_t q = t; q < (hi - lo) * 3; q += kSHDenseBlock) grad_positions[lo * 3 + q] = 0.f;
       }
@@ -344,13 +388,17 @@ struct SHFlushViews {
 };
 
 // OVERWRITE: grad_params = the batch's sum (the caller knows the rows hold nothing yet: no zero fill before, no read here)
-template <int K, int D, bool OVERWRITE>
+// A16: grad_params is 16 B aligned and read / written in float4 units.  A block's rows are one contiguous span of
+// 128 K D floats, a multiple of four at every D, so the span of every block starts 16 B aligned as well; rows of 3 or
+// 27 floats (D = 1, 9) sit back to back in shared memory (odd stride: conflict-free scalar STS) and go out as the
+// span's float4s plus, in the last block, a tail of at most three floats.  !A16: 4 B units, at any alignment.
+template <int K, int D, bool OVERWRITE, bool A16 = true>
 __global__ void __launch_bounds__(kSHDenseBlock, 4)
 sh_bwd_flush_kernel(int64_t n, int num_views, const __grid_constant__ SHFlushViews views,
                     const float* __restrict__ positions, float* __restrict__ grad_params) {
   constexpr int RL = K * D, R4 = RL / 4, S4 = (R4 + 1) | 1;   // odd float4 stride: conflict-free LDS.128 / STS.128
-  static_assert(RL % 4 == 0, "row length must be a multiple of 4 floats");
-  __shared__ float4 s_row[kSHDenseBlock * S4];
+  constexpr bool V4 = RL % 4 == 0;                             // rows of whole float4s: padded rows in shared memory
+  __shared__ float4 s_row[V4 ? kSHDenseBlock * S4 : kSHDenseBlock * RL / 4];
   const int t = threadIdx.x;
   const int64_t i0 = (int64_t)blockIdx.x * kSHDenseBlock, i = i0 + t;
   const int nrows = (int)min((int64_t)kSHDenseBlock, n - i0);
@@ -377,21 +425,58 @@ sh_bwd_flush_kernel(int64_t n, int num_views, const __grid_constant__ SHFlushVie
         for (int j = 0; j < D; ++j) acc[k * D + j] = fmaf(g[k], b[j], acc[k * D + j]);
     }
   }
+  float* s_f = reinterpret_cast<float*>(s_row);
+  if constexpr (V4) {
 #pragma unroll
-  for (int q4 = 0; q4 < R4; ++q4)
-    s_row[t * S4 + q4] = make_float4(acc[4 * q4], acc[4 * q4 + 1], acc[4 * q4 + 2], acc[4 * q4 + 3]);
+    for (int q4 = 0; q4 < R4; ++q4)
+      s_row[t * S4 + q4] = make_float4(acc[4 * q4], acc[4 * q4 + 1], acc[4 * q4 + 2], acc[4 * q4 + 3]);
+  } else {
+#pragma unroll
+    for (int q = 0; q < RL; ++q) s_f[t * RL + q] = acc[q];
+  }
   __syncthreads();
-  float4* dst = reinterpret_cast<float4*>(grad_params + i0 * RL);   // the block's rows are contiguous
+  if constexpr (V4 && A16) {
+    float4* dst = reinterpret_cast<float4*>(grad_params + i0 * RL);   // the block's rows are contiguous
 #pragma unroll
-  for (int m = 0; m < R4; ++m) {
-    const int q = t + m * kSHDenseBlock, r = q / R4, part = q - r * R4;
-    if (q < nrows * R4) {
-      float4 a = s_row[r * S4 + part];
-      if (!OVERWRITE) {
-        const float4 o = dst[q];
-        a.x += o.x; a.y += o.y; a.z += o.z; a.w += o.w;
+    for (int m = 0; m < R4; ++m) {
+      const int q = t + m * kSHDenseBlock, r = q / R4, part = q - r * R4;
+      if (q < nrows * R4) {
+        float4 a = s_row[r * S4 + part];
+        if (!OVERWRITE) {
+          const float4 o = dst[q];
+          a.x += o.x; a.y += o.y; a.z += o.z; a.w += o.w;
+        }
+        dst[q] = a;
       }
-      dst[q] = a;
+    }
+  } else if constexpr (A16) {   // odd row length: s_row holds the span as it lies in global memory
+    float4* dst = reinterpret_cast<float4*>(grad_params + i0 * RL);
+    const int nf = nrows * RL, n4 = nf >> 2;
+#pragma unroll
+    for (int m = 0; m < (RL + 3) / 4; ++m) {
+      const int q = t + m * kSHDenseBlock;
+      if (q < n4) {
+        float4 a = s_row[q];
+        if (!OVERWRITE) {
+          const float4 o = dst[q];
+          a.x += o.x; a.y += o.y; a.z += o.z; a.w += o.w;
+        }
+        dst[q] = a;
+      }
+    }
+    if (t < nf - 4 * n4) {   // last block only: the span ends inside a float4
+      const int q = 4 * n4 + t;
+      grad_params[i0 * RL + q] = OVERWRITE ? s_f[q] : s_f[q] + grad_params[i0 * RL + q];
+    }
+  } else {
+    float* dst = grad_params + i0 * RL;
+#pragma unroll
+    for (int m = 0; m < RL; ++m) {
+      const int q = t + m * kSHDenseBlock, r = q / RL, part = q - r * RL;
+      if (q < nrows * RL) {
+        const float a = s_f[V4 ? r * 4 * S4 + part : q];
+        dst[q] = OVERWRITE ? a : a + dst[q];
+      }
     }
   }
 }
@@ -405,18 +490,27 @@ struct SHViewsOut {
   const float* cam[kSHMaxDeferred];
 };
 
-template <int K, int D>
+// A16: the rows are read as float4 (K D a multiple of 4 and `params` 16 B aligned); else one float at a time (rows of
+// 3 or 27 floats, or a misaligned `params`).  Either way the sum runs in sh_fwd_kernel's order, so the colours are
+// evaluate_sh_at's.
+template <int K, int D, bool A16 = true>
 __global__ void __launch_bounds__(128)
 sh_fwd_views_kernel(int64_t n, int num_views, const __grid_constant__ SHViewsOut views,
                     const float* __restrict__ params, const float* __restrict__ positions) {
+  static_assert(!A16 || (K * D) % 4 == 0, "float4 rows need K * D to be a multiple of 4");
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   float c[K * D];
-  const float4* r4 = reinterpret_cast<const float4*>(params + i * K * D);
+  if constexpr (A16) {
+    const float4* r4 = reinterpret_cast<const float4*>(params + i * K * D);
 #pragma unroll
-  for (int q = 0; q < K * D / 4; ++q) {
-    const float4 v = __ldg(r4 + q);
-    c[4 * q] = v.x; c[4 * q + 1] = v.y; c[4 * q + 2] = v.z; c[4 * q + 3] = v.w;
+    for (int q = 0; q < K * D / 4; ++q) {
+      const float4 v = __ldg(r4 + q);
+      c[4 * q] = v.x; c[4 * q + 1] = v.y; c[4 * q + 2] = v.z; c[4 * q + 3] = v.w;
+    }
+  } else {
+#pragma unroll
+    for (int q = 0; q < K * D; ++q) c[q] = __ldg(params + i * K * D + q);
   }
   const float px = positions[3 * i], py = positions[3 * i + 1], pz = positions[3 * i + 2];
   for (int v = 0; v < num_views; ++v) {
@@ -427,11 +521,16 @@ sh_fwd_views_kernel(int64_t n, int num_views, const __grid_constant__ SHViewsOut
     sh_basis<float, D>(dx * inv, dy * inv, dz * inv, b);
 #pragma unroll
     for (int k = 0; k < K; ++k) {
-      float acc = 0.f;   // same summation order as sh_fwd_kernel (groups of four)
+      float acc = 0.f;
+      if constexpr (D % 4 == 0) {   // same summation order as sh_fwd_kernel: groups of four ...
 #pragma unroll
-      for (int j = 0; j < D / 4; ++j)
-        acc += b[4 * j] * c[k * D + 4 * j] + b[4 * j + 1] * c[k * D + 4 * j + 1] + b[4 * j + 2] * c[k * D + 4 * j + 2] +
-               b[4 * j + 3] * c[k * D + 4 * j + 3];
+        for (int j = 0; j < D / 4; ++j)
+          acc += b[4 * j] * c[k * D + 4 * j] + b[4 * j + 1] * c[k * D + 4 * j + 1] +
+                 b[4 * j + 2] * c[k * D + 4 * j + 2] + b[4 * j + 3] * c[k * D + 4 * j + 3];
+      } else {                      // ... or one term at a time (its scalar branch)
+#pragma unroll
+        for (int j = 0; j < D; ++j) acc += b[j] * c[k * D + j];
+      }
       const float val = acc + 0.5f;
       views.out[v][i * K + k] = val < 0.f ? 0.f : (val > 1.f ? 1.f : val);
     }
@@ -756,6 +855,47 @@ static int check_sh(const GsSHParams* p, const char* who) {
   return GS_OK;
 }
 
+// The shapes the batched forward, the flush and the dense backward serve: f32, K = 3, degree 0..3
+static bool sh_fast_shape(const GsSHParams* p) {
+  return p->dtype == GS_F32 && p->num_channels == 3 &&
+         (p->num_coeffs == 1 || p->num_coeffs == 4 || p->num_coeffs == 9 || p->num_coeffs == 16);
+}
+
+static bool aligned16(const void* ptr) { return ((uintptr_t)ptr & 15) == 0; }
+
+template <int D, bool A16>
+static void launch_sh_dense(bool fill, bool from_out, const GsSHParams* p, const void* params, const void* positions,
+                            const int64_t* indexes, const void* cam, const void* grad_out, void* grad_params,
+                            void* grad_positions, void* grad_cam, cudaStream_t st) {
+  const unsigned blocks = (unsigned)ceil_div(p->num_indexes, kSHDenseBlock);
+#define GS_SH_DENSE(FILLV, FROMV)                                                                                  \
+  sh_bwd_dense_kernel<3, D, FILLV, FROMV, A16><<<blocks, kSHDenseBlock, 0, st>>>(                                 \
+      *p, (const float*)params, (const float*)positions, indexes, (const float*)cam, (const float*)grad_out,       \
+      (float*)grad_params, (float*)grad_positions, (float*)grad_cam)
+  if (fill) { if (from_out) GS_SH_DENSE(true, true); else GS_SH_DENSE(true, false); }
+  else { if (from_out) GS_SH_DENSE(false, true); else GS_SH_DENSE(false, false); }
+#undef GS_SH_DENSE
+}
+
+template <int D, bool A16>
+static void launch_sh_flush(bool overwrite, int64_t n, int num_views, const SHFlushViews& views, const void* positions,
+                            void* grad_params, cudaStream_t st) {
+  const unsigned blocks = (unsigned)ceil_div(n, kSHDenseBlock);
+  if (overwrite)
+    sh_bwd_flush_kernel<3, D, true, A16><<<blocks, kSHDenseBlock, 0, st>>>(n, num_views, views, (const float*)positions,
+                                                                            (float*)grad_params);
+  else
+    sh_bwd_flush_kernel<3, D, false, A16><<<blocks, kSHDenseBlock, 0, st>>>(n, num_views, views, (const float*)positions,
+                                                                             (float*)grad_params);
+}
+
+template <int D, bool A16>
+static void launch_sh_fwd_views(int64_t n, int num_views, const SHViewsOut& views, const void* params,
+                                const void* positions, cudaStream_t st) {
+  sh_fwd_views_kernel<3, D, A16><<<(unsigned)ceil_div(n, 128), 128, 0, st>>>(n, num_views, views, (const float*)params,
+                                                                             (const float*)positions);
+}
+
 extern "C" {
 
 int gs_sh_fwd(const GsSHParams* p, const void* params, const void* positions, const int64_t* indexes,
@@ -794,8 +934,7 @@ int gs_sh_bwd(const GsSHParams* p, const void* params, const void* positions, co
   }
   cudaStream_t st = (cudaStream_t)stream;
   const size_t es = p->dtype == GS_F32 ? 4 : 8;
-  const bool dense = p->indexes_sorted_unique && p->dtype == GS_F32 && grad_params != nullptr && p->num_indexes > 0 &&
-                     p->num_channels == 3 && (p->num_coeffs == 16 || p->num_coeffs == 4);
+  const bool dense = p->indexes_sorted_unique && grad_params != nullptr && p->num_indexes > 0 && sh_fast_shape(p);
   const bool from_out = p->params_is_forward_output != 0;
   if (from_out && (!dense || grad_positions || grad_camera_pos)) {
     set_error("gs_sh_bwd: params_is_forward_output needs the dense path and no position / camera gradient");
@@ -809,20 +948,17 @@ int gs_sh_bwd(const GsSHParams* p, const void* params, const void* positions, co
   if (p->num_indexes == 0) return GS_OK;
   GS_CHECK_ARG(params && positions && indexes && camera_pos && grad_out, "gs_sh_bwd: null tensor");
   if (dense) {
-    const unsigned blocks = (unsigned)ceil_div(p->num_indexes, kSHDenseBlock);
-#define GS_SH_DENSE_(DD, FILLV, FROMV)                                                                            \
-    sh_bwd_dense_kernel<3, DD, FILLV, FROMV><<<blocks, kSHDenseBlock, 0, st>>>(                                  \
-        *p, (const float*)params, (const float*)positions, indexes, (const float*)camera_pos,                   \
-        (const float*)grad_out, (float*)grad_params, (float*)grad_positions, (float*)grad_camera_pos)
-#define GS_SH_DENSE(DD, FILLV) \
-    do { if (from_out) GS_SH_DENSE_(DD, FILLV, true); else GS_SH_DENSE_(DD, FILLV, false); } while (0)
-    if (p->num_coeffs == 16) {
-      if (fill) GS_SH_DENSE(16, true); else GS_SH_DENSE(16, false);
-    } else {
-      if (fill) GS_SH_DENSE(4, true); else GS_SH_DENSE(4, false);
+    // 16 B units where the rows allow them (D = 4, 16) and the pointers they go through are 16 B aligned
+    const bool a16 = aligned16(grad_params) && (from_out || aligned16(params));
+#define GS_SH_DENSE_ARGS fill, from_out, p, params, positions, indexes, camera_pos, grad_out, grad_params, \
+                         grad_positions, grad_camera_pos, st
+    switch (p->num_coeffs) {
+      case 1: launch_sh_dense<1, false>(GS_SH_DENSE_ARGS); break;
+      case 4: if (a16) launch_sh_dense<4, true>(GS_SH_DENSE_ARGS); else launch_sh_dense<4, false>(GS_SH_DENSE_ARGS); break;
+      case 9: launch_sh_dense<9, false>(GS_SH_DENSE_ARGS); break;
+      default: if (a16) launch_sh_dense<16, true>(GS_SH_DENSE_ARGS); else launch_sh_dense<16, false>(GS_SH_DENSE_ARGS);
     }
-#undef GS_SH_DENSE
-#undef GS_SH_DENSE_
+#undef GS_SH_DENSE_ARGS
     GS_LAUNCH_CHECK();
     return GS_OK;
   }
@@ -866,8 +1002,9 @@ int gs_sh_bwd_stage_counted(const GsSHParams* p, const void* forward_out, const 
 int gs_sh_bwd_flush(const GsSHParams* p, int32_t num_views, const void* const* staged,
                     const void* const* camera_positions, const void* positions, void* grad_params, void* stream) {
   GS_CHECK_ARG(p != nullptr, "gs_sh_bwd_flush: null params");
-  if (p->dtype != GS_F32 || p->num_channels != 3 || (p->num_coeffs != 16 && p->num_coeffs != 4)) {
-    set_error("gs_sh_bwd_flush: f32, K = 3 and D in {4, 16} only");
+  if (!sh_fast_shape(p)) {
+    set_error("gs_sh_bwd_flush: f32, K = 3 and D in {1, 4, 9, 16} only (got dtype %d, K = %d, D = %d)", p->dtype,
+              p->num_channels, p->num_coeffs);
     return GS_ERR_UNSUPPORTED;
   }
   GS_CHECK_ARG(num_views >= 0 && num_views <= kSHMaxDeferred, "gs_sh_bwd_flush: at most 16 views per flush");
@@ -888,13 +1025,16 @@ int gs_sh_bwd_flush(const GsSHParams* p, int32_t num_views, const void* const* s
     views.cam[v] = v < num_views ? (const float*)camera_positions[v] : nullptr;
     GS_CHECK_ARG(v >= num_views || (views.staged[v] && views.cam[v]), "gs_sh_bwd_flush: null view");
   }
-  const unsigned blocks = (unsigned)ceil_div(p->num_points, kSHDenseBlock);
-#define GS_SH_FLUSH(DD, OW)                                                                                        \
-  sh_bwd_flush_kernel<3, DD, OW><<<blocks, kSHDenseBlock, 0, st>>>(p->num_points, num_views, views,               \
-                                                                    (const float*)positions, (float*)grad_params)
-  if (p->num_coeffs == 16) { if (overwrite) GS_SH_FLUSH(16, true); else GS_SH_FLUSH(16, false); }
-  else { if (overwrite) GS_SH_FLUSH(4, true); else GS_SH_FLUSH(4, false); }
-#undef GS_SH_FLUSH
+  // float4 units when grad_params is 16 B aligned (a bucket slice after an odd parameter count is only 4 B aligned)
+  const bool a16 = aligned16(grad_params);
+#define GS_SH_FLUSH_ARGS overwrite, p->num_points, num_views, views, positions, grad_params, st
+  switch (p->num_coeffs) {
+    case 1: if (a16) launch_sh_flush<1, true>(GS_SH_FLUSH_ARGS); else launch_sh_flush<1, false>(GS_SH_FLUSH_ARGS); break;
+    case 4: if (a16) launch_sh_flush<4, true>(GS_SH_FLUSH_ARGS); else launch_sh_flush<4, false>(GS_SH_FLUSH_ARGS); break;
+    case 9: if (a16) launch_sh_flush<9, true>(GS_SH_FLUSH_ARGS); else launch_sh_flush<9, false>(GS_SH_FLUSH_ARGS); break;
+    default: if (a16) launch_sh_flush<16, true>(GS_SH_FLUSH_ARGS); else launch_sh_flush<16, false>(GS_SH_FLUSH_ARGS);
+  }
+#undef GS_SH_FLUSH_ARGS
   GS_LAUNCH_CHECK();
   return GS_OK;
 }
@@ -902,8 +1042,9 @@ int gs_sh_bwd_flush(const GsSHParams* p, int32_t num_views, const void* const* s
 int gs_sh_fwd_views(const GsSHParams* p, int32_t num_views, const void* params, const void* positions,
                     const void* const* camera_positions, void* const* outs, void* stream) {
   GS_CHECK_ARG(p != nullptr, "gs_sh_fwd_views: null params");
-  if (p->dtype != GS_F32 || p->num_channels != 3 || (p->num_coeffs != 16 && p->num_coeffs != 4)) {
-    set_error("gs_sh_fwd_views: f32, K = 3 and D in {4, 16} only");
+  if (!sh_fast_shape(p)) {
+    set_error("gs_sh_fwd_views: f32, K = 3 and D in {1, 4, 9, 16} only (got dtype %d, K = %d, D = %d)", p->dtype,
+              p->num_channels, p->num_coeffs);
     return GS_ERR_UNSUPPORTED;
   }
   GS_CHECK_ARG(num_views >= 0 && num_views <= kSHMaxDeferred, "gs_sh_fwd_views: at most 16 views per call");
@@ -915,14 +1056,17 @@ int gs_sh_fwd_views(const GsSHParams* p, int32_t num_views, const void* params, 
     views.cam[v] = v < num_views ? (const float*)camera_positions[v] : nullptr;
     GS_CHECK_ARG(v >= num_views || (views.out[v] && views.cam[v]), "gs_sh_fwd_views: null view");
   }
-  const unsigned blocks = (unsigned)ceil_div(p->num_points, 128);
   cudaStream_t st = (cudaStream_t)stream;
-  if (p->num_coeffs == 16)
-    sh_fwd_views_kernel<3, 16><<<blocks, 128, 0, st>>>(p->num_points, num_views, views, (const float*)params,
-                                                       (const float*)positions);
-  else
-    sh_fwd_views_kernel<3, 4><<<blocks, 128, 0, st>>>(p->num_points, num_views, views, (const float*)params,
-                                                      (const float*)positions);
+  const bool a16 = aligned16(params);   // float4 rows at D = 4, 16; rows of 3 or 27 floats are read one float at a time
+#define GS_SH_VIEWS_ARGS p->num_points, num_views, views, params, positions, st
+  switch (p->num_coeffs) {
+    case 1: launch_sh_fwd_views<1, false>(GS_SH_VIEWS_ARGS); break;
+    case 4: if (a16) launch_sh_fwd_views<4, true>(GS_SH_VIEWS_ARGS); else launch_sh_fwd_views<4, false>(GS_SH_VIEWS_ARGS); break;
+    case 9: launch_sh_fwd_views<9, false>(GS_SH_VIEWS_ARGS); break;
+    default:
+      if (a16) launch_sh_fwd_views<16, true>(GS_SH_VIEWS_ARGS); else launch_sh_fwd_views<16, false>(GS_SH_VIEWS_ARGS);
+  }
+#undef GS_SH_VIEWS_ARGS
   GS_LAUNCH_CHECK();
   return GS_OK;
 }

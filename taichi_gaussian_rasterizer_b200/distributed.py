@@ -76,15 +76,15 @@ class GradientBucket:
     fill of the culled rows.  Results are the same sums; parameters the kernels cannot serve this way (other
     dtypes, features used without SH) keep the normal autograd accumulation.
 
-    The SH coefficient gradient (N, 3, 4 | 16, f32) of the batch is formed ONCE, by ``flush()`` (called on exit and by
+    The SH coefficient gradient (N, 3, 1 | 4 | 9 | 16, f32: spherical_harmonics.sh_fast_path) of the batch is formed ONCE, by ``flush()`` (called on exit and by
     ``all_reduce``): each view only stages its masked colour gradient (N, 3) and the flush adds
     sum_v staged_v (x) basis(position - camera_v) — one pass over the coefficient rows per batch (or per 16 views)
     instead of one read-modify-write pass per view (grad_sinks.DeferredSH).  Anything that reads the SH gradient
     inside the context (an optimizer step, say) must call ``flush()`` first."""
     from . import grad_sinks
+    from .spherical_harmonics import sh_fast_path
     served = [p for p in self.params if p.is_cuda and p.grad is not None]
-    deferred = [p for p in served if p.dtype == torch.float32 and p.ndim == 3 and p.shape[1] == 3
-                and p.shape[2] in (4, 16)]
+    deferred = [p for p in served if sh_fast_path(p)]
     for p in served:
       grad_sinks.register_grad_sink(p, p.grad)
     for p in deferred:

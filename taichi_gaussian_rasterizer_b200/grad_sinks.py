@@ -102,6 +102,21 @@ class DeferredSH:
     self.pending, self.points, self.hold = [], None, False
     return pending, points
 
+  @staticmethod
+  def chunk_bounds(n: int, chunks: int):
+    """Row bounds [0, ..., n] of ``flush(chunks=)``: up to ``chunks`` non-empty slices of about equal size, every
+    inner bound a multiple of 4 rows.  A slice then starts a multiple of 4 floats into the sink at any row width
+    (3 D floats), so the flush kernel keeps the sink's 16 B alignment and a reducer offset stays a multiple of 4 floats."""
+    if n <= 0:
+      return [0, 0]
+    chunks = max(1, min(int(chunks), n))
+    bounds = [0]
+    for c in range(1, chunks + 1):
+      b = min(n, -(-((n * c) // chunks) // 4) * 4)
+      if b > bounds[-1]:
+        bounds.append(b)
+    return bounds
+
   def flush(self, chunks: int = 1, after_chunk=None):
     """``chunks`` > 1: the rows are flushed in that many slices and ``after_chunk(lo, hi)`` is called after each
     slice's kernel has been enqueued (GradientBucket.all_reduce starts reducing a slice while the next one is formed)."""
@@ -109,16 +124,13 @@ class DeferredSH:
       self.points = None
       return False
     self._order_after_producers()
-    n = self.sink.shape[0]
-    chunks = max(1, min(int(chunks), n))
-    bounds = [(n * c) // chunks for c in range(chunks + 1)]
-    for c in range(chunks):
-      lo, hi = bounds[c], bounds[c + 1]
+    bounds = self.chunk_bounds(self.sink.shape[0], chunks)
+    for lo, hi in zip(bounds, bounds[1:]):
       if len(self.pending) == 0:   # clean sink, nothing staged: the rows become zeros
         self.sink[lo:hi].zero_()
       else:
         flush_sh_views(self.sink, self.points, [p[0] for p in self.pending], [p[1] for p in self.pending],
-                       self.overwrite_next, **({"rows": (lo, hi)} if chunks > 1 else {}))
+                       self.overwrite_next, **({"rows": (lo, hi)} if len(bounds) > 2 else {}))
       if after_chunk is not None:
         after_chunk(lo, hi)
     if self.sink.is_cuda:

@@ -25,6 +25,15 @@ def check_sh_degree(sh_features):
   return n - 1
 
 
+def sh_fast_path(sh_params: torch.Tensor) -> bool:
+  """Whether the batched forward (evaluate_sh_views), the counted forward / backward (render_gaussians(...,
+  overlap_capacity=)), the dense backward and the deferred gradient of GradientBucket.fused_accumulation() serve these
+  coefficients: float32, 3 channels, degree 0..3, i.e. (N, 3, 1 | 4 | 9 | 16).  Other shapes take the generic kernels
+  (or are refused where there is no generic path)."""
+  return sh_params.dtype == torch.float32 and sh_params.ndim == 3 and sh_params.shape[1] == 3 \
+    and sh_params.shape[2] in (1, 4, 9, 16)
+
+
 class _SHFunction(torch.autograd.Function):
 
   @staticmethod
@@ -34,8 +43,8 @@ class _SHFunction(torch.autograd.Function):
     p = N.GsSHParams(N.dtype_code(params.dtype), k, d, int(bool(sorted_unique)), m, v, 0, 0)
     ctx.count = count   # (1,) int32 on the device: only the first count[0] rows of indexes / out are valid
     if count is not None:
-      assert precomputed is not None and sorted_unique and params.dtype == torch.float32 and k == 3 and d in (4, 16), \
-        "counted SH evaluation: precomputed f32 colours of the ascending visible set, 3 channels, degree 1 or 3"
+      assert precomputed is not None and sorted_unique and sh_fast_path(params), \
+        "counted SH evaluation: precomputed f32 colours of the ascending visible set, 3 channels, degree 0..3"
     if precomputed is not None:     # evaluated ahead of time on the capacity buffers (launch_sh_forward_counted)
       assert precomputed.shape == (v, k)
       out = precomputed
@@ -53,8 +62,7 @@ class _SHFunction(torch.autograd.Function):
   def backward(ctx, doutput):
     params, points, indexes, camera_pos, out = ctx.saved_tensors
     need = ctx.needs_input_grad
-    dense = ctx.sorted_unique and params.dtype == torch.float32 and params.shape[1] == 3 and params.shape[2] in (4, 16) \
-      and indexes.shape[0] > 0
+    dense = ctx.sorted_unique and sh_fast_path(params) and indexes.shape[0] > 0
     sink = grad_sink(params) if (need[0] and dense) else None
     g_points = torch.empty_like(points) if need[1] else None
     g_cam = torch.empty_like(camera_pos) if need[3] else None
@@ -119,14 +127,14 @@ def launch_sh_forward_counted(sh_params, positions, indexes_capacity, count_devi
 def evaluate_sh_views(sh_params: torch.Tensor, positions: torch.Tensor, camera_positions) -> list:
   """Colours of ALL gaussians for every view of a batch, one dense (M, K) tensor per camera position (extension, not
   in the reference): the coefficient rows are read once per batch instead of once per view (gs_sh_fwd_views; f32,
-  K = 3, degree 1 or 3).  Pass a view's tensor to ``render_gaussians(..., sh_colors=...)``, which gathers the visible
+  K = 3, degree 0..3).  Pass a view's tensor to ``render_gaussians(..., sh_colors=...)``, which gathers the visible
   rows and builds the same autograd node as ``evaluate_sh_at`` (gradients reach ``sh_params``).  Worth it when most
   gaussians are in view in most views; values are those of ``evaluate_sh_at``."""
   check_sh_degree(sh_params)
   N.require_cuda(sh_params, positions)
   m, k, d = sh_params.shape
-  assert sh_params.dtype == torch.float32 and k == 3 and d in (4, 16), \
-    f"evaluate_sh_views: float32, 3 channels, degree 1 or 3 (got {sh_params.dtype}, {tuple(sh_params.shape)})"
+  assert sh_fast_path(sh_params), \
+    f"evaluate_sh_views: float32, 3 channels, degree 0..3 (got {sh_params.dtype}, {tuple(sh_params.shape)})"
   params = sh_params.detach().contiguous()
   pos = positions.detach().to(torch.float32).contiguous()
   cams = [c.detach().to(torch.float32).contiguous() for c in camera_positions]
